@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --steps K --warmup W --dump-outputs DIR  (also writes DIR/<name>.npy, see dump_outputs)
 
 metric   chain-steps x observations / second.  One chain-step = one (mcmciter, pidx)
          schedule element for one chain = one full-data log-likelihood evaluation
@@ -43,6 +44,8 @@ os.environ["NCCL_DEBUG_FILE"] = "/dev/stderr"
 N_OBS = 1_000_000
 CHAINS_PER_GPU = 4096
 NU = 2
+# cfg 4 is timed in blocks of this many iterations per extmcmc_run_block (see measure_cfg34)
+CFG4_BLOCK_ITERS = 10
 
 
 def cfg2_data():
@@ -228,6 +231,41 @@ def timed_steps(ws, _abi, C, K, W, flush=True, it0=1):
     return total
 
 
+def last_step_outputs(ws, _abi, n_iters):
+    """What a caller of the timed path receives after its last step (iteration n_iters, both
+    updates), as float64 arrays with the chain axis last: the chain state and its log-likelihood,
+    that iteration's proposals, their log-likelihoods and the accept decisions (from the device
+    history ring), the step size of every update and the running chain statistics."""
+    p, C = ws.p, ws.C
+    theta, ll = ws.refresh_state()
+    prop, llp, acc = np.empty((NU, p, C)), np.empty((NU, C)), np.empty((NU, C), dtype=np.uint8)
+    ws._ck(ws.lib.extmcmc_get_history(ws.handle, (n_iters - 1) * NU, n_iters * NU, None, _abi.dptr(prop), None,
+                                      _abi.dptr(llp), acc.ctypes.data_as(_abi.c_uint8_p)))
+    st = ws.stats()
+    out = {"theta": theta, "loglik": ll, "theta_prop": prop, "loglik_prop": llp, "accepted": acc,
+           "eps": np.concatenate([ws.eps(u) for u in range(1, NU + 1)]),
+           "mean": st["mean"], "cov": st["cov"], "rolling_accept_rate": st["rolling_ar"],
+           "n_accept": st["n_accept"], "n_prop": st["n_prop"]}
+    return {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in out.items()}
+
+
+def dump_outputs(dirname, arrays, dist=None):
+    """Writes dirname/<name>.npy for every array; with several ranks the chains of all ranks are
+    gathered (rank order along the chain axis) and rank 0 writes them."""
+    if dist is not None:
+        import torch
+        for k, a in arrays.items():
+            t = torch.from_numpy(a).cuda()
+            parts = [torch.empty_like(t) for _ in range(dist.get_world_size())]
+            dist.all_gather(parts, t)
+            arrays[k] = torch.cat(parts, dim=-1).cpu().numpy()
+        if dist.get_rank() != 0:
+            return
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
+
+
 def ncu_traffic(kernel_substr, csv_name):
     """dram__bytes_read.sum + dram__bytes_write.sum of one kernel launch, read at run time from the
     committed summary of an `ncu --set full` capture (tools/ncu_summary.py) under profiles/."""
@@ -406,7 +444,7 @@ def measure_cfg34(args, workload, em, _abi, local, steps, chain_offset=0):
     # iterations per extmcmc_run_block: cfg 4 runs blocks of 10 iterations (30 schedule elements, like the
     # cfg 5 sub-record and well below run_()'s default block of 128 elements) -- the last element of a block
     # cannot leave its bookkeeping to the next element's kernels, which costs ~4 us per block; cfg 3: 1
-    IPB = 10 if workload == "cfg4" else 1
+    IPB = CFG4_BLOCK_ITERS if workload == "cfg4" else 1
 
     def make(instrument):
         mcmc = em.MCMC(ups, backend=em.CUDAMCMCBackend(n_chains=C, device=local, seed=7, history="none", block_len=NUc * IPB,
@@ -415,7 +453,7 @@ def measure_cfg34(args, workload, em, _abi, local, steps, chain_offset=0):
         init_(mcmc, 1, data, th0)
         return mcmc.workspace
     up = lambda n: -(-n // IPB) * IPB            # whole blocks
-    K, Wm = up(steps), up(3)
+    K, Wm = steps, up(3)                         # main() admits only whole blocks of timed steps
     ws = make(False)
     sampler = ClockSampler(local)
     _generic_timed(ws, _abi, NUc, 0, Wm, ipb=IPB)
@@ -504,6 +542,8 @@ def run_ours(args):
     barrier()
     ms_total = timed_steps(ws, _abi, C, K, 0, it0=Wm + 1)
     barrier()
+    if args.dump_outputs:   # read back before the untimed continuation below moves the chains on
+        dump_outputs(args.dump_outputs, last_step_outputs(ws, _abi, Wm + K), dist)
     ext = [Wm + 1 + K]   # a timed region shorter than three samples: keep the same load going, untimed
 
     def hold():
@@ -780,7 +820,6 @@ def run_reference(args):
     ups = cfg2_updates(em)
     o = orc.Oracle(em.GsnTargetLaw([0.0]), ups, x, cfg2_theta_init(x, n_chains), n_chains, seed=3)
     K, Wm = args.steps, max(args.warmup, 1)
-    K = min(K, 200)
     sched = list(em.MCMCSchedule(Wm + K, NU))
     o.run(sched[:Wm * NU], n_threads=nthr, record=False)
     t0 = time.perf_counter()
@@ -837,7 +876,17 @@ def main():
     ap.add_argument("--cfg3-steps", type=int, default=5)
     ap.add_argument("--cfg4-steps", type=int, default=400)
     ap.add_argument("--ref-ess-iters", type=int, default=2000, help="reference arm: iterations of the ESS trace")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="cfg2: after the timed steps, write what the last one computed (chain state, log-likelihoods, "
+                         "proposals, decisions, step sizes, chain statistics) as DIR/<name>.npy, float64; the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared array for array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.cfg4_steps % CFG4_BLOCK_ITERS or (args.workload == "cfg4" and args.steps % CFG4_BLOCK_ITERS):
+        ap.error(f"cfg4 is timed in whole blocks of {CFG4_BLOCK_ITERS} iterations: its steps must be a multiple of that")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "cfg2"):
+        ap.error("--dump-outputs writes the outputs of the cfg2 timed path (--impl ours, --workload cfg2)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload != "cfg2":
