@@ -16,6 +16,7 @@ from .updates import RandomWalkUpdate, MALAUpdate, HamiltonianMCUpdate
 from .gsn_target import GsnTargetLaw
 from .hier_normal import HierNormalLaw
 from .logistic import LogisticLaw
+from .device_law import DeviceLaw
 from .workspaces import (CUDAMCMCBackend, CUDAGlobalWorkspace, CUDALocalWorkspace,
                          DeviceGeneratedObs, init_global_workspace, create_workspace,
                          create_workspaces, state, state_prop, ll, ll_prop, accepted, set_accepted_, llr,

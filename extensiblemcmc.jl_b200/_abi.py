@@ -16,7 +16,7 @@ ABI_VERSION = 2
 # status codes
 OK, EINVAL, EUNSUPPORTED, ECUDA, ENCCL, EOOM, EDOMAIN, ESTALE = 0, -1, -2, -3, -4, -5, -6, -7
 # laws
-LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL = 1, 2, 3, 4
+LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = 1, 2, 3, 4, 5
 # kernels
 KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = 1, 2, 3, 4
 # priors
@@ -107,6 +107,8 @@ SIGNATURES = {
     "extmcmc_last_error": (C.c_char_p, [Handle]),
     "extmcmc_upload_obs": (C.c_int32, [Handle, c_double_p, C.c_int64, C.c_int32, c_double_p]),
     "extmcmc_generate_obs_normal": (C.c_int32, [Handle, C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_uint64]),
+    "extmcmc_set_user_law": (C.c_int32, [Handle, C.c_char_p, C.c_int32]),
+    "extmcmc_user_law_check": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_char_p, C.c_int64]),
     "extmcmc_set_update": (C.c_int32, [Handle, C.c_int32, C.POINTER(Update)]),
     "extmcmc_set_state": (C.c_int32, [Handle, c_double_p]),
     "extmcmc_set_seed": (C.c_int32, [Handle, C.c_uint64]),

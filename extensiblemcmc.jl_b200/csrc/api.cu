@@ -21,6 +21,7 @@
 #include "block_kernels.h"
 #include "step_kernels.h"
 #include "sweep.h"
+#include "user_law.h"
 
 using namespace extmcmc;
 
@@ -81,6 +82,7 @@ struct extmcmc_handle {
     int64_t n_obs_largest = 0;           // observations of the largest group
     int64_t *goff_dev = nullptr, *glen_dev = nullptr;  // [G] padded group offsets / true lengths
     double *y_dev = nullptr;             // LOGISTIC: responses, padded like the rows of X
+    UserLaw ulaw;                        // USER: the compiled law (extmcmc_set_user_law)
     int logi_D = 0;                      // LOGISTIC: padded feature dimension
     unsigned int *tail_counter = nullptr; // CTA counter of the fused sweep tail
     bool tail = false;                   // the obs-mapped sweep finishes the reduction itself
@@ -207,7 +209,10 @@ int32_t ensure_plan(extmcmc_t h) {
         h->plan = plan_sweep_gsnmv(h->cfg.obs_dim, h->d.C, h->n_obs_local, h->cfg.sweep_variant, h->num_sms);
     else if (h->cfg.law == EXTMCMC_LAW_LOGISTIC)
         h->plan = plan_sweep_logistic(h->cfg.obs_dim, h->d.C, h->n_obs_local, h->num_sms);
-    else
+    else if (h->cfg.law == EXTMCMC_LAW_USER) {
+        if (!h->ulaw.loaded) return fail(h, EXTMCMC_EINVAL, "no user law: call extmcmc_set_user_law first");
+        h->plan = plan_sweep_user(h->ulaw, h->d.C, h->n_obs_local, h->cfg.sweep_variant, h->num_sms);
+    } else
         return fail(h, EXTMCMC_EUNSUPPORTED, "law not implemented on the GPU path");
     h->d.S = h->plan.S;
     // fused tail of the obs-mapped 1-D sweep (few chains, many segments): see sweep.h
@@ -218,11 +223,11 @@ int32_t ensure_plan(extmcmc_t h) {
         if (rct) return rct;
         CK(h, cudaMemset(h->tail_counter, 0, sizeof(unsigned int)));
     }
-    h->d.use_ssum = (obs_sharded(h) || h->cfg.law == EXTMCMC_LAW_LOGISTIC || h->tail) ? 1 : 0;
+    h->d.use_ssum = (obs_sharded(h) || law_self_finished(h->cfg.law) || h->tail) ? 1 : 0;
     // Gaussian laws: two quantities (second- and first-order sums) x G groups x S segments;
-    // logistic: ll_part[S][C] followed by g_part[S][d][C]
-    size_t part_rows = h->cfg.law == EXTMCMC_LAW_LOGISTIC ? (size_t)h->plan.S * (h->cfg.obs_dim + 1)
-                                                          : (size_t)2 * h->d.G * h->plan.S;
+    // logistic and user laws: ll_part[S][C] followed by g_part[S][p][C]
+    size_t part_rows = law_self_finished(h->cfg.law) ? (size_t)h->plan.S * (h->cfg.n_params + 1)
+                                                     : (size_t)2 * h->d.G * h->plan.S;
     part_rows = std::max(part_rows, (size_t)h->num_sms * 3);   // segments of the observation-mapped block kernel
     part_rows = std::max(part_rows, (size_t)2 * h->d.G * 4);   // members of a team of the team-resident block kernel
     int32_t rc = dev_alloc(h, &h->d.partial, part_rows * h->d.C);
@@ -431,6 +436,20 @@ int32_t enqueue_sweep(extmcmc_t h, bool instrument, bool grad = false, const dou
             h->ev_pending.push_back(ev);
         }
         return EXTMCMC_OK;
+    } else if (h->cfg.law == EXTMCMC_LAW_USER) {
+        // same contract as the logistic law: the sweep reads the parameters from src and finishes
+        // ll (-> ll_dst) and, with grad, the gradient (-> grad_dst) itself; never sharded by observation
+        UserSweepArgs a{};
+        a.obs = h->obs_dev; a.n_obs = h->n_obs_local; a.theta = src; a.C = h->d.C;
+        a.ll_part = h->d.partial; a.g_part = h->d.partial + (size_t)h->plan.S * h->d.C;
+        a.err_flag = h->d.err_flag; a.S = h->plan.S;
+        CK(h, launch_sweep_user(h->plan, h->ulaw, a, grad, ll_dst, grad_dst, h->stream));
+        h->launches += h->plan.launches;
+        if (instrument) {
+            CK(h, cudaEventRecord(ev.second, h->stream));
+            h->ev_pending.push_back(ev);
+        }
+        return EXTMCMC_OK;
     } else {
         launch_sweep_gsnmv(h->plan, h->obs_dev, h->n_obs_local, h->d.lawc, h->d.C, h->d.partial, h->stream);
     }
@@ -469,7 +488,7 @@ int32_t enqueue_sweep(extmcmc_t h, bool instrument, bool grad = false, const dou
 // in for the partial buffer (one "segment" per group).
 DevState grad_view(extmcmc_t h) {
     DevState v = h->d;
-    if (obs_sharded(h) && h->cfg.law != EXTMCMC_LAW_LOGISTIC) { v.partial = h->gsum; v.S = 1; }
+    if (obs_sharded(h) && !law_self_finished(h->cfg.law)) { v.partial = h->gsum; v.S = 1; }
     return v;
 }
 
@@ -485,7 +504,7 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
         const bool next_rw = k + 1 < n_steps && !kind_is_mala(kinds[k + 1]);
         const int mode = step_advance(h->dcache, kinds[k], grad_valid, dc_valid);
         if (kind_is_mala(kinds[k])) {
-            const bool logi = h->cfg.law == EXTMCMC_LAW_LOGISTIC;
+            const bool logi = law_self_finished(h->cfg.law);   // the sweep finishes ll and gradient
             int finalize_cur = 0;
             DevState gv = grad_view(h);
             if (mode == 1) {
@@ -527,7 +546,7 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
             fused = next_rw;
             // a MALA element follows and will need the law constants of the (then) current state for
             // its gradient sweep: let this accept kernel write them (fuse_next = 2)
-            cur_prepared = next_mala && h->cfg.law != EXTMCMC_LAW_LOGISTIC && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL;
+            cur_prepared = next_mala && !law_self_finished(h->cfg.law) && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL;
             launch_accept(h->d, d_descs, k, fused ? 1 : (cur_prepared ? 2 : 0), dflags, h->stream, from_cache);
             h->launches += 1;
         }
@@ -560,6 +579,8 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
     if (n_steps > h->cfg.history_window)
         return fail(h, EXTMCMC_EINVAL, "block longer than history_window");
     if (obs_sharded(h) && !h->comm) return fail(h, EXTMCMC_EINVAL, "EXTMCMC_SHARD_OBS needs extmcmc_comm_init first");
+    if (h->cfg.law == EXTMCMC_LAW_USER && h->any_mala && h->ulaw.loaded && !h->ulaw.grad)
+        return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with logpdf_grad (extmcmc_set_user_law with_grad = 1)");
     for (int s = 0; s < n_steps; ++s)
         if (steps[s].pidx < 0 || steps[s].pidx >= h->cfg.n_updates || steps[s].mcmciter < 1)
             return fail(h, EXTMCMC_EINVAL, "step out of range");
@@ -787,6 +808,12 @@ int32_t extmcmc_create(const extmcmc_config_t *cfg, extmcmc_t *out) {
         if (cfg->obs_dim != 1 || cfg->n_params < 3)
             return fail(nullptr, EXTMCMC_EINVAL, "HIER_NORMAL needs obs_dim = 1 and n_params = G + 2 >= 3");
         break;
+    case EXTMCMC_LAW_USER:
+        if (cfg->obs_dim < 1 || cfg->obs_dim > kUserMaxObsDim || cfg->n_params > kUserMaxParams)
+            return fail(nullptr, EXTMCMC_EUNSUPPORTED, "USER needs 1 <= obs_dim <= 64 and 1 <= n_params <= 64");
+        if (cfg->shard_mode == EXTMCMC_SHARD_OBS && cfg->world_size > 1)
+            return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws are not implemented under EXTMCMC_SHARD_OBS with several ranks");
+        break;
     default:
         // the reference's convention for a missing method: error("... not implemented")
         return fail(nullptr, EXTMCMC_EUNSUPPORTED, "target law not implemented on the GPU path");
@@ -842,13 +869,13 @@ int32_t extmcmc_create(const extmcmc_config_t *cfg, extmcmc_t *out) {
     d.obs_dim = cfg->obs_dim;
     d.G = cfg->law == EXTMCMC_LAW_HIER_NORMAL ? cfg->n_params - 2 : 1;
     d.lawc_k = cfg->law == EXTMCMC_LAW_GSN_IID_1D ? 3
-             : cfg->law == EXTMCMC_LAW_LOGISTIC ? 1
+             : law_self_finished(cfg->law) ? 1
              : cfg->law == EXTMCMC_LAW_HIER_NORMAL ? d.G
              : cfg->obs_dim + cfg->obs_dim * (cfg->obs_dim + 1) / 2 + 1;
     // the accept kernel reads the finished sum from ssum when another kernel produced it:
     // the NCCL all-reduce under observation sharding, or the logistic sweep's own finalize
     d.use_ssum = ((cfg->shard_mode == EXTMCMC_SHARD_OBS && cfg->world_size > 1) ||
-                  cfg->law == EXTMCMC_LAW_LOGISTIC) ? 1 : 0;
+                  law_self_finished(cfg->law)) ? 1 : 0;
     int32_t rc = 0;
     const size_t covn = cfg->stats_mode == 0 ? (size_t)p * p : (cfg->stats_mode == 1 ? (size_t)p : 0);
     if ((rc = dev_alloc(h, &d.theta, (size_t)p * C)) || (rc = dev_alloc(h, &d.ll, (size_t)C)) ||
@@ -921,6 +948,7 @@ int32_t extmcmc_destroy(extmcmc_t h) {
     for (void *p : h->allocs) cudaFree(p);
     if (h->obs_dev) cudaFree(h->obs_dev);
     if (h->y_dev) cudaFree(h->y_dev);
+    user_law_unload(h->ulaw);
     if (h->rp_prop) cudaFree(h->rp_prop);
     if (h->rp_exp) cudaFree(h->rp_exp);
     if (h->flush_buf) cudaFree(h->flush_buf);
@@ -1000,6 +1028,23 @@ int32_t extmcmc_upload_obs(extmcmc_t h, const double *obs, int64_t n_obs, int32_
         h->dc_valid = false;
         return EXTMCMC_OK;
     }
+    if (h->cfg.law == EXTMCMC_LAW_USER) {
+        // rows [n_pad][D], n_pad even: every tile of the sweep is a whole number of 16-byte units
+        if (y) return fail(h, EXTMCMC_EINVAL, "USER takes no y: responses and covariates are columns of the rows");
+        const size_t n_pad = ((size_t)n_obs + 1) & ~(size_t)1, nd = (size_t)n_obs * obs_dim;
+        if (h->obs_dev) { cudaFree(h->obs_dev); h->obs_dev = nullptr; }
+        CK(h, cudaMalloc(&h->obs_dev, n_pad * obs_dim * sizeof(double)));
+        CK(h, cudaMemsetAsync(h->obs_dev, 0, n_pad * obs_dim * sizeof(double), h->stream));
+        CK(h, cudaMemcpyAsync(h->obs_dev, obs, nd * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        CK(h, cudaStreamSynchronize(h->stream));
+        h->n_obs_local = n_obs;
+        h->n_obs_largest = n_obs;
+        h->plan_valid = false;
+        h->n_total_known = false;
+        h->grad_valid = false;
+        h->dc_valid = false;
+        return EXTMCMC_OK;
+    }
     std::vector<int64_t> glen(h->d.G, 0);
     if (h->cfg.law == EXTMCMC_LAW_HIER_NORMAL) {
         // y[i] = group index of observation i (0-based), non-decreasing
@@ -1070,8 +1115,10 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
         return fail(h, EXTMCMC_EUNSUPPORTED, "transition kernel not implemented on the GPU path");
     if (mala) {
         if (h->cfg.law != EXTMCMC_LAW_GSN_IID_1D && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL &&
-            h->cfg.law != EXTMCMC_LAW_LOGISTIC)
-            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a law with a device gradient (GSN_IID_1D, HIER_NORMAL, LOGISTIC)");
+            h->cfg.law != EXTMCMC_LAW_LOGISTIC && h->cfg.law != EXTMCMC_LAW_USER)
+            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a law with a device gradient (GSN_IID_1D, HIER_NORMAL, LOGISTIC, USER)");
+        if (h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.loaded && !h->ulaw.grad)
+            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with logpdf_grad (extmcmc_set_user_law with_grad = 1)");
         if (upd->prior != EXTMCMC_PRIOR_IMPROPER && upd->prior != EXTMCMC_PRIOR_NORMAL)
             return fail(h, EXTMCMC_EUNSUPPORTED, "MALA supports ImproperPrior and Normal priors only");
         if (upd->pos)
@@ -1287,6 +1334,45 @@ int32_t extmcmc_set_state(extmcmc_t h, const double *theta) {
     return EXTMCMC_OK;
 }
 
+int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                               char *log, int64_t log_bytes) {
+    if (log && log_bytes > 0) log[0] = 0;
+    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
+    if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
+        return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
+    std::string lg, cubin;
+    const int32_t rc = user_law_compile(source, n_params, obs_dim, with_grad != 0, lg, cubin, nullptr);
+    if (log && log_bytes > 0) {
+        const size_t n = std::min(lg.size(), (size_t)log_bytes - 1);
+        std::memcpy(log, lg.data(), n);
+        log[n] = 0;
+    }
+    if (rc) g_create_error = lg;
+    return rc;
+}
+
+int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad) {
+    if (!h) return EXTMCMC_EINVAL;
+    if (h->cfg.law != EXTMCMC_LAW_USER) return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_law needs a handle of law EXTMCMC_LAW_USER");
+    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
+    std::string log, cubin;
+    uint64_t hash = 0;
+    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, with_grad != 0, log, cubin, &hash);
+    if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
+    if (rc) return fail(h, rc, log);
+    CK(h, cudaSetDevice(h->cfg.device));
+    CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
+    invalidate_graphs(h);
+    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, with_grad != 0, hash);
+    if (e != cudaSuccess) {
+        user_law_unload(h->ulaw);
+        return fail(h, EXTMCMC_ECUDA, std::string("loading the user law: ") + cudaGetErrorString(e));
+    }
+    h->plan_valid = false;
+    h->grad_valid = false;
+    return EXTMCMC_OK;
+}
+
 // ---- checkpoint / resume ------------------------------------------------------------------------
 }  // extern "C"
 namespace {
@@ -1329,7 +1415,8 @@ int32_t extmcmc_checkpoint_size(extmcmc_t h, int64_t *bytes_out) {
     if (!h || !bytes_out) return EXTMCMC_EINVAL;
     for (int u = 0; u < h->cfg.n_updates; ++u)
         if (!h->upd_set[u]) return fail(h, EXTMCMC_EINVAL, "update " + std::to_string(u) + " not set");
-    size_t tot = sizeof(CkptHeader);
+    if (h->cfg.law == EXTMCMC_LAW_USER && !h->ulaw.loaded) return fail(h, EXTMCMC_EINVAL, "no user law: call extmcmc_set_user_law first");
+    size_t tot = sizeof(CkptHeader) + (h->cfg.law == EXTMCMC_LAW_USER ? sizeof(uint64_t) : 0);   // + hash of the law
     ckpt_walk(h, [&](void *, void *, size_t b) { tot += b; return EXTMCMC_OK; });
     *bytes_out = (int64_t)tot;
     return EXTMCMC_OK;
@@ -1348,6 +1435,7 @@ int32_t extmcmc_checkpoint_save(extmcmc_t h, void *blob, int64_t bytes) {
     char *out = (char *)blob;
     std::memcpy(out, &hd, sizeof hd);
     out += sizeof hd;
+    if (h->cfg.law == EXTMCMC_LAW_USER) { std::memcpy(out, &h->ulaw.hash, sizeof(uint64_t)); out += sizeof(uint64_t); }
     return ckpt_walk(h, [&](void *dev, void *host, size_t b) -> int32_t {
         if (dev) { CK(h, cudaMemcpy(out, dev, b, cudaMemcpyDeviceToHost)); }
         else std::memcpy(out, host, b);
@@ -1366,9 +1454,15 @@ int32_t extmcmc_checkpoint_load(extmcmc_t h, const void *blob, int64_t bytes) {
     if (hd.magic != kCkptMagic || hd.abi != EXTMCMC_ABI_VERSION || hd.C != h->d.C || hd.p != h->d.p || hd.NU != h->d.NU ||
         hd.W != h->d.W || hd.stats_mode != h->d.stats_mode || hd.law != h->d.law)
         return fail(h, EXTMCMC_EINVAL, "checkpoint does not match this handle (chains, parameters, updates, windows, law)");
+    const char *in = (const char *)blob + sizeof hd;
+    if (h->cfg.law == EXTMCMC_LAW_USER) {
+        uint64_t hash;
+        std::memcpy(&hash, in, sizeof hash);
+        if (hash != h->ulaw.hash) return fail(h, EXTMCMC_EINVAL, "checkpoint was written under another user law");
+        in += sizeof hash;
+    }
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaStreamSynchronize(h->stream));
-    const char *in = (const char *)blob + sizeof hd;
     rc = ckpt_walk(h, [&](void *dev, void *host, size_t b) -> int32_t {
         if (dev) { CK(h, cudaMemcpy(dev, in, b, cudaMemcpyHostToDevice)); }
         else std::memcpy(host, in, b);
@@ -1651,7 +1745,7 @@ int32_t extmcmc_eval_loglik(extmcmc_t h, double *ll_out) {
     int32_t rc;
     if ((rc = ensure_plan(h))) return rc;
     if ((rc = ensure_total_obs(h))) return rc;
-    if (h->cfg.law == EXTMCMC_LAW_LOGISTIC) {
+    if (law_self_finished(h->cfg.law)) {
         if ((rc = enqueue_sweep(h, h->cfg.instrument != 0, false, h->d.theta, h->scratch_ll, nullptr))) return rc;
     } else {
         launch_prepare_current(h->d, h->stream);
@@ -1669,15 +1763,16 @@ int32_t extmcmc_eval_loglik(extmcmc_t h, double *ll_out) {
 int32_t extmcmc_eval_grad(extmcmc_t h, double *ll_out, double *grad_out) {
     if (!h || !grad_out) return EXTMCMC_EINVAL;
     if (!h->obs_dev || !h->state_set) return fail(h, EXTMCMC_EINVAL, "observations and state required");
-    if (h->cfg.law != EXTMCMC_LAW_GSN_IID_1D && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL &&
-        h->cfg.law != EXTMCMC_LAW_LOGISTIC)
+    if ((h->cfg.law != EXTMCMC_LAW_GSN_IID_1D && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL &&
+         h->cfg.law != EXTMCMC_LAW_LOGISTIC && h->cfg.law != EXTMCMC_LAW_USER) ||
+        (h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.loaded && !h->ulaw.grad))
         return fail(h, EXTMCMC_EUNSUPPORTED, "this law has no device gradient");
     if (obs_sharded(h) && !h->comm) return fail(h, EXTMCMC_EINVAL, "EXTMCMC_SHARD_OBS needs extmcmc_comm_init first");
     CK(h, cudaSetDevice(h->cfg.device));
     int32_t rc;
     if ((rc = ensure_plan(h))) return rc;
     if ((rc = ensure_total_obs(h))) return rc;
-    if (h->cfg.law == EXTMCMC_LAW_LOGISTIC) {
+    if (law_self_finished(h->cfg.law)) {
         if ((rc = enqueue_sweep(h, h->cfg.instrument != 0, true, h->d.theta, h->scratch_ll, h->d.grad_cur))) return rc;
     } else {
         launch_prepare_current(h->d, h->stream);

@@ -20,6 +20,12 @@ constexpr int kMaxPriorParams = 1 + 4 * kMaxPriorFactors;
 constexpr int kDataCacheMaxG = 16;   // most observation groups the data-sum cache serves (= kCoopG, step_kernels.cu)
 constexpr int kMaxObsDim = 16;       // general-d Gaussian law on the device: d <= 16
 
+// Laws whose sweep finishes ll (into ssum / ll_prop) and the gradient itself: the step kernels take
+// the log-likelihood as it comes and prepare no law constants.
+__host__ __device__ constexpr bool law_self_finished(int law) {
+    return law == EXTMCMC_LAW_LOGISTIC || law == EXTMCMC_LAW_USER;
+}
+
 // prior families the compact (SpecLean) step kernels carry
 inline bool lean_prior(int kind) {
     return kind == EXTMCMC_PRIOR_IMPROPER || kind == EXTMCMC_PRIOR_IMPROPER_POS || kind == EXTMCMC_PRIOR_NORMAL;

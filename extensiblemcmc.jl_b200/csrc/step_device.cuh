@@ -55,6 +55,8 @@ struct MatRef {
 // law is LAW, every random-walk update of the handle is a UniformRandomWalk, every prior is one of
 // Improper / ImproperPos / Normal and no update carries a HaarioTypeAdaptation -- the host checks
 // this per handle (DevState.lean) and picks the instantiation; the arithmetic is the same code.
+// The laws whose sweep finishes ll and gradient (law_self_finished) share SpecLean<LOGISTIC>: their
+// step kernels do not depend on the law otherwise.
 struct SpecAny {
     static constexpr int kLaw = -1;
     static constexpr bool kLean = false;
@@ -348,7 +350,7 @@ __device__ __forceinline__ void law_prepare(const DevState &d, int64_t c, const 
 template <class SP = SpecAny>
 __device__ __forceinline__ double law_finalize(const DevState &d, int64_t c, double S, const double *th) {
     const int law = sp_law<SP>(d);
-    if (law == EXTMCMC_LAW_LOGISTIC) return S;  // the logistic sweep finishes ll itself
+    if (law_self_finished(law)) return S;  // the sweep finished ll itself
     if (law == EXTMCMC_LAW_GSN_IID_1D)  // N*c0 - S/(2 var)
         return (double)d.n_obs_total * d.lawc[d.C + c] - S * d.lawc[2 * d.C + c];
     if (law == EXTMCMC_LAW_HIER_NORMAL) {

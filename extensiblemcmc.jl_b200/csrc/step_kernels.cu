@@ -614,7 +614,7 @@ template <class F>
 static inline void with_spec(const DevState &d, F f) {
     if (d.lean && d.law == EXTMCMC_LAW_GSN_IID_1D) f(SpecLean<EXTMCMC_LAW_GSN_IID_1D>{});
     else if (d.lean && d.law == EXTMCMC_LAW_HIER_NORMAL) f(SpecLean<EXTMCMC_LAW_HIER_NORMAL>{});
-    else if (d.lean && d.law == EXTMCMC_LAW_LOGISTIC) f(SpecLean<EXTMCMC_LAW_LOGISTIC>{});
+    else if (d.lean && law_self_finished(d.law)) f(SpecLean<EXTMCMC_LAW_LOGISTIC>{});
     else f(SpecAny{});
 }
 void launch_propose(const DevState &d, const StepDesc *descs, int k, cudaStream_t st) {

@@ -1,0 +1,160 @@
+// Likelihood sweep of a user-defined law (EXTMCMC_LAW_USER): the kernel template that NVRTC
+// instantiates at run time around the user's `Law`, `set_parameters` and `logpdf` (+ `logpdf_grad`),
+// see user_law.cu and INTEGRATION.md.  nvcc compiles this header too (user_law.cu: the argument
+// struct and the shape constants the host planner shares with the kernel); the template is only
+// instantiated in the NVRTC program, where the user's functions are visible.
+//
+// grid = (observation segments S, chain groups).  A CTA streams the rows of its segment HBM/L2 ->
+// shared memory with 1-D TMA bulk copies (tma.cuh) in a ring of kUserStages tiles.  A thread holds
+// R chains: for each it calls set_parameters once on the evaluated state theta[P][C] and keeps the
+// Law in registers for the whole sweep, then walks the rows j = lane (mod L) of every tile:
+//   L = 1  ("chains"): every thread of the CTA reads the same row (broadcast), R chains per thread;
+//   L = 32 ("lanes") : a warp shares one chain, lane l takes rows l, l + 32, ... of each tile.
+// Each thread accumulates its rows in order; the lanes of a chain are combined by a fixed xor-shuffle
+// tree; per-segment sums go to ll_part[S][C] and g_part[S][P][C], which the finalize kernel
+// (user_law.cu) adds in segment order.  No atomics: the result does not depend on the schedule.
+#pragma once
+#ifndef __CUDACC_RTC__
+#include <cstdint>
+#endif
+#include "tma.cuh"
+
+namespace extmcmc {
+
+constexpr int kUserNT = 128;             // threads per CTA, both mappings
+constexpr int kUserStages = 3;           // tiles in flight per CTA
+constexpr int kUserTileDoubles = 1024;   // shared memory per stage: 8 KB
+constexpr int kUserMaxParams = 64;       // n_params of a user law (register file: theta, Law, gradient)
+constexpr int kUserMaxObsDim = 64;       // obs_dim of a user law (>= 16 rows per tile)
+
+// Rows per tile: an even number, so that a tile is a whole number of 16-byte units whatever D is
+// (the device buffer holds an even number of rows, zero-padded).
+__host__ __device__ constexpr int user_tile_rows(int D) { return (kUserTileDoubles / D) & ~1; }
+
+// Chains per thread the "chains" mapping may use: the accumulators (ll, and the gradient with GRAD)
+// of all R chains live in registers next to the R Laws.
+__host__ __device__ constexpr int user_max_R(int P, bool grad) {
+    return (grad ? 2 * P + 1 : P + 1) * 4 <= 40 ? 4 : (grad ? 2 * P + 1 : P + 1) * 2 <= 40 ? 2 : 1;
+}
+
+struct UserSweepArgs {
+    const double *obs;     // [n_pad][D] row-major, n_pad = n_obs rounded up to even (zero rows)
+    int64_t n_obs;
+    const double *theta;   // [P][C] the evaluated state (proposal or current)
+    int64_t C;
+    double *ll_part;       // [S][C]
+    double *g_part;        // [S][P][C] (GRAD)
+    int32_t *err_flag;     // set when a chain's set_parameters returns false
+    int S;
+};
+
+#ifdef __CUDACC_RTC__
+template <class LawT, int P, int D, int R, int L, bool GRAD>
+__device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
+    constexpr int TR = user_tile_rows(D), ST = kUserStages;
+    constexpr int CPB = kUserNT / L * R;   // chains per CTA
+    static_assert(L == 1 || R == 1, "the lanes mapping holds one chain per warp");
+    __shared__ __align__(128) double tile[ST][TR * D];
+    __shared__ __align__(8) uint64_t bar[ST];
+    const int tid = threadIdx.x;
+    const int lane = L == 1 ? 0 : (tid & (L - 1));
+    const int seg = blockIdx.x;
+    const int64_t C = a.C;
+    const int64_t cbase = (int64_t)blockIdx.y * CPB;
+
+    // segment bounds on even rows: every bulk copy starts 16-byte aligned
+    const int64_t n_pairs = (a.n_obs + 1) >> 1;
+    const int64_t lo = 2 * ((int64_t)seg * n_pairs / a.S);
+    int64_t hi = 2 * ((int64_t)(seg + 1) * n_pairs / a.S);
+    if (hi > a.n_obs) hi = a.n_obs;
+    const int64_t len = hi - lo;
+    const int n_tiles = (int)((len + TR - 1) / TR);
+
+    if (tid == 0) {
+#pragma unroll
+        for (int s = 0; s < ST; ++s) mbar_init(&bar[s], 1);
+        mbar_fence_init();
+    }
+    __syncthreads();
+    auto issue = [&](int t) {
+        const int st = t % ST;
+        const int64_t off = (int64_t)t * TR;
+        const int cnt = (int)((len - off) < (int64_t)TR ? (len - off) : (int64_t)TR);
+        const uint32_t bytes = (uint32_t)((cnt + 1) >> 1) * (16u * D);   // pairs of rows
+        mbar_expect_tx(&bar[st], bytes);
+        bulk_g2s(&tile[st][0], a.obs + (lo + off) * D, bytes, &bar[st]);
+    };
+    if (tid == 0)
+        for (int t = 0; t < ST && t < n_tiles; ++t) issue(t);
+
+    // Only the (constant) observations were touched so far.  The evaluated state is written by the
+    // preceding step kernel: wait for it, then let our own successor's prologue start.
+    griddep_wait();
+    griddep_launch_dependents();
+
+    LawT law[R];
+    bool ok[R];
+    double acc[R];
+    double g[GRAD ? R : 1][GRAD ? P : 1];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
+        double th[P];
+#pragma unroll
+        for (int k = 0; k < P; ++k) th[k] = c < C ? a.theta[(int64_t)k * C + c] : 0.0;
+        ok[r] = c < C && set_parameters(law[r], th);
+        acc[r] = 0.0;
+        if (GRAD) {
+#pragma unroll
+            for (int k = 0; k < P; ++k) g[r][k] = 0.0;
+        }
+    }
+
+    for (int t = 0; t < n_tiles; ++t) {
+        const int st = t % ST;
+        mbar_wait(&bar[st], (uint32_t)(t / ST) & 1u);
+        const int64_t off = (int64_t)t * TR;
+        // rows beyond the segment (and the zero padding) never reach logpdf
+        const int cnt = (int)((len - off) < (int64_t)TR ? (len - off) : (int64_t)TR);
+        const double *xs = &tile[st][0];
+#pragma unroll 4
+        for (int j = lane; j < cnt; j += L) {
+            const double *x = xs + j * D;
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                if (!ok[r]) continue;
+                if constexpr (GRAD) acc[r] += logpdf_grad(law[r], x, g[r]);
+                else acc[r] += logpdf(law[r], x);
+            }
+        }
+        __syncthreads();   // everyone is done with this stage before it is refilled
+        if (tid == 0 && t + ST < n_tiles) issue(t + ST);
+    }
+
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
+        double v = acc[r];
+        if (L > 1) {
+#pragma unroll
+            for (int o = L / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        }
+        if (lane == 0 && c < C) a.ll_part[(int64_t)seg * C + c] = ok[r] ? v : nan;
+        if (GRAD) {
+#pragma unroll
+            for (int k = 0; k < P; ++k) {
+                double w = g[r][k];
+                if (L > 1) {
+#pragma unroll
+                    for (int o = L / 2; o > 0; o >>= 1) w += __shfl_xor_sync(0xffffffffu, w, o);
+                }
+                if (lane == 0 && c < C) a.g_part[((int64_t)seg * P + k) * C + c] = ok[r] ? w : nan;
+            }
+        }
+        if (lane == 0 && c < C && !ok[r] && seg == 0) *a.err_flag = 1;
+    }
+}
+#endif
+
+}  // namespace extmcmc

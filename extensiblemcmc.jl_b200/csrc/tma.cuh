@@ -1,6 +1,8 @@
 // 1-D TMA bulk copy (cp.async.bulk, SASS UBLKCP) + mbarrier helpers shared by the sweeps.
 #pragma once
+#ifndef __CUDACC_RTC__   // NVRTC (user laws, user_law.cu) has no standard headers: the input defines the types
 #include <cstdint>
+#endif
 
 namespace extmcmc {
 

@@ -1,0 +1,54 @@
+"""DeviceLaw -- a user-defined target law on the device.
+
+The reference lets users bring their own law: `set_parameters!(P, θ)` and `loglikelihood(P, obs)`
+(docs/src/get_started/basic_use.md, src/example/gsn_target.jl).  Here the same two functions are
+written in CUDA C++ and compiled at run time into the likelihood sweep (csrc/sweep_user.cuh,
+csrc/user_law.cu; the contract is in include/extmcmc.h and INTEGRATION.md):
+
+    struct Law { ... };                                              // per-chain constants
+    __device__ bool   set_parameters(Law &L, const double *th);     // th[0..EXTMCMC_P-1]
+    __device__ double logpdf(const Law &L, const double *x);        // x[0..EXTMCMC_D-1], one row
+    __device__ double logpdf_grad(const Law &L, const double *x, double *g);   // gradient=True
+
+Data: dict(P=DeviceLaw(source, n_params, obs_dim), obs=rows [N, obs_dim]); responses and
+covariates are columns of the rows.  The constructor compiles the law for sm_100a (no device
+needed) and raises ValueError with the compiler's log when it does not compile.
+"""
+import ctypes as C
+
+from . import _abi
+
+
+class DeviceLaw:
+    def __init__(self, source, n_params, obs_dim=1, gradient=False):
+        self.source = str(source)
+        self._n_params = int(n_params)
+        self._obs_dim = int(obs_dim)
+        self.gradient = bool(gradient)
+        lib = _abi.load()
+        buf = C.create_string_buffer(1 << 16)
+        rc = lib.extmcmc_user_law_check(self.source.encode(), self._n_params, self._obs_dim,
+                                        1 if self.gradient else 0, buf, len(buf))
+        self.log = buf.value.decode(errors="replace")   # NVRTC + ptxas log (registers, spill bytes)
+        if rc == _abi.EINVAL:
+            raise ValueError("the device law does not compile:\n" + self.log)
+        if rc != _abi.OK:
+            raise _abi.ExtMCMCError(rc, self.log or lib.extmcmc_last_error(None).decode())
+
+    def abi_law(self):
+        return _abi.LAW_USER
+
+    @property
+    def n_params(self):
+        return self._n_params
+
+    @property
+    def obs_dim(self):
+        return self._obs_dim
+
+    def abi_y(self, data=None):
+        return None                                  # responses are columns of the rows
+
+    def abi_attach(self, lib, handle):
+        """Compiles (cached) and installs the law on a freshly created library handle."""
+        return lib.extmcmc_set_user_law(handle, self.source.encode(), 1 if self.gradient else 0)

@@ -104,7 +104,7 @@ class CUDAGlobalWorkspace(GlobalWorkspace):
         if not hasattr(law, "abi_law"):
             raise NotImplementedError(
                 f"target law {type(law).__name__} is not implemented on the GPU path "
-                "(user-defined laws cannot cross the C ABI)")
+                "(write it as a DeviceLaw: set_parameters / logpdf in CUDA C++)")
         self.backend = backend
         self.lib = lib
         self.M = int(num_mcmc_steps)
@@ -149,6 +149,8 @@ class CUDAGlobalWorkspace(GlobalWorkspace):
             msg = lib.extmcmc_last_error(None)
             raise _abi.ExtMCMCError(rc, msg.decode() if msg else "")
         try:
+            if hasattr(law, "abi_attach"):                      # DeviceLaw: compile and install the law
+                self._ck(law.abi_attach(lib, self.handle))
             if backend.comm_id is not None:
                 ida = np.frombuffer(bytes(backend.comm_id), dtype=np.uint8).copy()
                 self._ck(lib.extmcmc_comm_init(self.handle, ida.ctypes.data_as(_abi.c_uint8_p)))

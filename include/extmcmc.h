@@ -60,8 +60,10 @@ enum {
                                     (src/example/gsn_target.jl:1-29)            */
     EXTMCMC_LAW_LOGISTIC    = 3, /* Bayesian logistic regression, theta = beta[d]
                                     (no reference law; build-defined, cfg 3)    */
-    EXTMCMC_LAW_HIER_NORMAL = 4  /* hierarchical normal, theta = [theta_1..G, mu, tau]
+    EXTMCMC_LAW_HIER_NORMAL = 4, /* hierarchical normal, theta = [theta_1..G, mu, tau]
                                     (no reference law; build-defined, cfg 4)    */
+    EXTMCMC_LAW_USER        = 5  /* user-defined law: CUDA C++ source compiled at run time,
+                                    see extmcmc_set_user_law                    */
 };
 
 /* ---- transition kernels (src/transition_kernels/random_walk.jl, src/updates.jl) */
@@ -213,6 +215,7 @@ int32_t extmcmc_abi_version(void);
  * (src/workspaces.jl:229-237).  Row-major obs[n_obs][obs_dim]; y = responses (LOGISTIC)
  * or the 0-based group index of every observation, sorted ascending (HIER_NORMAL);
  * NULL otherwise.  The library copies.  n_obs >= 1 (EXTMCMC_EINVAL otherwise).
+ * (EXTMCMC_LAW_USER: rows of obs_dim columns, y = NULL.)
  * Under EXTMCMC_SHARD_OBS each rank uploads only its own slice. */
 int32_t extmcmc_upload_obs(extmcmc_t h, const double *obs, int64_t n_obs,
                            int32_t obs_dim, const double *y);
@@ -220,6 +223,41 @@ int32_t extmcmc_upload_obs(extmcmc_t h, const double *obs, int64_t n_obs,
  * global indices [first, first + n_obs) (BASELINE cfg 5: N = 1e9). */
 int32_t extmcmc_generate_obs_normal(extmcmc_t h, int64_t first, int64_t n_obs,
                                     double mean, double sd, uint64_t seed);
+/* ---- user-defined laws (EXTMCMC_LAW_USER) ----------------------------------
+ * The reference's user law -- set_parameters!(P, theta) and loglikelihood(P, obs) -- written as one
+ * string of CUDA C++ (not Julia) that defines:
+ *
+ *   struct Law { ... };   per-chain constants, kept in registers for the whole sweep
+ *   // set_parameters!(P, theta): th[0..P-1] = the chain's full parameter vector; return false when
+ *   // theta is outside the law's domain (the chain's ll is then NaN, its proposal is rejected and
+ *   // extmcmc_sync returns EXTMCMC_EDOMAIN)
+ *   __device__ bool set_parameters(Law &L, const double *th);
+ *   // one term of loglikelihood(P, obs): x[0..D-1] = one observation row
+ *   __device__ double logpdf(const Law &L, const double *x);
+ *   // optional (with_grad = 1; needed by MALA and extmcmc_eval_grad): returns logpdf and ADDS
+ *   // d logpdf / d th into g[0..P-1]
+ *   __device__ double logpdf_grad(const Law &L, const double *x, double *g);
+ *
+ * P = n_params and D = obs_dim are the macros EXTMCMC_P / EXTMCMC_D (compile-time constants).  The
+ * fixed-width integer types are defined; no header can be included.  Responses and covariates are
+ * extra columns of the observation row (extmcmc_upload_obs with y = NULL).  The law is compiled for
+ * sm_100a with -fmad=false: a law written like the reference rounds like it; write fma() where
+ * fusion is wanted.  Limits: 1 <= n_params <= 64, 1 <= obs_dim <= 64 (registers).  Not with
+ * EXTMCMC_SHARD_OBS over several ranks (EXTMCMC_EUNSUPPORTED).  Compilation needs NVRTC 12
+ * (libnvrtc.so.12, loaded on first use; every built-in law runs without it). */
+/* Compiles the law for the handle (law EXTMCMC_LAW_USER) and replaces the one it had; any time after
+ * extmcmc_create.  Invalidates the plan and the cached graphs as extmcmc_upload_obs does.
+ * EXTMCMC_EINVAL when it does not compile (extmcmc_last_error carries the NVRTC log),
+ * EXTMCMC_EUNSUPPORTED when NVRTC cannot be loaded.  A run or eval on an EXTMCMC_LAW_USER handle
+ * without a law returns EXTMCMC_EINVAL. */
+int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad);
+/* Compiles every kernel the library can pick for (n_params, obs_dim, with_grad) for sm_100a, without a
+ * handle or a device: a law that passes cannot fail to compile later (the result is cached for the
+ * process).  log (may be NULL) receives the NUL-terminated NVRTC and ptxas log (registers, spill
+ * bytes), truncated to log_bytes.  Returns EXTMCMC_OK, EXTMCMC_EINVAL or EXTMCMC_EUNSUPPORTED. */
+int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                               char *log, int64_t log_bytes);
+
 /* Replaces RandomWalkUpdate(rw, coords; prior, adpt) src/updates.jl:170-182. */
 int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd);
 /* theta[p * n_chains] chain-major SoA; replaces theta_init (src/run.jl:34-45).
@@ -246,7 +284,8 @@ int32_t extmcmc_set_lambda_fn(extmcmc_t h, int32_t u, extmcmc_lambda_fn f, void 
  * count, rolling-acceptance tags).  The RNG has no state: a resumed run continues the same Philox
  * streams, so `run 2M` and `run M, save, load into a fresh handle with the same configuration,
  * updates and observations, run M with MCMCSchedule(...; start = ...)` (src/schedule.jl:28) are
- * bit-identical.  The history ring is not part of the blob.  _load checks the shape header.
+ * bit-identical.  The history ring is not part of the blob.  _load checks the shape header (and, for
+ * EXTMCMC_LAW_USER, a hash of the compiled law: a blob of another law is refused).
  * (Gradients and the data-sum cache of HIER_NORMAL are not part of the blob either: they are
  * recomputed on demand by the kernels that produced them, to the same bits.) */
 int32_t extmcmc_checkpoint_size(extmcmc_t h, int64_t *bytes_out);
@@ -344,7 +383,8 @@ int32_t extmcmc_flush_l2(extmcmc_t h);
 int32_t extmcmc_measure_fp64_peak(extmcmc_t h, double *tflops_out);
 /* FP64 tensor-core (DMMA m8n8k4) micro-benchmark: TFLOP/s. */
 int32_t extmcmc_measure_dmma_peak(extmcmc_t h, double *tflops_out);
-/* Name of the sweep kernel variant selected for the current shapes. */
+/* Name of the sweep kernel variant selected for the current shapes (user laws: user_chains_R1/R2/R4,
+ * user_lanes). */
 const char *extmcmc_sweep_variant_name(extmcmc_t h);
 
 #ifdef __cplusplus

@@ -80,7 +80,7 @@ struct Config                     # extmcmc_config_t
 end
 
 # enumerations of the header
-const LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL = Int32(1), Int32(2), Int32(3), Int32(4)
+const LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = Int32(1), Int32(2), Int32(3), Int32(4), Int32(5)
 const KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = Int32(1), Int32(2), Int32(3), Int32(4)
 const ADAPT_NONE, ADAPT_UNIF_RW, ADAPT_HAARIO, ADAPT_MALA = Int32(0), Int32(1), Int32(2), Int32(3)
 const PRIOR_PRODUCT, PRIOR_MVNORMAL = Int32(5), Int32(11)
@@ -101,6 +101,32 @@ CUDAMCMCBackend(; n_chains=1, device=0, seed=0, block_len=128, report_chain=1) =
 struct LogisticLaw; d::Int; end
 "Hierarchical normal model, theta = [theta_1..G, mu, tau] (EXTMCMC_LAW_HIER_NORMAL); data = (P = HierNormalLaw(G), obs = y, groups = 1-based group of every observation, sorted)"
 struct HierNormalLaw; G::Int; end
+
+"""
+    DeviceLaw(source::String, n_params, obs_dim; gradient=false)
+
+A user-defined law on the device (EXTMCMC_LAW_USER): the counterparts of `set_parameters!(P, θ)` and
+one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_parameters`, `logpdf`, and
+`logpdf_grad` with `gradient = true`; contract in include/extmcmc.h and INTEGRATION.md).  Compiled for
+sm_100a when constructed (no device needed); a source that does not compile throws with the compiler's
+log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values); responses are columns of the rows.
+"""
+struct DeviceLaw
+    source::String
+    n_params::Int
+    obs_dim::Int
+    gradient::Bool
+    log::String
+    function DeviceLaw(source::String, n_params, obs_dim; gradient=false)
+        buf = zeros(UInt8, 1 << 16)
+        rc = GC.@preserve buf ccall((:extmcmc_user_law_check, LIB), Int32,
+                                    (Cstring, Int32, Int32, Int32, Ptr{UInt8}, Int64),
+                                    source, n_params, obs_dim, gradient ? 1 : 0, pointer(buf), length(buf))
+        log = unsafe_string(pointer(buf))
+        rc == 0 || throw(ArgumentError("the device law does not compile (status $rc):\n" * log))
+        new(source, n_params, obs_dim, gradient, log)
+    end
+end
 
 "MALAUpdate(tau, coords; prior, adpt): theta° = theta + tau^2/2 grad(ll + log prior)(theta) + tau z (src/updates.jl:216-218 is an empty stub)"
 struct CUDAMALAUpdate{TP,TA} <: eMCMC.MCMCGradientBasedUpdate
@@ -167,7 +193,8 @@ prior_abi(pr) = error("prior $(typeof(pr)) not implemented on the GPU path")
 law_abi(P::eMCMC.GsnTargetLaw) = length(P.P.μ) == 1 ? (LAW_GSN_IID_1D, 1) : (LAW_GSN_MV, length(P.P.μ))
 law_abi(P::LogisticLaw) = (LAW_LOGISTIC, P.d)
 law_abi(P::HierNormalLaw) = (LAW_HIER_NORMAL, 1)
-law_abi(P) = error("target law $(typeof(P)) is not implemented on the GPU path (user-defined laws cannot cross the C ABI)")
+law_abi(P::DeviceLaw) = (LAW_USER, P.obs_dim)
+law_abi(P) = error("target law $(typeof(P)) is not implemented on the GPU path (write it as a DeviceLaw: set_parameters / logpdf in CUDA C++)")
 
 # ---- transition kernels and adaptations -> (kernel id, step vector, pos flags) --------------------
 kernel_abi(rw::eMCMC.UniformRandomWalk) = (KERNEL_RW_UNIFORM, Float64.(collect(rw.ϵ)), UInt8.(collect(rw.pos)))
@@ -243,6 +270,10 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
     h = Ref{Ptr{Cvoid}}(C_NULL)
     rc = ccall((:extmcmc_create, LIB), Int32, (Ref{Config}, Ref{Ptr{Cvoid}}), cfg, h)
     rc == 0 || error("extmcmc_create: ", last_error(C_NULL))
+    if data.P isa DeviceLaw                              # compiled once per process (cached by the check)
+        check(h[], ccall((:extmcmc_set_user_law, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
+                         h[], data.P.source, data.P.gradient ? 1 : 0))
+    end
     keep = Any[]
     for (u, updt) in enumerate(updates)
         coords = Int32.(collect(updt.coords) .- 1)       # 0-based at the ABI

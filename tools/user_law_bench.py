@@ -1,0 +1,123 @@
+"""User-defined device laws against the built-in sweep, at the shape of BASELINE cfg 2 (4096 chains,
+1e6 observations, the two adaptive uniform walks of bench.py): the built-in GSN_IID_1D law and its
+DeviceLaw restatement (tests/user_laws.py) in one process, alternating, each timed step after the L2
+flush bench.py uses.  Reports ms per iteration, chain-step x observation per second, the instrumented
+sweep time per launch, the cold and cached JIT compile time, and a Poisson-regression DeviceLaw at
+d = 8 (4096 chains, 1e6 rows) in ms per iteration.  One JSON object on stdout (and in --out), with
+the card's name and power limit read in the same process.
+
+    python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--out FILE]
+"""
+import argparse
+import ctypes
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+import bench  # noqa: E402  (cfg 2 data, updates, initial state, step arrays, timed loop)
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
+
+
+def make(em, law, x, ups, th0, **bk):
+    from extensiblemcmc_jl_b200.mcmc import init_
+    mcmc = em.MCMC(ups, backend=em.CUDAMCMCBackend(n_chains=th0.shape[1], seed=3, history="none", **bk))
+    init_(mcmc, 1, dict(P=law, obs=x), th0)
+    return mcmc.workspace
+
+
+def sweep_ms(ws, _abi, K):
+    lib, h = ws.lib, ws.handle
+    msw, nl = ctypes.c_float(), ctypes.c_int64()
+    ws._ck(lib.extmcmc_run_block(h, bench.steps_for(None, _abi, 1, 5), 5 * bench.NU))
+    ws.sync()
+    ws._ck(lib.extmcmc_get_sweep_time(h, ctypes.byref(msw), ctypes.byref(nl)))
+    it = 6
+    for _ in range(K):
+        ws._ck(lib.extmcmc_flush_l2(h))
+        ws._ck(lib.extmcmc_run_block(h, bench.steps_for(None, _abi, it, 1), bench.NU))
+        it += 1
+    ws.sync()
+    ws._ck(lib.extmcmc_get_sweep_time(h, ctypes.byref(msw), ctypes.byref(nl)))
+    return msw.value / max(nl.value, 1)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--steps", type=int, default=300)
+    ap.add_argument("--warmup", type=int, default=30)
+    ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    import extensiblemcmc_jl_b200 as em
+    from extensiblemcmc_jl_b200 import _abi
+    from tests import user_laws as ul
+
+    out = {"card": card(), "workload": "BASELINE cfg 2 shape: 4096 chains x 1e6 observations, 2 adaptive uniform walks"}
+    t0 = time.perf_counter()
+    user_gsn = em.DeviceLaw(ul.GSN1D, 2, 1)              # cold: NVRTC + ptxas of every instantiation
+    out["jit_cold_s"] = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    em.DeviceLaw(ul.GSN1D, 2, 1)                         # the same input again: the process-wide cache
+    out["jit_cached_s"] = time.perf_counter() - t0
+
+    x = bench.cfg2_data()
+    C, N, NU = bench.CHAINS_PER_GPU, x.shape[0], bench.NU
+    th0 = bench.cfg2_theta_init(x, C)
+    ws = {"builtin": make(em, em.GsnTargetLaw([0.0]), x, bench.cfg2_updates(em), th0, block_len=NU),
+          "device_law": make(em, user_gsn, x[:, None], bench.cfg2_updates(em), th0, block_len=NU)}
+    out["variant"] = {k: w.lib.extmcmc_sweep_variant_name(w.handle).decode() for k, w in ws.items()}
+    times = {k: [] for k in ws}
+    for _ in range(args.reps):                           # alternating, the same warm-up each time
+        for k, w in ws.items():
+            times[k].append(bench.timed_steps(w, _abi, C, args.steps, args.warmup) / args.steps)
+    for k, w in ws.items():
+        ms = float(np.median(times[k]))
+        out[k] = {"ms_per_iter": ms, "ms_per_iter_reps": times[k],
+                  "chain_step_obs_per_s": C * NU * N / (ms * 1e-3)}
+        w.close()
+    for k, law, xx in (("builtin", em.GsnTargetLaw([0.0]), x), ("device_law", user_gsn, x[:, None])):
+        wi = make(em, law, xx, bench.cfg2_updates(em), th0, block_len=5 * NU, use_graphs=False, instrument=True)
+        out[k]["sweep_ms"] = sweep_ms(wi, _abi, args.steps // 3)
+        wi.close()
+    out["device_over_builtin"] = out["device_law"]["ms_per_iter"] / out["builtin"]["ms_per_iter"]
+
+    # Poisson regression with log link, d = 8 (intercept + 7 covariates), two uniform walks of 4 coordinates
+    d = 8
+    rng = np.random.default_rng(5)
+    X = np.empty((N, d))
+    X[:, :d - 1] = rng.standard_normal((N, d - 1)) / np.sqrt(d - 1)
+    beta = 0.3 * rng.standard_normal(d)
+    X[:, d - 1] = rng.poisson(np.exp(beta[0] + X[:, :d - 1] @ beta[1:]))
+    ups = [em.RandomWalkUpdate(em.UniformRandomWalk([1e-3] * 4), [1, 2, 3, 4]),
+           em.RandomWalkUpdate(em.UniformRandomWalk([1e-3] * 4), [5, 6, 7, 8])]
+    thp = beta[:, None] + 1e-3 * rng.standard_normal((d, C))
+    t0 = time.perf_counter()
+    preg = em.DeviceLaw(ul.POISSON_REG, d, d)
+    jit = time.perf_counter() - t0
+    wp = make(em, preg, X, ups, thp, block_len=NU)
+    tp = [bench.timed_steps(wp, _abi, C, args.steps, args.warmup) / args.steps for _ in range(args.reps)]
+    out["poisson_reg_d8"] = {"ms_per_iter": float(np.median(tp)), "ms_per_iter_reps": tp, "jit_cold_s": jit,
+                             "variant": wp.lib.extmcmc_sweep_variant_name(wp.handle).decode(),
+                             "chain_step_obs_per_s": C * NU * N / (float(np.median(tp)) * 1e-3)}
+    wp.close()
+    line = json.dumps(out)
+    print(line)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
+
+
+if __name__ == "__main__":
+    main()
