@@ -33,6 +33,26 @@ def test_sample_laws_compile_without_spills(name, P, D):
     assert "sm_100a" in log
 
 
+# the 64 x 64 shape limit (kUserMaxParams = kUserMaxObsDim = 64), with the gradient.  Known cost: the
+# gradient kernels spill (theta, the Law and the gradient do not fit the 255 registers of a thread;
+# ~1 KB of spill stores, ~3 KB of loads); the plain kernels do not.  The values are checked on the
+# device in test_gpu_user_law_kernels.py::test_shape_limit_64.
+@pytest.mark.parametrize("name,P,D", [("poisson_reg", 64, 64), ("logistic", 63, 64)])
+def test_sample_laws_compile_at_the_shape_limit(name, P, D):
+    rc, log = _check(ul.LAWS[name][0], P, D, True)
+    assert rc == _abi.OK, log
+    blocks = re.findall(r"Compiling entry function '(extmcmc_user_\w+)'.*?(\d+) bytes spill stores, (\d+) bytes spill loads",
+                        log, re.S)
+    spills = {k: (int(st), int(ld)) for k, st, ld in blocks}
+    # P = 64: the accumulators of even one extra chain per thread do not fit, R = 1 only
+    assert set(spills) == {"extmcmc_user_chains_r1_g0", "extmcmc_user_chains_r1_g1",
+                           "extmcmc_user_lanes_g0", "extmcmc_user_lanes_g1"}, log
+    for k, s in spills.items():
+        if k.endswith("_g0"):
+            assert s == (0, 0), (k, s)
+    assert "sm_100a" in log
+
+
 def test_law_without_gradient_compiles_only_the_plain_kernels():
     rc, log = _check(ul.POISSON_RATE, 1, 1, False)
     assert rc == _abi.OK, log

@@ -1,5 +1,6 @@
 """Sources of the device laws the user-law tests and tools/user_law_bench.py use (CUDA C++, the
-contract of include/extmcmc.h), with numpy fp64 references of their per-row terms and gradients."""
+contract of include/extmcmc.h), with numpy references of their per-row terms and gradients (fp64 by
+default; dtype=np.longdouble gives the extended-precision reference)."""
 import numpy as np
 
 LOG2PI = 1.8378770664093453
@@ -91,8 +92,9 @@ __device__ double logpdf(const Law &L, const double *x) {
 """
 
 
-def gsn1d_terms(theta, X):
+def gsn1d_terms(theta, X, dtype=np.float64):
     """[N, C] per-row log-densities and [P, N, C] gradients; theta [2, C], X [N, 1]."""
+    theta, X = np.asarray(theta, dtype), np.asarray(X, dtype)
     mu, var = theta[0][None, :], theta[1][None, :]
     d = X[:, :1] - mu
     t = -(LOG2PI + np.log(var)) / 2.0 - d * d / (2.0 * var)
@@ -100,7 +102,8 @@ def gsn1d_terms(theta, X):
     return t, g
 
 
-def logistic_terms(theta, X):
+def logistic_terms(theta, X, dtype=np.float64):
+    theta, X = np.asarray(theta, dtype), np.asarray(X, dtype)
     P = theta.shape[0]
     e = X[:, :P] @ theta
     y = X[:, P:P + 1]
@@ -110,7 +113,8 @@ def logistic_terms(theta, X):
     return t, g
 
 
-def poisson_reg_terms(theta, X):
+def poisson_reg_terms(theta, X, dtype=np.float64):
+    theta, X = np.asarray(theta, dtype), np.asarray(X, dtype)
     P = theta.shape[0]
     e = theta[0][None, :] + X[:, :P - 1] @ theta[1:]
     y = X[:, P - 1:P]
