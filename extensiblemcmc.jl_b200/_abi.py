@@ -17,6 +17,7 @@ ABI_VERSION = 2
 OK, EINVAL, EUNSUPPORTED, ECUDA, ENCCL, EOOM, EDOMAIN, ESTALE = 0, -1, -2, -3, -4, -5, -6, -7
 # laws
 LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = 1, 2, 3, 4, 5
+USER_GRAD_NONE, USER_GRAD_HAND, USER_GRAD_FORWARD = 0, 1, 2
 # kernels
 KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = 1, 2, 3, 4
 # priors

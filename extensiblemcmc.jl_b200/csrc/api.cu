@@ -580,7 +580,7 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
         return fail(h, EXTMCMC_EINVAL, "block longer than history_window");
     if (obs_sharded(h) && !h->comm) return fail(h, EXTMCMC_EINVAL, "EXTMCMC_SHARD_OBS needs extmcmc_comm_init first");
     if (h->cfg.law == EXTMCMC_LAW_USER && h->any_mala && h->ulaw.loaded && !h->ulaw.grad)
-        return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with logpdf_grad (extmcmc_set_user_law with_grad = 1)");
+        return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with a gradient (extmcmc_set_user_law with_grad = 1 or 2)");
     for (int s = 0; s < n_steps; ++s)
         if (steps[s].pidx < 0 || steps[s].pidx >= h->cfg.n_updates || steps[s].mcmciter < 1)
             return fail(h, EXTMCMC_EINVAL, "step out of range");
@@ -1118,7 +1118,7 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
             h->cfg.law != EXTMCMC_LAW_LOGISTIC && h->cfg.law != EXTMCMC_LAW_USER)
             return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a law with a device gradient (GSN_IID_1D, HIER_NORMAL, LOGISTIC, USER)");
         if (h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.loaded && !h->ulaw.grad)
-            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with logpdf_grad (extmcmc_set_user_law with_grad = 1)");
+            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with a gradient (extmcmc_set_user_law with_grad = 1 or 2)");
         if (upd->prior != EXTMCMC_PRIOR_IMPROPER && upd->prior != EXTMCMC_PRIOR_NORMAL)
             return fail(h, EXTMCMC_EUNSUPPORTED, "MALA supports ImproperPrior and Normal priors only");
         if (upd->pos)
@@ -1334,14 +1334,38 @@ int32_t extmcmc_set_state(extmcmc_t h, const double *theta) {
     return EXTMCMC_OK;
 }
 
+}  // extern "C"
+namespace {
+// with_grad of the C ABI -> UserGrad: EXTMCMC_USER_GRAD_FORWARD, or any other non-zero value: hand-written
+int user_grad_mode(int32_t with_grad) {
+    return with_grad == EXTMCMC_USER_GRAD_FORWARD ? kUserGradForward : with_grad ? kUserGradHand : kUserValue;
+}
+std::string forward_limit_message(int32_t n_params) {
+    return "forward-mode gradients (with_grad = EXTMCMC_USER_GRAD_FORWARD) need 1 <= n_params <= " +
+           std::to_string(kUserMaxForwardParams) + " (every parameter-dependent field of the Law holds n_params + 1 "
+           "doubles in registers); got n_params = " + std::to_string(n_params) + ": write logpdf_grad (with_grad = 1)";
+}
+}  // namespace
+extern "C" {
+
 int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                char *log, int64_t log_bytes) {
     if (log && log_bytes > 0) log[0] = 0;
     if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
     if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
         return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
+    const int mode = user_grad_mode(with_grad);
+    if (mode == kUserGradForward && n_params > kUserMaxForwardParams) {
+        const std::string msg = forward_limit_message(n_params);
+        if (log && log_bytes > 0) {
+            const size_t n = std::min(msg.size(), (size_t)log_bytes - 1);
+            std::memcpy(log, msg.data(), n);
+            log[n] = 0;
+        }
+        return fail(nullptr, EXTMCMC_EUNSUPPORTED, msg);
+    }
     std::string lg, cubin;
-    const int32_t rc = user_law_compile(source, n_params, obs_dim, with_grad != 0, lg, cubin, nullptr);
+    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, lg, cubin, nullptr);
     if (log && log_bytes > 0) {
         const size_t n = std::min(lg.size(), (size_t)log_bytes - 1);
         std::memcpy(log, lg.data(), n);
@@ -1355,15 +1379,18 @@ int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad)
     if (!h) return EXTMCMC_EINVAL;
     if (h->cfg.law != EXTMCMC_LAW_USER) return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_law needs a handle of law EXTMCMC_LAW_USER");
     if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
+    const int mode = user_grad_mode(with_grad);
+    if (mode == kUserGradForward && h->cfg.n_params > kUserMaxForwardParams)
+        return fail(h, EXTMCMC_EUNSUPPORTED, forward_limit_message(h->cfg.n_params));
     std::string log, cubin;
     uint64_t hash = 0;
-    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, with_grad != 0, log, cubin, &hash);
+    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, log, cubin, &hash);
     if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
     if (rc) return fail(h, rc, log);
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
     invalidate_graphs(h);
-    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, with_grad != 0, hash);
+    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, mode, hash);
     if (e != cudaSuccess) {
         user_law_unload(h->ulaw);
         return fail(h, EXTMCMC_ECUDA, std::string("loading the user law: ") + cudaGetErrorString(e));

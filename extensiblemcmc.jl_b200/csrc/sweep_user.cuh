@@ -1,6 +1,7 @@
 // Likelihood sweep of a user-defined law (EXTMCMC_LAW_USER): the kernel template that NVRTC
-// instantiates at run time around the user's `Law`, `set_parameters` and `logpdf` (+ `logpdf_grad`),
-// see user_law.cu and INTEGRATION.md.  nvcc compiles this header too (user_law.cu: the argument
+// instantiates at run time around the user's `Law`, `set_parameters` and `logpdf` (+ `logpdf_grad`,
+// or forward-mode derivatives of a `Law<real>` template through dual.cuh), see user_law.cu and
+// INTEGRATION.md.  nvcc compiles this header too (user_law.cu: the argument
 // struct and the shape constants the host planner shares with the kernel); the template is only
 // instantiated in the NVRTC program, where the user's functions are visible.
 //
@@ -13,10 +14,16 @@
 // Each thread accumulates its rows in order; the lanes of a chain are combined by a fixed xor-shuffle
 // tree; per-segment sums go to ll_part[S][C] and g_part[S][P][C], which the finalize kernel
 // (user_law.cu) adds in segment order.  No atomics: the result does not depend on the schedule.
+//
+// G selects what a row contributes: kUserValue calls logpdf; kUserGradHand calls the user's
+// logpdf_grad; kUserGradForward runs LawT = Law<Dual<P>>: theta enters set_parameters as duals seeded
+// with the unit vectors, so logpdf returns the row's value and its P partial derivatives, which go to
+// the same accumulators as the hand-written gradient's.
 #pragma once
 #ifndef __CUDACC_RTC__
 #include <cstdint>
 #endif
+#include "dual.cuh"
 #include "tma.cuh"
 
 namespace extmcmc {
@@ -31,10 +38,22 @@ constexpr int kUserMaxObsDim = 64;       // obs_dim of a user law (>= 16 rows pe
 // (the device buffer holds an even number of rows, zero-padded).
 __host__ __device__ constexpr int user_tile_rows(int D) { return (kUserTileDoubles / D) & ~1; }
 
+constexpr int kUserMaxForwardParams = 16;   // n_params of a forward-mode law (P + 1 doubles per field)
+
+// What a sweep computes, and how a law provides its gradient (the values of with_grad, extmcmc.h)
+enum UserGrad : int { kUserValue = 0, kUserGradHand = 1, kUserGradForward = 2 };
+
+// Doubles a thread holds per chain, for the register budget: a Law of ~P doubles and ll, plus the P
+// gradient accumulators with a gradient; under forward mode every field of the Law<Dual<P>> holds
+// P + 1 doubles: P such fields and the accumulators make (P + 1)^2.
+__host__ __device__ constexpr int user_chain_doubles(int P, int grad) {
+    return grad == kUserGradForward ? (P + 1) * (P + 1) : grad ? 2 * P + 1 : P + 1;
+}
 // Chains per thread the "chains" mapping may use: the accumulators (ll, and the gradient with GRAD)
-// of all R chains live in registers next to the R Laws.
-__host__ __device__ constexpr int user_max_R(int P, bool grad) {
-    return (grad ? 2 * P + 1 : P + 1) * 4 <= 40 ? 4 : (grad ? 2 * P + 1 : P + 1) * 2 <= 40 ? 2 : 1;
+// of all R chains live in registers next to the R Laws.  grad: a UserGrad (the kernels of a law are
+// planned for the mode it was compiled in: its value kernels run at the R of its gradient kernels).
+__host__ __device__ constexpr int user_max_R(int P, int grad) {
+    return user_chain_doubles(P, grad) * 4 <= 40 ? 4 : user_chain_doubles(P, grad) * 2 <= 40 ? 2 : 1;
 }
 
 struct UserSweepArgs {
@@ -49,8 +68,9 @@ struct UserSweepArgs {
 };
 
 #ifdef __CUDACC_RTC__
-template <class LawT, int P, int D, int R, int L, bool GRAD>
+template <class LawT, int P, int D, int R, int L, int G>
 __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
+    constexpr bool GRAD = G != kUserValue;
     constexpr int TR = user_tile_rows(D), ST = kUserStages;
     constexpr int CPB = kUserNT / L * R;   // chains per CTA
     static_assert(L == 1 || R == 1, "the lanes mapping holds one chain per warp");
@@ -99,10 +119,21 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
-        double th[P];
+        if constexpr (G == kUserGradForward) {
+            Dual<P> th[P];
 #pragma unroll
-        for (int k = 0; k < P; ++k) th[k] = c < C ? a.theta[(int64_t)k * C + c] : 0.0;
-        ok[r] = c < C && set_parameters(law[r], th);
+            for (int k = 0; k < P; ++k) {
+                th[k].v = c < C ? a.theta[(int64_t)k * C + c] : 0.0;
+#pragma unroll
+                for (int j = 0; j < P; ++j) th[k].t[j] = j == k ? 1.0 : 0.0;
+            }
+            ok[r] = c < C && set_parameters(law[r], th);
+        } else {
+            double th[P];
+#pragma unroll
+            for (int k = 0; k < P; ++k) th[k] = c < C ? a.theta[(int64_t)k * C + c] : 0.0;
+            ok[r] = c < C && set_parameters(law[r], th);
+        }
         acc[r] = 0.0;
         if (GRAD) {
 #pragma unroll
@@ -123,8 +154,16 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
             for (int r = 0; r < R; ++r) {
                 if (!ok[r]) continue;
-                if constexpr (GRAD) acc[r] += logpdf_grad(law[r], x, g[r]);
-                else acc[r] += logpdf(law[r], x);
+                if constexpr (G == kUserGradForward) {
+                    const auto v = logpdf(law[r], x);
+                    acc[r] += v.v;
+#pragma unroll
+                    for (int k = 0; k < P; ++k) g[r][k] += v.t[k];
+                } else if constexpr (GRAD) {
+                    acc[r] += logpdf_grad(law[r], x, g[r]);
+                } else {
+                    acc[r] += logpdf(law[r], x);
+                }
             }
         }
         __syncthreads();   // everyone is done with this stage before it is refilled

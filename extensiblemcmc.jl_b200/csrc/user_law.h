@@ -10,25 +10,27 @@
 
 namespace extmcmc {
 
-// Compiles every instantiation the planner can pick for (P, D, grad) to an sm_100a cubin, or takes it
-// from the process-wide cache keyed by the exact NVRTC input.  log: NVRTC + ptxas log.  Returns
+// Compiles every instantiation the planner can pick for (P, D, mode) to an sm_100a cubin, or takes it
+// from the process-wide cache keyed by the exact NVRTC input.  mode: a UserGrad (sweep_user.cuh; the
+// caller checks P <= kUserMaxForwardParams for kUserGradForward).  log: NVRTC + ptxas log.  Returns
 // EXTMCMC_OK, EXTMCMC_EINVAL (the source does not compile) or EXTMCMC_EUNSUPPORTED (no NVRTC).
-int32_t user_law_compile(const char *source, int P, int D, bool grad, std::string &log, std::string &cubin,
+int32_t user_law_compile(const char *source, int P, int D, int mode, std::string &log, std::string &cubin,
                          uint64_t *input_hash);
 
 struct UserLaw {
     bool loaded = false;
-    bool grad = false;
+    bool grad = false;                      // the law has gradient kernels (mode != kUserValue)
+    int mode = kUserValue;                  // UserGrad: how they compute it
     int P = 0, D = 0;
     uint64_t hash = 0;                      // FNV-1a of the NVRTC input (checkpoint blobs record it)
     cudaLibrary_t lib = nullptr;
-    cudaKernel_t chains[3][2] = {};         // [R = 1, 2, 4][GRAD]
+    cudaKernel_t chains[3][2] = {};         // [R = 1, 2, 4][GRAD] (GRAD: hand-written or forward mode)
     cudaKernel_t lanes[2] = {};             // [GRAD]
     int occ_chains[3] = {1, 1, 1}, occ_lanes = 1;   // resident CTAs per SM
 };
 
 // Loads the cubin into u (replacing what u held).  Returns a CUDA error.
-cudaError_t user_law_load(UserLaw &u, const std::string &cubin, int P, int D, bool grad, uint64_t hash);
+cudaError_t user_law_load(UserLaw &u, const std::string &cubin, int P, int D, int mode, uint64_t hash);
 void user_law_unload(UserLaw &u);
 
 SweepPlan plan_sweep_user(const UserLaw &u, int64_t C, int64_t n_obs, int force_variant, int num_sms);

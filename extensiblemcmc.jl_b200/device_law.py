@@ -10,6 +10,13 @@ csrc/user_law.cu; the contract is in include/extmcmc.h and INTEGRATION.md):
     __device__ double logpdf(const Law &L, const double *x);        // x[0..EXTMCMC_D-1], one row
     __device__ double logpdf_grad(const Law &L, const double *x, double *g);   // gradient=True
 
+With gradient="forward" the law is written once, generic over its scalar, and the library derives the
+gradient in forward mode (dual numbers, csrc/dual.cuh; at most 16 parameters):
+
+    template <class real> struct Law { real b[EXTMCMC_P]; };
+    template <class real> __device__ bool set_parameters(Law<real> &L, const real *th);
+    template <class real> __device__ real logpdf(const Law<real> &L, const double *x);
+
 Data: dict(P=DeviceLaw(source, n_params, obs_dim), obs=rows [N, obs_dim]); responses and
 covariates are columns of the rows.  The constructor compiles the law for sm_100a (no device
 needed) and raises ValueError with the compiler's log when it does not compile.
@@ -21,14 +28,21 @@ from . import _abi
 
 class DeviceLaw:
     def __init__(self, source, n_params, obs_dim=1, gradient=False):
+        """gradient: False (none), True (the source defines logpdf_grad) or "forward"."""
+        if isinstance(gradient, str) and gradient == "forward":
+            self._with_grad = _abi.USER_GRAD_FORWARD
+        elif isinstance(gradient, (bool, int)) and gradient in (False, True):
+            self._with_grad = _abi.USER_GRAD_HAND if gradient else _abi.USER_GRAD_NONE
+        else:
+            raise ValueError(f"gradient must be False, True or 'forward', not {gradient!r}")
         self.source = str(source)
         self._n_params = int(n_params)
         self._obs_dim = int(obs_dim)
-        self.gradient = bool(gradient)
+        self.gradient = "forward" if self._with_grad == _abi.USER_GRAD_FORWARD else bool(gradient)
         lib = _abi.load()
         buf = C.create_string_buffer(1 << 16)
         rc = lib.extmcmc_user_law_check(self.source.encode(), self._n_params, self._obs_dim,
-                                        1 if self.gradient else 0, buf, len(buf))
+                                        self._with_grad, buf, len(buf))
         self.log = buf.value.decode(errors="replace")   # NVRTC + ptxas log (registers, spill bytes)
         if rc == _abi.EINVAL:
             raise ValueError("the device law does not compile:\n" + self.log)
@@ -51,4 +65,4 @@ class DeviceLaw:
 
     def abi_attach(self, lib, handle):
         """Compiles (cached) and installs the law on a freshly created library handle."""
-        return lib.extmcmc_set_user_law(handle, self.source.encode(), 1 if self.gradient else 0)
+        return lib.extmcmc_set_user_law(handle, self.source.encode(), self._with_grad)

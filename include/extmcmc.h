@@ -66,6 +66,15 @@ enum {
                                     see extmcmc_set_user_law                    */
 };
 
+/* ---- how a user-defined law provides its gradient (with_grad of extmcmc_set_user_law) */
+enum {
+    EXTMCMC_USER_GRAD_NONE    = 0, /* no gradient: no MALA, no extmcmc_eval_grad            */
+    EXTMCMC_USER_GRAD_HAND    = 1, /* the source defines logpdf_grad (any other non-zero
+                                      value than EXTMCMC_USER_GRAD_FORWARD means the same)   */
+    EXTMCMC_USER_GRAD_FORWARD = 2  /* the source is generic over its scalar; the library
+                                      derives the gradient in forward mode (dual numbers)    */
+};
+
 /* ---- transition kernels (src/transition_kernels/random_walk.jl, src/updates.jl) */
 enum {
     EXTMCMC_KERNEL_RW_UNIFORM   = 1, /* UniformRandomWalk, random_walk.jl:45-94  */
@@ -238,6 +247,22 @@ int32_t extmcmc_generate_obs_normal(extmcmc_t h, int64_t first, int64_t n_obs,
  *   // d logpdf / d th into g[0..P-1]
  *   __device__ double logpdf_grad(const Law &L, const double *x, double *g);
  *
+ * Forward mode (with_grad = EXTMCMC_USER_GRAD_FORWARD): the same law written once, generic over its
+ * scalar, and no logpdf_grad -- the gradient is derived as ForwardDiff derives it from generic Julia:
+ *
+ *   template <class real> struct Law { ... };   every parameter-dependent field of type real
+ *   template <class real> __device__ bool set_parameters(Law<real> &L, const real *th);
+ *   template <class real> __device__ real logpdf(const Law<real> &L, const double *x);   // x: data
+ *
+ * Value sweeps run Law<double>; gradient sweeps run Law<extmcmc::Dual<P>>, a value and its P partial
+ * derivatives (csrc/dual.cuh), whose value parts are the very double operations of Law<double>: under
+ * -fmad=false the log-likelihood of a gradient sweep is bit-identical to the value sweep's.  Dual
+ * supports + - * / (with double operands on either side), compound assignment, comparisons (on the
+ * value), exp expm1 log log1p sqrt pow fabs fmin fmax fma sin cos tanh erf erfc normcdf, isinf isnan
+ * isfinite.  Any other function of a real (lgamma, ...) and any conversion of a real to double do not
+ * compile (EXTMCMC_EINVAL, the log names the call).  Limit: 1 <= n_params <= 16 (each real field holds
+ * n_params + 1 doubles in registers); larger is EXTMCMC_EUNSUPPORTED.
+ *
  * P = n_params and D = obs_dim are the macros EXTMCMC_P / EXTMCMC_D (compile-time constants).  The
  * fixed-width integer types are defined; no header can be included.  Responses and covariates are
  * extra columns of the observation row (extmcmc_upload_obs with y = NULL).  The law is compiled for
@@ -248,13 +273,15 @@ int32_t extmcmc_generate_obs_normal(extmcmc_t h, int64_t first, int64_t n_obs,
 /* Compiles the law for the handle (law EXTMCMC_LAW_USER) and replaces the one it had; any time after
  * extmcmc_create.  Invalidates the plan and the cached graphs as extmcmc_upload_obs does.
  * EXTMCMC_EINVAL when it does not compile (extmcmc_last_error carries the NVRTC log),
- * EXTMCMC_EUNSUPPORTED when NVRTC cannot be loaded.  A run or eval on an EXTMCMC_LAW_USER handle
- * without a law returns EXTMCMC_EINVAL. */
+ * EXTMCMC_EUNSUPPORTED when NVRTC cannot be loaded, or for a forward-mode law with n_params > 16.
+ * with_grad: EXTMCMC_USER_GRAD_*.  A run or eval on an EXTMCMC_LAW_USER handle without a law returns
+ * EXTMCMC_EINVAL. */
 int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad);
 /* Compiles every kernel the library can pick for (n_params, obs_dim, with_grad) for sm_100a, without a
  * handle or a device: a law that passes cannot fail to compile later (the result is cached for the
  * process).  log (may be NULL) receives the NUL-terminated NVRTC and ptxas log (registers, spill
- * bytes), truncated to log_bytes.  Returns EXTMCMC_OK, EXTMCMC_EINVAL or EXTMCMC_EUNSUPPORTED. */
+ * bytes), truncated to log_bytes.  Returns EXTMCMC_OK, EXTMCMC_EINVAL or EXTMCMC_EUNSUPPORTED (the log
+ * then says why). */
 int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                char *log, int64_t log_bytes);
 

@@ -84,6 +84,7 @@ const LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = Int3
 const KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = Int32(1), Int32(2), Int32(3), Int32(4)
 const ADAPT_NONE, ADAPT_UNIF_RW, ADAPT_HAARIO, ADAPT_MALA = Int32(0), Int32(1), Int32(2), Int32(3)
 const PRIOR_PRODUCT, PRIOR_MVNORMAL = Int32(5), Int32(11)
+const USER_GRAD_NONE, USER_GRAD_HAND, USER_GRAD_FORWARD = Int32(0), Int32(1), Int32(2)
 
 # ---- backend, build-defined laws and the MALA update (an empty stub in the reference) ------------
 struct CUDAMCMCBackend <: eMCMC.MCMCBackend
@@ -107,24 +108,31 @@ struct HierNormalLaw; G::Int; end
 
 A user-defined law on the device (EXTMCMC_LAW_USER): the counterparts of `set_parameters!(P, θ)` and
 one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_parameters`, `logpdf`, and
-`logpdf_grad` with `gradient = true`; contract in include/extmcmc.h and INTEGRATION.md).  Compiled for
-sm_100a when constructed (no device needed); a source that does not compile throws with the compiler's
-log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values); responses are columns of the rows.
+`logpdf_grad` with `gradient = true`; contract in include/extmcmc.h and INTEGRATION.md).  With
+`gradient = :forward` the law is written generic over its scalar (`template <class real> struct Law`,
+`set_parameters`, `logpdf`) and the gradient is derived in forward mode, as ForwardDiff would (at most
+16 parameters).  Compiled for sm_100a when constructed (no device needed); a source that does not
+compile throws with the compiler's log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values);
+responses are columns of the rows.
 """
 struct DeviceLaw
     source::String
     n_params::Int
     obs_dim::Int
-    gradient::Bool
+    with_grad::Int32                                     # USER_GRAD_NONE / _HAND / _FORWARD
     log::String
     function DeviceLaw(source::String, n_params, obs_dim; gradient=false)
+        with_grad = gradient === :forward ? USER_GRAD_FORWARD :
+                    gradient === true ? USER_GRAD_HAND :
+                    gradient === false ? USER_GRAD_NONE :
+                    throw(ArgumentError("gradient must be false, true or :forward, not $(repr(gradient))"))
         buf = zeros(UInt8, 1 << 16)
         rc = GC.@preserve buf ccall((:extmcmc_user_law_check, LIB), Int32,
                                     (Cstring, Int32, Int32, Int32, Ptr{UInt8}, Int64),
-                                    source, n_params, obs_dim, gradient ? 1 : 0, pointer(buf), length(buf))
+                                    source, n_params, obs_dim, with_grad, pointer(buf), length(buf))
         log = unsafe_string(pointer(buf))
         rc == 0 || throw(ArgumentError("the device law does not compile (status $rc):\n" * log))
-        new(source, n_params, obs_dim, gradient, log)
+        new(source, n_params, obs_dim, with_grad, log)
     end
 end
 
@@ -272,7 +280,7 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
     rc == 0 || error("extmcmc_create: ", last_error(C_NULL))
     if data.P isa DeviceLaw                              # compiled once per process (cached by the check)
         check(h[], ccall((:extmcmc_set_user_law, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
-                         h[], data.P.source, data.P.gradient ? 1 : 0))
+                         h[], data.P.source, data.P.with_grad))
     end
     keep = Any[]
     for (u, updt) in enumerate(updates)

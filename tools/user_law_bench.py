@@ -3,10 +3,14 @@
 DeviceLaw restatement (tests/user_laws.py) in one process, alternating, each timed step after the L2
 flush bench.py uses.  Reports ms per iteration, chain-step x observation per second, the instrumented
 sweep time per launch, the cold and cached JIT compile time, and a Poisson-regression DeviceLaw at
-d = 8 (4096 chains, 1e6 rows) in ms per iteration.  One JSON object on stdout (and in --out), with
-the card's name and power limit read in the same process.
+d = 8 (4096 chains, 1e6 rows) in ms per iteration.  The forward arm runs MALA on the same Poisson
+regression (two MALA updates of 4 coordinates) with the hand-written gradient (tests/user_laws.py)
+and with forward-mode gradients (tests/user_laws_forward.py), alternating: ms per iteration and
+gradient-sweep ms per launch of each.  One JSON object on stdout (and in --out), with the card's name
+and power limit read in the same process.
 
-    python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--out FILE]
+    python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--forward-only]
+                                   [--forward-steps 30] [--out FILE]
 """
 import argparse
 import ctypes
@@ -58,13 +62,66 @@ def main():
     ap.add_argument("--steps", type=int, default=300)
     ap.add_argument("--warmup", type=int, default=30)
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--forward-steps", type=int, default=30, help="timed steps of each forward-arm rep")
+    ap.add_argument("--forward-only", action="store_true", help="only the forward arm")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import extensiblemcmc_jl_b200 as em
     from extensiblemcmc_jl_b200 import _abi
     from tests import user_laws as ul
 
-    out = {"card": card(), "workload": "BASELINE cfg 2 shape: 4096 chains x 1e6 observations, 2 adaptive uniform walks"}
+    out = {"card": card()}
+    if not args.forward_only:
+        builtin_arms(args, em, _abi, ul, out)
+    forward_arm(args, em, _abi, out)
+    line = json.dumps(out)
+    print(line)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
+
+
+def poisson_problem(em, N, C, d=8):
+    """Poisson regression with log link, d = 8 (intercept + 7 covariates): rows, true beta, initial state."""
+    rng = np.random.default_rng(5)
+    X = np.empty((N, d))
+    X[:, :d - 1] = rng.standard_normal((N, d - 1)) / np.sqrt(d - 1)
+    beta = 0.3 * rng.standard_normal(d)
+    X[:, d - 1] = rng.poisson(np.exp(beta[0] + X[:, :d - 1] @ beta[1:]))
+    thp = beta[:, None] + 1e-3 * rng.standard_normal((d, C))
+    return X, thp
+
+
+def forward_arm(args, em, _abi, out):
+    from tests import user_laws as ul
+    from tests import user_laws_forward as uf
+    d, C, N = 8, bench.CHAINS_PER_GPU, 1_000_000
+    X, thp = poisson_problem(em, N, C, d)
+    ups = lambda: [em.MALAUpdate(1e-3, [1, 2, 3, 4]), em.MALAUpdate(1e-3, [5, 6, 7, 8])]   # noqa: E731
+    laws = {"hand": em.DeviceLaw(ul.POISSON_REG, d, d, gradient=True),
+            "forward": em.DeviceLaw(uf.POISSON_REG, d, d, gradient="forward")}
+    res = {"workload": "Poisson regression d = 8, 4096 chains x 1e6 rows, 2 MALA updates of 4 coordinates "
+                       "(one gradient sweep each per iteration)"}
+    ws = {k: make(em, law, X, ups(), thp, block_len=bench.NU) for k, law in laws.items()}
+    times = {k: [] for k in ws}
+    for _ in range(args.reps):                           # alternating, the same warm-up each time
+        for k, w in ws.items():
+            times[k].append(bench.timed_steps(w, _abi, C, args.forward_steps, 3) / args.forward_steps)
+    for k, w in ws.items():
+        res[k] = {"ms_per_iter": float(np.median(times[k])), "ms_per_iter_reps": times[k],
+                  "variant": w.lib.extmcmc_sweep_variant_name(w.handle).decode()}
+        w.close()
+    for k, law in laws.items():
+        wi = make(em, law, X, ups(), thp, block_len=5 * bench.NU, use_graphs=False, instrument=True)
+        res[k]["grad_sweep_ms"] = sweep_ms(wi, _abi, max(args.forward_steps // 3, 3))
+        wi.close()
+    res["forward_over_hand_iter"] = res["forward"]["ms_per_iter"] / res["hand"]["ms_per_iter"]
+    res["forward_over_hand_sweep"] = res["forward"]["grad_sweep_ms"] / res["hand"]["grad_sweep_ms"]
+    out["poisson_reg_d8_mala"] = res
+
+
+def builtin_arms(args, em, _abi, ul, out):
+    out["workload"] = "BASELINE cfg 2 shape: 4096 chains x 1e6 observations, 2 adaptive uniform walks"
     t0 = time.perf_counter()
     user_gsn = em.DeviceLaw(ul.GSN1D, 2, 1)              # cold: NVRTC + ptxas of every instantiation
     out["jit_cold_s"] = time.perf_counter() - t0
@@ -95,14 +152,9 @@ def main():
 
     # Poisson regression with log link, d = 8 (intercept + 7 covariates), two uniform walks of 4 coordinates
     d = 8
-    rng = np.random.default_rng(5)
-    X = np.empty((N, d))
-    X[:, :d - 1] = rng.standard_normal((N, d - 1)) / np.sqrt(d - 1)
-    beta = 0.3 * rng.standard_normal(d)
-    X[:, d - 1] = rng.poisson(np.exp(beta[0] + X[:, :d - 1] @ beta[1:]))
+    X, thp = poisson_problem(em, N, C, d)
     ups = [em.RandomWalkUpdate(em.UniformRandomWalk([1e-3] * 4), [1, 2, 3, 4]),
            em.RandomWalkUpdate(em.UniformRandomWalk([1e-3] * 4), [5, 6, 7, 8])]
-    thp = beta[:, None] + 1e-3 * rng.standard_normal((d, C))
     t0 = time.perf_counter()
     preg = em.DeviceLaw(ul.POISSON_REG, d, d)
     jit = time.perf_counter() - t0
@@ -112,11 +164,6 @@ def main():
                              "variant": wp.lib.extmcmc_sweep_variant_name(wp.handle).decode(),
                              "chain_step_obs_per_s": C * NU * N / (float(np.median(tp)) * 1e-3)}
     wp.close()
-    line = json.dumps(out)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as f:
-            f.write(line + "\n")
 
 
 if __name__ == "__main__":
