@@ -110,6 +110,9 @@ SIGNATURES = {
     "extmcmc_generate_obs_normal": (C.c_int32, [Handle, C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_uint64]),
     "extmcmc_set_user_law": (C.c_int32, [Handle, C.c_char_p, C.c_int32]),
     "extmcmc_user_law_check": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_char_p, C.c_int64]),
+    "extmcmc_set_user_law_chunked": (C.c_int32, [Handle, C.c_char_p, C.c_int32]),
+    "extmcmc_user_law_check_chunked": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32,
+                                                   C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "extmcmc_set_update": (C.c_int32, [Handle, C.c_int32, C.POINTER(Update)]),
     "extmcmc_set_state": (C.c_int32, [Handle, c_double_p]),
     "extmcmc_set_seed": (C.c_int32, [Handle, C.c_uint64]),

@@ -444,7 +444,7 @@ int32_t enqueue_sweep(extmcmc_t h, bool instrument, bool grad = false, const dou
         a.ll_part = h->d.partial; a.g_part = h->d.partial + (size_t)h->plan.S * h->d.C;
         a.err_flag = h->d.err_flag; a.S = h->plan.S;
         CK(h, launch_sweep_user(h->plan, h->ulaw, a, grad, ll_dst, grad_dst, h->stream));
-        h->launches += h->plan.launches;
+        h->launches += user_sweep_launches(h->ulaw, grad);
         if (instrument) {
             CK(h, cudaEventRecord(ev.second, h->stream));
             h->ev_pending.push_back(ev);
@@ -1343,7 +1343,43 @@ int user_grad_mode(int32_t with_grad) {
 std::string forward_limit_message(int32_t n_params) {
     return "forward-mode gradients (with_grad = EXTMCMC_USER_GRAD_FORWARD) need 1 <= n_params <= " +
            std::to_string(kUserMaxForwardParams) + " (every parameter-dependent field of the Law holds n_params + 1 "
-           "doubles in registers); got n_params = " + std::to_string(n_params) + ": write logpdf_grad (with_grad = 1)";
+           "doubles in registers); got n_params = " + std::to_string(n_params) + ": write logpdf_grad (with_grad = 1).  The chunked entry points (extmcmc_set_user_law_chunked, "
+           "extmcmc_user_law_check_chunked) take forward-mode laws of up to 64 parameters.";
+}
+void copy_log(const std::string &msg, char *log, int64_t log_bytes) {
+    if (log && log_bytes > 0) {
+        const size_t n = std::min(msg.size(), (size_t)log_bytes - 1);
+        std::memcpy(log, msg.data(), n);
+        log[n] = 0;
+    }
+}
+// extmcmc_user_law_check and its chunked form; K: the resolved chunk width of forward mode
+int32_t user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int mode, int K, char *log,
+                       int64_t log_bytes) {
+    std::string lg, cubin;
+    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, K, lg, cubin, nullptr);
+    copy_log(lg, log, log_bytes);
+    if (rc) g_create_error = lg;
+    return rc;
+}
+// extmcmc_set_user_law and its chunked form
+int32_t set_user_law(extmcmc_t h, const char *source, int mode, int K) {
+    std::string log, cubin;
+    uint64_t hash = 0;
+    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, K, log, cubin, &hash);
+    if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
+    if (rc) return fail(h, rc, log);
+    CK(h, cudaSetDevice(h->cfg.device));
+    CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
+    invalidate_graphs(h);
+    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, mode, K, hash);
+    if (e != cudaSuccess) {
+        user_law_unload(h->ulaw);
+        return fail(h, EXTMCMC_ECUDA, std::string("loading the user law: ") + cudaGetErrorString(e));
+    }
+    h->plan_valid = false;
+    h->grad_valid = false;
+    return EXTMCMC_OK;
 }
 }  // namespace
 extern "C" {
@@ -1357,22 +1393,26 @@ int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs
     const int mode = user_grad_mode(with_grad);
     if (mode == kUserGradForward && n_params > kUserMaxForwardParams) {
         const std::string msg = forward_limit_message(n_params);
-        if (log && log_bytes > 0) {
-            const size_t n = std::min(msg.size(), (size_t)log_bytes - 1);
-            std::memcpy(log, msg.data(), n);
-            log[n] = 0;
-        }
+        copy_log(msg, log, log_bytes);
         return fail(nullptr, EXTMCMC_EUNSUPPORTED, msg);
     }
-    std::string lg, cubin;
-    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, lg, cubin, nullptr);
-    if (log && log_bytes > 0) {
-        const size_t n = std::min(lg.size(), (size_t)log_bytes - 1);
-        std::memcpy(log, lg.data(), n);
-        log[n] = 0;
+    return user_law_check(source, n_params, obs_dim, mode, n_params, log, log_bytes);
+}
+
+int32_t extmcmc_user_law_check_chunked(const char *source, int32_t n_params, int32_t obs_dim, int32_t chunk,
+                                       int32_t *chunk_used, char *log, int64_t log_bytes) {
+    if (log && log_bytes > 0) log[0] = 0;
+    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
+    if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
+        return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
+    int K = 0;
+    std::string err;
+    if (user_law_chunk(n_params, chunk, K, err)) {
+        copy_log(err, log, log_bytes);
+        return fail(nullptr, EXTMCMC_EINVAL, err);
     }
-    if (rc) g_create_error = lg;
-    return rc;
+    if (chunk_used) *chunk_used = K;
+    return user_law_check(source, n_params, obs_dim, kUserGradForward, K, log, log_bytes);
 }
 
 int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad) {
@@ -1382,22 +1422,18 @@ int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad)
     const int mode = user_grad_mode(with_grad);
     if (mode == kUserGradForward && h->cfg.n_params > kUserMaxForwardParams)
         return fail(h, EXTMCMC_EUNSUPPORTED, forward_limit_message(h->cfg.n_params));
-    std::string log, cubin;
-    uint64_t hash = 0;
-    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, log, cubin, &hash);
-    if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
-    if (rc) return fail(h, rc, log);
-    CK(h, cudaSetDevice(h->cfg.device));
-    CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
-    invalidate_graphs(h);
-    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, mode, hash);
-    if (e != cudaSuccess) {
-        user_law_unload(h->ulaw);
-        return fail(h, EXTMCMC_ECUDA, std::string("loading the user law: ") + cudaGetErrorString(e));
-    }
-    h->plan_valid = false;
-    h->grad_valid = false;
-    return EXTMCMC_OK;
+    return set_user_law(h, source, mode, h->cfg.n_params);
+}
+
+int32_t extmcmc_set_user_law_chunked(extmcmc_t h, const char *source, int32_t chunk) {
+    if (!h) return EXTMCMC_EINVAL;
+    if (h->cfg.law != EXTMCMC_LAW_USER)
+        return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_law_chunked needs a handle of law EXTMCMC_LAW_USER");
+    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
+    int K = 0;
+    std::string err;
+    if (user_law_chunk(h->cfg.n_params, chunk, K, err)) return fail(h, EXTMCMC_EINVAL, err);
+    return set_user_law(h, source, kUserGradForward, K);
 }
 
 // ---- checkpoint / resume ------------------------------------------------------------------------

@@ -16,9 +16,13 @@
 // (user_law.cu) adds in segment order.  No atomics: the result does not depend on the schedule.
 //
 // G selects what a row contributes: kUserValue calls logpdf; kUserGradHand calls the user's
-// logpdf_grad; kUserGradForward runs LawT = Law<Dual<P>>: theta enters set_parameters as duals seeded
-// with the unit vectors, so logpdf returns the row's value and its P partial derivatives, which go to
-// the same accumulators as the hand-written gradient's.
+// logpdf_grad; kUserGradForward runs LawT = Law<Dual<K>>: theta enters set_parameters as duals seeded
+// with the unit vectors of coordinates [CI*K, CI*K + K), so logpdf returns the row's value and those K
+// partial derivatives, which go to the same accumulators as the hand-written gradient's.  K = P is one
+// sweep for the whole gradient; K < P is chunk CI of ceil(P/K) sweeps (ForwardDiff's chunk mode).  A
+// tangent component is the same expression whatever K is, so the chunks together produce the bits of
+// the unchunked sweep.  The chunk is a template parameter on purpose: with a compile-time seed the
+// tangents of every field copied from theta fold into immediates.
 #pragma once
 #ifndef __CUDACC_RTC__
 #include <cstdint>
@@ -38,22 +42,25 @@ constexpr int kUserMaxObsDim = 64;       // obs_dim of a user law (>= 16 rows pe
 // (the device buffer holds an even number of rows, zero-padded).
 __host__ __device__ constexpr int user_tile_rows(int D) { return (kUserTileDoubles / D) & ~1; }
 
-constexpr int kUserMaxForwardParams = 16;   // n_params of a forward-mode law (P + 1 doubles per field)
+constexpr int kUserMaxForwardParams = 16;   // n_params of an unchunked forward-mode law (P + 1 doubles per field)
+constexpr int kUserMaxChunk = 16;           // tangents per chunk of a chunked forward-mode law
+constexpr int kUserMaxChunks = 16;          // chunk sweeps per gradient (bounds the JIT)
 
 // What a sweep computes, and how a law provides its gradient (the values of with_grad, extmcmc.h)
 enum UserGrad : int { kUserValue = 0, kUserGradHand = 1, kUserGradForward = 2 };
 
 // Doubles a thread holds per chain, for the register budget: a Law of ~P doubles and ll, plus the P
-// gradient accumulators with a gradient; under forward mode every field of the Law<Dual<P>> holds
-// P + 1 doubles: P such fields and the accumulators make (P + 1)^2.
-__host__ __device__ constexpr int user_chain_doubles(int P, int grad) {
-    return grad == kUserGradForward ? (P + 1) * (P + 1) : grad ? 2 * P + 1 : P + 1;
+// gradient accumulators with a gradient; under forward mode with chunk width K every field of the
+// Law<Dual<K>> holds K + 1 doubles: P such fields and the accumulators make (P + 1)(K + 1).
+__host__ __device__ constexpr int user_chain_doubles(int P, int grad, int K) {
+    return grad == kUserGradForward ? (P + 1) * (K + 1) : grad ? 2 * P + 1 : P + 1;
 }
 // Chains per thread the "chains" mapping may use: the accumulators (ll, and the gradient with GRAD)
-// of all R chains live in registers next to the R Laws.  grad: a UserGrad (the kernels of a law are
-// planned for the mode it was compiled in: its value kernels run at the R of its gradient kernels).
-__host__ __device__ constexpr int user_max_R(int P, int grad) {
-    return user_chain_doubles(P, grad) * 4 <= 40 ? 4 : user_chain_doubles(P, grad) * 2 <= 40 ? 2 : 1;
+// of all R chains live in registers next to the R Laws.  grad: a UserGrad, K: the chunk width of forward
+// mode (the kernels of a law are planned for the mode it was compiled in: its value kernels run at the
+// R of its gradient kernels).
+__host__ __device__ constexpr int user_max_R(int P, int grad, int K) {
+    return user_chain_doubles(P, grad, K) * 4 <= 40 ? 4 : user_chain_doubles(P, grad, K) * 2 <= 40 ? 2 : 1;
 }
 
 struct UserSweepArgs {
@@ -68,9 +75,16 @@ struct UserSweepArgs {
 };
 
 #ifdef __CUDACC_RTC__
-template <class LawT, int P, int D, int R, int L, int G>
+// K, CI: chunk width and chunk index of a forward-mode sweep (LawT = Law<Dual<K>>); chunk 0 writes
+// ll_part and raises err_flag, every chunk writes only its own rows g_part[S][CI*K ..][C].
+template <class LawT, int P, int D, int R, int L, int G, int K = P, int CI = 0>
 __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
     constexpr bool GRAD = G != kUserValue;
+    constexpr bool FWD = G == kUserGradForward;
+    constexpr int NG = FWD ? K : P;          // gradient accumulators per chain
+    constexpr int K0 = FWD ? CI * K : 0;     // first coordinate they belong to
+    constexpr bool WRITE_LL = K0 == 0;
+    static_assert(K0 < P && K <= P, "chunk out of range");
     constexpr int TR = user_tile_rows(D), ST = kUserStages;
     constexpr int CPB = kUserNT / L * R;   // chains per CTA
     static_assert(L == 1 || R == 1, "the lanes mapping holds one chain per warp");
@@ -115,17 +129,17 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
     LawT law[R];
     bool ok[R];
     double acc[R];
-    double g[GRAD ? R : 1][GRAD ? P : 1];
+    double g[GRAD ? R : 1][GRAD ? NG : 1];
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
-        if constexpr (G == kUserGradForward) {
-            Dual<P> th[P];
+        if constexpr (FWD) {
+            Dual<K> th[P];
 #pragma unroll
             for (int k = 0; k < P; ++k) {
                 th[k].v = c < C ? a.theta[(int64_t)k * C + c] : 0.0;
 #pragma unroll
-                for (int j = 0; j < P; ++j) th[k].t[j] = j == k ? 1.0 : 0.0;
+                for (int j = 0; j < K; ++j) th[k].t[j] = K0 + j == k ? 1.0 : 0.0;
             }
             ok[r] = c < C && set_parameters(law[r], th);
         } else {
@@ -137,7 +151,7 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
         acc[r] = 0.0;
         if (GRAD) {
 #pragma unroll
-            for (int k = 0; k < P; ++k) g[r][k] = 0.0;
+            for (int k = 0; k < NG; ++k) g[r][k] = 0.0;
         }
     }
 
@@ -154,11 +168,11 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
             for (int r = 0; r < R; ++r) {
                 if (!ok[r]) continue;
-                if constexpr (G == kUserGradForward) {
+                if constexpr (FWD) {
                     const auto v = logpdf(law[r], x);
                     acc[r] += v.v;
 #pragma unroll
-                    for (int k = 0; k < P; ++k) g[r][k] += v.t[k];
+                    for (int k = 0; k < NG; ++k) g[r][k] += v.t[k];
                 } else if constexpr (GRAD) {
                     acc[r] += logpdf_grad(law[r], x, g[r]);
                 } else {
@@ -174,24 +188,27 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
-        double v = acc[r];
-        if (L > 1) {
+        if constexpr (WRITE_LL) {
+            double v = acc[r];
+            if (L > 1) {
 #pragma unroll
-            for (int o = L / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+                for (int o = L / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            }
+            if (lane == 0 && c < C) a.ll_part[(int64_t)seg * C + c] = ok[r] ? v : nan;
         }
-        if (lane == 0 && c < C) a.ll_part[(int64_t)seg * C + c] = ok[r] ? v : nan;
         if (GRAD) {
 #pragma unroll
-            for (int k = 0; k < P; ++k) {
+            for (int k = 0; k < NG; ++k) {
+                if (K0 + k >= P) break;   // the tangents past P of a narrower last chunk: seeded zero, not written
                 double w = g[r][k];
                 if (L > 1) {
 #pragma unroll
                     for (int o = L / 2; o > 0; o >>= 1) w += __shfl_xor_sync(0xffffffffu, w, o);
                 }
-                if (lane == 0 && c < C) a.g_part[((int64_t)seg * P + k) * C + c] = ok[r] ? w : nan;
+                if (lane == 0 && c < C) a.g_part[((int64_t)seg * P + K0 + k) * C + c] = ok[r] ? w : nan;
             }
         }
-        if (lane == 0 && c < C && !ok[r] && seg == 0) *a.err_flag = 1;
+        if (WRITE_LL && lane == 0 && c < C && !ok[r] && seg == 0) *a.err_flag = 1;
     }
 }
 #endif

@@ -17,6 +17,10 @@ gradient in forward mode (dual numbers, csrc/dual.cuh; at most 16 parameters):
     template <class real> __device__ bool set_parameters(Law<real> &L, const real *th);
     template <class real> __device__ real logpdf(const Law<real> &L, const double *x);
 
+Up to 64 parameters in forward mode with chunk="auto" or a chunk width: the gradient is then ceil(P/K)
+sweeps of K tangents each (ForwardDiff's chunk mode); the library picks K for "auto", and law.chunk
+reports the width compiled.
+
 Data: dict(P=DeviceLaw(source, n_params, obs_dim), obs=rows [N, obs_dim]); responses and
 covariates are columns of the rows.  The constructor compiles the law for sm_100a (no device
 needed) and raises ValueError with the compiler's log when it does not compile.
@@ -27,22 +31,43 @@ from . import _abi
 
 
 class DeviceLaw:
-    def __init__(self, source, n_params, obs_dim=1, gradient=False):
-        """gradient: False (none), True (the source defines logpdf_grad) or "forward"."""
+    def __init__(self, source, n_params, obs_dim=1, gradient=False, chunk=None):
+        """gradient: False (none), True (the source defines logpdf_grad) or "forward".
+        chunk (forward mode only): None (unchunked, at most 16 parameters), "auto" (the library's width)
+        or a chunk width; the library checks the width against n_params."""
         if isinstance(gradient, str) and gradient == "forward":
             self._with_grad = _abi.USER_GRAD_FORWARD
         elif isinstance(gradient, (bool, int)) and gradient in (False, True):
             self._with_grad = _abi.USER_GRAD_HAND if gradient else _abi.USER_GRAD_NONE
         else:
             raise ValueError(f"gradient must be False, True or 'forward', not {gradient!r}")
+        if chunk is not None and self._with_grad != _abi.USER_GRAD_FORWARD:
+            raise ValueError(f"chunk needs gradient='forward', not gradient={gradient!r}")
+        if chunk is None or (isinstance(chunk, str) and chunk == "auto"):
+            self._chunk_arg = None if chunk is None else 0
+        elif isinstance(chunk, int) and not isinstance(chunk, bool) and chunk >= 1:
+            self._chunk_arg = chunk
+        else:
+            raise ValueError(f"chunk must be None, 'auto' or a positive width, not {chunk!r}")
         self.source = str(source)
         self._n_params = int(n_params)
         self._obs_dim = int(obs_dim)
         self.gradient = "forward" if self._with_grad == _abi.USER_GRAD_FORWARD else bool(gradient)
+        self.chunk = None                            # forward mode: the chunk width compiled
         lib = _abi.load()
         buf = C.create_string_buffer(1 << 16)
-        rc = lib.extmcmc_user_law_check(self.source.encode(), self._n_params, self._obs_dim,
-                                        self._with_grad, buf, len(buf))
+        if self._chunk_arg is None:
+            rc = lib.extmcmc_user_law_check(self.source.encode(), self._n_params, self._obs_dim,
+                                            self._with_grad, buf, len(buf))
+            if rc == _abi.OK and self._with_grad == _abi.USER_GRAD_FORWARD:
+                self.chunk = self._n_params
+        else:
+            used = C.c_int32(0)
+            rc = lib.extmcmc_user_law_check_chunked(self.source.encode(), self._n_params, self._obs_dim,
+                                                    self._chunk_arg, C.byref(used), buf, len(buf))
+            if rc == _abi.EINVAL and used.value == 0:   # the width was refused before compiling
+                raise ValueError(buf.value.decode(errors="replace"))
+            self.chunk = used.value
         self.log = buf.value.decode(errors="replace")   # NVRTC + ptxas log (registers, spill bytes)
         if rc == _abi.EINVAL:
             raise ValueError("the device law does not compile:\n" + self.log)
@@ -65,4 +90,6 @@ class DeviceLaw:
 
     def abi_attach(self, lib, handle):
         """Compiles (cached) and installs the law on a freshly created library handle."""
+        if self._chunk_arg is not None:
+            return lib.extmcmc_set_user_law_chunked(handle, self.source.encode(), self._chunk_arg)
         return lib.extmcmc_set_user_law(handle, self.source.encode(), self._with_grad)

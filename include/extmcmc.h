@@ -263,6 +263,12 @@ int32_t extmcmc_generate_obs_normal(extmcmc_t h, int64_t first, int64_t n_obs,
  * compile (EXTMCMC_EINVAL, the log names the call).  Limit: 1 <= n_params <= 16 (each real field holds
  * n_params + 1 doubles in registers); larger is EXTMCMC_EUNSUPPORTED.
  *
+ * Chunked forward mode (extmcmc_set_user_law_chunked): the same source, up to n_params = 64.  A
+ * gradient is ceil(P / K) sweeps of Law<extmcmc::Dual<K>>, each seeded with the unit vectors of K
+ * coordinates, as ForwardDiff's chunk mode does; the chunk width K is part of the compiled program.
+ * At K = P the program, its hash and its results are those of with_grad = EXTMCMC_USER_GRAD_FORWARD;
+ * with the same sweep plan every K gives the same bits.
+ *
  * P = n_params and D = obs_dim are the macros EXTMCMC_P / EXTMCMC_D (compile-time constants).  The
  * fixed-width integer types are defined; no header can be included.  Responses and covariates are
  * extra columns of the observation row (extmcmc_upload_obs with y = NULL).  The law is compiled for
@@ -284,6 +290,18 @@ int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad)
  * then says why). */
 int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                char *log, int64_t log_bytes);
+/* Chunked forward mode: extmcmc_user_law_check with with_grad = EXTMCMC_USER_GRAD_FORWARD for a chunk
+ * width.  chunk: a width in 1..min(16, n_params) that splits n_params into at most 16 chunks, or 0 for
+ * the library's choice (n_params <= 16: the width n_params, the unchunked program; above, the balanced
+ * width ceil(P / ceil(P / 5))).  chunk_used (may be NULL) receives the width compiled.  EXTMCMC_EINVAL
+ * for a bad width (the log says why) or a source that does not compile, EXTMCMC_EUNSUPPORTED outside
+ * 1 <= n_params <= 64 or without NVRTC. */
+int32_t extmcmc_user_law_check_chunked(const char *source, int32_t n_params, int32_t obs_dim, int32_t chunk,
+                                       int32_t *chunk_used, char *log, int64_t log_bytes);
+/* extmcmc_set_user_law for a forward-mode law at a chunk width (chunk: as extmcmc_user_law_check_chunked).
+ * A checkpoint records the width with the law: a blob written at another width is refused
+ * (EXTMCMC_EINVAL), since the width can change the sweep plan and so the last bits of the sums. */
+int32_t extmcmc_set_user_law_chunked(extmcmc_t h, const char *source, int32_t chunk);
 
 /* Replaces RandomWalkUpdate(rw, coords; prior, adpt) src/updates.jl:170-182. */
 int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd);

@@ -104,14 +104,15 @@ struct LogisticLaw; d::Int; end
 struct HierNormalLaw; G::Int; end
 
 """
-    DeviceLaw(source::String, n_params, obs_dim; gradient=false)
+    DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing)
 
 A user-defined law on the device (EXTMCMC_LAW_USER): the counterparts of `set_parameters!(P, θ)` and
 one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_parameters`, `logpdf`, and
 `logpdf_grad` with `gradient = true`; contract in include/extmcmc.h and INTEGRATION.md).  With
 `gradient = :forward` the law is written generic over its scalar (`template <class real> struct Law`,
 `set_parameters`, `logpdf`) and the gradient is derived in forward mode, as ForwardDiff would (at most
-16 parameters).  Compiled for sm_100a when constructed (no device needed); a source that does not
+16 parameters; with `chunk = :auto` or a chunk width, up to 64 in chunks of that many tangents, as
+ForwardDiff's chunk mode: `law.chunk` is the width the library compiled).  Compiled for sm_100a when constructed (no device needed); a source that does not
 compile throws with the compiler's log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values);
 responses are columns of the rows.
 """
@@ -120,19 +121,33 @@ struct DeviceLaw
     n_params::Int
     obs_dim::Int
     with_grad::Int32                                     # USER_GRAD_NONE / _HAND / _FORWARD
+    chunk_arg::Int32                                     # -1: unchunked; 0: the library's width; K
+    chunk::Int                                           # forward mode: the width compiled (0 otherwise)
     log::String
-    function DeviceLaw(source::String, n_params, obs_dim; gradient=false)
+    function DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing)
         with_grad = gradient === :forward ? USER_GRAD_FORWARD :
                     gradient === true ? USER_GRAD_HAND :
                     gradient === false ? USER_GRAD_NONE :
                     throw(ArgumentError("gradient must be false, true or :forward, not $(repr(gradient))"))
+        chunk === nothing || with_grad == USER_GRAD_FORWARD ||
+            throw(ArgumentError("chunk needs gradient = :forward"))
+        chunk_arg = chunk === nothing ? Int32(-1) : chunk === :auto ? Int32(0) :
+                    chunk isa Integer && !(chunk isa Bool) && chunk >= 1 ? Int32(chunk) :
+                    throw(ArgumentError("chunk must be nothing, :auto or a positive width, not $(repr(chunk))"))
         buf = zeros(UInt8, 1 << 16)
-        rc = GC.@preserve buf ccall((:extmcmc_user_law_check, LIB), Int32,
-                                    (Cstring, Int32, Int32, Int32, Ptr{UInt8}, Int64),
-                                    source, n_params, obs_dim, with_grad, pointer(buf), length(buf))
+        used = Ref{Int32}(with_grad == USER_GRAD_FORWARD ? n_params : 0)
+        rc = if chunk_arg < 0
+            GC.@preserve buf ccall((:extmcmc_user_law_check, LIB), Int32,
+                                   (Cstring, Int32, Int32, Int32, Ptr{UInt8}, Int64),
+                                   source, n_params, obs_dim, with_grad, pointer(buf), length(buf))
+        else
+            GC.@preserve buf ccall((:extmcmc_user_law_check_chunked, LIB), Int32,
+                                   (Cstring, Int32, Int32, Int32, Ptr{Int32}, Ptr{UInt8}, Int64),
+                                   source, n_params, obs_dim, chunk_arg, used, pointer(buf), length(buf))
+        end
         log = unsafe_string(pointer(buf))
         rc == 0 || throw(ArgumentError("the device law does not compile (status $rc):\n" * log))
-        new(source, n_params, obs_dim, with_grad, log)
+        new(source, n_params, obs_dim, with_grad, chunk_arg, used[], log)
     end
 end
 
@@ -279,8 +294,13 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
     rc = ccall((:extmcmc_create, LIB), Int32, (Ref{Config}, Ref{Ptr{Cvoid}}), cfg, h)
     rc == 0 || error("extmcmc_create: ", last_error(C_NULL))
     if data.P isa DeviceLaw                              # compiled once per process (cached by the check)
-        check(h[], ccall((:extmcmc_set_user_law, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
-                         h[], data.P.source, data.P.with_grad))
+        if data.P.chunk_arg < 0
+            check(h[], ccall((:extmcmc_set_user_law, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
+                             h[], data.P.source, data.P.with_grad))
+        else
+            check(h[], ccall((:extmcmc_set_user_law_chunked, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
+                             h[], data.P.source, data.P.chunk_arg))
+        end
     end
     keep = Any[]
     for (u, updt) in enumerate(updates)

@@ -6,11 +6,14 @@ sweep time per launch, the cold and cached JIT compile time, and a Poisson-regre
 d = 8 (4096 chains, 1e6 rows) in ms per iteration.  The forward arm runs MALA on the same Poisson
 regression (two MALA updates of 4 coordinates) with the hand-written gradient (tests/user_laws.py)
 and with forward-mode gradients (tests/user_laws_forward.py), alternating: ms per iteration and
-gradient-sweep ms per launch of each.  One JSON object on stdout (and in --out), with the card's name
-and power limit read in the same process.
+gradient-sweep ms per launch of each.  The chunked arm (--chunked) runs the same MALA problem at
+d = 32 and d = 64 (two MALA updates of d/2 coordinates) with the hand-written gradient and with chunked
+forward-mode gradients at the library's chunk width, and at d = 8 at chunk widths 8 (unchunked), 4
+and 2, each set alternating in one process.  One JSON object on stdout (and in --out), with the card's
+name and power limit read in the same process.
 
     python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--forward-only]
-                                   [--forward-steps 30] [--out FILE]
+                                   [--forward-steps 30] [--chunked] [--chunked-steps 6] [--out FILE]
 """
 import argparse
 import ctypes
@@ -64,6 +67,8 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--forward-steps", type=int, default=30, help="timed steps of each forward-arm rep")
     ap.add_argument("--forward-only", action="store_true", help="only the forward arm")
+    ap.add_argument("--chunked", action="store_true", help="only the chunked arm")
+    ap.add_argument("--chunked-steps", type=int, default=6, help="timed steps of each chunked-arm rep")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import extensiblemcmc_jl_b200 as em
@@ -71,9 +76,12 @@ def main():
     from tests import user_laws as ul
 
     out = {"card": card()}
-    if not args.forward_only:
-        builtin_arms(args, em, _abi, ul, out)
-    forward_arm(args, em, _abi, out)
+    if args.chunked:
+        chunked_arm(args, em, _abi, out)
+    else:
+        if not args.forward_only:
+            builtin_arms(args, em, _abi, ul, out)
+        forward_arm(args, em, _abi, out)
     line = json.dumps(out)
     print(line)
     if args.out:
@@ -82,7 +90,7 @@ def main():
 
 
 def poisson_problem(em, N, C, d=8):
-    """Poisson regression with log link, d = 8 (intercept + 7 covariates): rows, true beta, initial state."""
+    """Poisson regression with log link, intercept + d - 1 covariates: rows, initial state."""
     rng = np.random.default_rng(5)
     X = np.empty((N, d))
     X[:, :d - 1] = rng.standard_normal((N, d - 1)) / np.sqrt(d - 1)
@@ -92,29 +100,55 @@ def poisson_problem(em, N, C, d=8):
     return X, thp
 
 
-def forward_arm(args, em, _abi, out):
-    from tests import user_laws as ul
-    from tests import user_laws_forward as uf
-    d, C, N = 8, bench.CHAINS_PER_GPU, 1_000_000
+def mala_arms(args, em, _abi, d, laws, steps):
+    """Poisson regression at d under two MALA updates of d/2 coordinates, 4096 chains x 1e6 rows: every
+    law of `laws` (name -> DeviceLaw) in one process, alternating; ms per iteration and per gradient sweep."""
+    C, N = bench.CHAINS_PER_GPU, 1_000_000
     X, thp = poisson_problem(em, N, C, d)
-    ups = lambda: [em.MALAUpdate(1e-3, [1, 2, 3, 4]), em.MALAUpdate(1e-3, [5, 6, 7, 8])]   # noqa: E731
-    laws = {"hand": em.DeviceLaw(ul.POISSON_REG, d, d, gradient=True),
-            "forward": em.DeviceLaw(uf.POISSON_REG, d, d, gradient="forward")}
-    res = {"workload": "Poisson regression d = 8, 4096 chains x 1e6 rows, 2 MALA updates of 4 coordinates "
+    h = d // 2
+    ups = lambda: [em.MALAUpdate(1e-3, list(range(1, h + 1))), em.MALAUpdate(1e-3, list(range(h + 1, d + 1)))]  # noqa: E731
+    res = {"workload": f"Poisson regression d = {d}, 4096 chains x 1e6 rows, 2 MALA updates of {h} coordinates "
                        "(one gradient sweep each per iteration)"}
     ws = {k: make(em, law, X, ups(), thp, block_len=bench.NU) for k, law in laws.items()}
     times = {k: [] for k in ws}
     for _ in range(args.reps):                           # alternating, the same warm-up each time
         for k, w in ws.items():
-            times[k].append(bench.timed_steps(w, _abi, C, args.forward_steps, 3) / args.forward_steps)
+            times[k].append(bench.timed_steps(w, _abi, C, steps, 3) / steps)
     for k, w in ws.items():
         res[k] = {"ms_per_iter": float(np.median(times[k])), "ms_per_iter_reps": times[k],
-                  "variant": w.lib.extmcmc_sweep_variant_name(w.handle).decode()}
+                  "variant": w.lib.extmcmc_sweep_variant_name(w.handle).decode(),
+                  "chunk": getattr(laws[k], "chunk", None)}
         w.close()
     for k, law in laws.items():
         wi = make(em, law, X, ups(), thp, block_len=5 * bench.NU, use_graphs=False, instrument=True)
-        res[k]["grad_sweep_ms"] = sweep_ms(wi, _abi, max(args.forward_steps // 3, 3))
+        res[k]["grad_sweep_ms"] = sweep_ms(wi, _abi, max(steps // 3, 3))
         wi.close()
+    return res
+
+
+def chunked_arm(args, em, _abi, out):
+    from tests import user_laws as ul
+    from tests import user_laws_forward as uf
+    for d in (32, 64):
+        laws = {"hand": em.DeviceLaw(ul.POISSON_REG, d, d, gradient=True),
+                "chunked": em.DeviceLaw(uf.POISSON_REG, d, d, gradient="forward", chunk="auto")}
+        res = mala_arms(args, em, _abi, d, laws, args.chunked_steps)
+        res["chunked_over_hand_iter"] = res["chunked"]["ms_per_iter"] / res["hand"]["ms_per_iter"]
+        res["chunked_over_hand_sweep"] = res["chunked"]["grad_sweep_ms"] / res["hand"]["grad_sweep_ms"]
+        out[f"poisson_reg_d{d}_mala"] = res
+    d = 8
+    laws = {"hand": em.DeviceLaw(ul.POISSON_REG, d, d, gradient=True)}
+    laws.update({f"forward_k{k}": em.DeviceLaw(uf.POISSON_REG, d, d, gradient="forward", chunk=k) for k in (8, 4, 2)})
+    out["poisson_reg_d8_mala_widths"] = mala_arms(args, em, _abi, d, laws, args.forward_steps)
+
+
+def forward_arm(args, em, _abi, out):
+    from tests import user_laws as ul
+    from tests import user_laws_forward as uf
+    d = 8
+    laws = {"hand": em.DeviceLaw(ul.POISSON_REG, d, d, gradient=True),
+            "forward": em.DeviceLaw(uf.POISSON_REG, d, d, gradient="forward")}
+    res = mala_arms(args, em, _abi, d, laws, args.forward_steps)
     res["forward_over_hand_iter"] = res["forward"]["ms_per_iter"] / res["hand"]["ms_per_iter"]
     res["forward_over_hand_sweep"] = res["forward"]["grad_sweep_ms"] / res["hand"]["grad_sweep_ms"]
     out["poisson_reg_d8_mala"] = res

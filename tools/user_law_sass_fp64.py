@@ -2,9 +2,11 @@
 needed): the "lanes" kernel of the Poisson regression at P = D = 8 with the hand-written gradient
 (tests/user_laws.py) and with forward-mode gradients (tests/user_laws_forward.py), compiled by NVRTC
 with the library's options.  Prints the FP64 instructions of every loop of each kernel; the row loop
-is unrolled 4 times (sweep_user.cuh), so per row = count / 4.
+is unrolled 4 times (sweep_user.cuh), so per row = count / 4.  With --chunked P K: the "lanes" kernel
+of every chunk of the forward-mode Poisson regression at P = D compiled at chunk width K (the
+library's kernel extmcmc_user_lanes_f<K>c<c>), and the hand-written one at the same P.
 
-    python tools/user_law_sass_fp64.py
+    python tools/user_law_sass_fp64.py [--chunked P K]
 """
 import ctypes as C
 import os
@@ -22,13 +24,14 @@ try:
     nv = C.CDLL("libnvrtc.so.12")
 except OSError:
     nv = C.CDLL("/usr/local/cuda/lib64/libnvrtc.so.12")
-def build(src, P, D, mode):
+def build(src, P, D, mode, K=None, c=0):
     hdr = ['sweep_user.cuh', 'dual.cuh', 'tma.cuh']
-    law = {1: 'Law', 2: 'Law<extmcmc::Dual<EXTMCMC_P>>'}[mode]
+    law = {1: 'Law', 2: 'Law<extmcmc::Dual<EXTMCMC_P>>'}[mode] if K is None else f'Law<extmcmc::Dual<{K}>>'
+    tail = f"{mode}" if K is None else f"{mode}, {K}, {c}"
     s = f"#define EXTMCMC_P {P}\n#define EXTMCMC_D {D}\n"
     s += "typedef signed char int8_t; typedef unsigned char uint8_t; typedef int int32_t; typedef unsigned int uint32_t;\ntypedef long long int64_t; typedef unsigned long long uint64_t;\n"
     s += src + '\n#include "sweep_user.cuh"\n'
-    s += f'extern "C" __global__ void __launch_bounds__(128) k(extmcmc::UserSweepArgs a) {{ extmcmc::user_sweep<{law}, EXTMCMC_P, EXTMCMC_D, 1, 32, {mode}>(a); }}\n'
+    s += f'extern "C" __global__ void __launch_bounds__(128) k(extmcmc::UserSweepArgs a) {{ extmcmc::user_sweep<{law}, EXTMCMC_P, EXTMCMC_D, 1, 32, {tail}>(a); }}\n'
     prog = C.c_void_p()
     hs = (C.c_char_p * 3)(*[open(os.path.join(csrc, h), 'rb').read() for h in hdr])
     hn = (C.c_char_p * 3)(*[h.encode() for h in hdr])
@@ -38,7 +41,7 @@ def build(src, P, D, mode):
     n = C.c_size_t(); nv.nvrtcGetProgramLogSize(prog, C.byref(n)); lg = C.create_string_buffer(n.value); nv.nvrtcGetProgramLog(prog, lg)
     assert rc == 0, lg.value.decode()
     nv.nvrtcGetCUBINSize(prog, C.byref(n)); buf = C.create_string_buffer(n.value); nv.nvrtcGetCUBIN(prog, buf)
-    fn = os.path.join(TMP, f"m{mode}.cubin"); open(fn, 'wb').write(buf.raw)
+    fn = os.path.join(TMP, f"m{mode}_{K}_{c}.cubin"); open(fn, 'wb').write(buf.raw)
     return subprocess.run(['cuobjdump', '-sass', fn], capture_output=True, text=True).stdout
 FP64 = re.compile(r"\b(DADD|DMUL|DFMA|DSETP|DMNMX|DMMA|MUFU\.\w*64\w*|F2F\.F64\S*|DRND|F2I\.F64\S*|I2F\.F64\S*)\b")
 def loops(sass):
@@ -55,8 +58,15 @@ def loops(sass):
             out.append((lo, a, sum(1 for x in body if FP64.search(x)), len(body)))
     total = sum(1 for _, x in ins if FP64.search(x))
     return out, total
-for mode, src in ((1, ul.POISSON_REG), (2, uf.POISSON_REG)):
-    sass = build(src, 8, 8, mode)
+if len(sys.argv) == 4 and sys.argv[1] == "--chunked":
+    P, K = int(sys.argv[2]), int(sys.argv[3])
+    jobs = [("hand-written", ul.POISSON_REG, 1, None, 0)]
+    jobs += [(f"forward chunk {c} of width {K}", uf.POISSON_REG, 2, K, c) for c in range(-(-P // K))]
+else:
+    P = 8
+    jobs = [("hand-written", ul.POISSON_REG, 1, None, 0), ("forward", uf.POISSON_REG, 2, None, 0)]
+for name, src, mode, K, c in jobs:
+    sass = build(src, P, P, mode, K, c)
     lp, tot = loops(sass)
-    print("hand-written" if mode == 1 else "forward", "kernel FP64 total", tot)
+    print(name, "kernel FP64 total", tot)
     for l in lp: print("   loop %05x-%05x fp64 %d of %d instr" % l)
