@@ -18,6 +18,7 @@ OK, EINVAL, EUNSUPPORTED, ECUDA, ENCCL, EOOM, EDOMAIN, ESTALE = 0, -1, -2, -3, -
 # laws
 LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = 1, 2, 3, 4, 5
 USER_GRAD_NONE, USER_GRAD_HAND, USER_GRAD_FORWARD = 0, 1, 2
+USER_THETA_TERM = 1                                  # flags of a user law
 # kernels
 KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = 1, 2, 3, 4
 # priors
@@ -113,6 +114,9 @@ SIGNATURES = {
     "extmcmc_set_user_law_chunked": (C.c_int32, [Handle, C.c_char_p, C.c_int32]),
     "extmcmc_user_law_check_chunked": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32,
                                                    C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "extmcmc_set_user_law_ex": (C.c_int32, [Handle, C.c_char_p, C.c_int32, C.c_int32, C.c_int32]),
+    "extmcmc_user_law_check_ex": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                              C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "extmcmc_set_update": (C.c_int32, [Handle, C.c_int32, C.POINTER(Update)]),
     "extmcmc_set_state": (C.c_int32, [Handle, c_double_p]),
     "extmcmc_set_seed": (C.c_int32, [Handle, C.c_uint64]),

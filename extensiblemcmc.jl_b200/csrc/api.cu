@@ -811,6 +811,8 @@ int32_t extmcmc_create(const extmcmc_config_t *cfg, extmcmc_t *out) {
     case EXTMCMC_LAW_USER:
         if (cfg->obs_dim < 1 || cfg->obs_dim > kUserMaxObsDim || cfg->n_params > kUserMaxParams)
             return fail(nullptr, EXTMCMC_EUNSUPPORTED, "USER needs 1 <= obs_dim <= 64 and 1 <= n_params <= 64");
+        // When this is built, only rank 0 adds a law's logpdf_theta (EXTMCMC_USER_THETA_TERM): the per-chain
+        // sums of all ranks are added up, and the term belongs to the whole likelihood once.
         if (cfg->shard_mode == EXTMCMC_SHARD_OBS && cfg->world_size > 1)
             return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws are not implemented under EXTMCMC_SHARD_OBS with several ranks");
         break;
@@ -1353,20 +1355,60 @@ void copy_log(const std::string &msg, char *log, int64_t log_bytes) {
         log[n] = 0;
     }
 }
-// extmcmc_user_law_check and its chunked form; K: the resolved chunk width of forward mode
-int32_t user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int mode, int K, char *log,
-                       int64_t log_bytes) {
+// The options of every user-law entry point, checked and resolved to a UserGrad mode and the chunk
+// width K of forward mode.  chunked: the width comes from `chunk` (the _chunked and _ex entry points);
+// otherwise forward mode is the unchunked program and keeps its limit of kUserMaxForwardParams.
+int32_t user_law_options(int32_t P, int32_t with_grad, bool chunked, int32_t chunk, int32_t flags, int &mode, int &K,
+                         std::string &err) {
+    if (flags & ~EXTMCMC_USER_THETA_TERM) {
+        err = "unknown user-law flags " + std::to_string(flags) + " (known: EXTMCMC_USER_THETA_TERM = 1)";
+        return EXTMCMC_EINVAL;
+    }
+    mode = user_grad_mode(with_grad);
+    K = P;
+    if (mode != kUserGradForward) {
+        if (chunk == 0) return EXTMCMC_OK;
+        err = "chunk must be 0 unless with_grad = EXTMCMC_USER_GRAD_FORWARD; got " + std::to_string(chunk);
+        return EXTMCMC_EINVAL;
+    }
+    if (chunked) return user_law_chunk(P, chunk, K, err);
+    if (P <= kUserMaxForwardParams) return EXTMCMC_OK;
+    err = forward_limit_message(P);
+    return EXTMCMC_EUNSUPPORTED;
+}
+// every extmcmc_user_law_check* entry point
+int32_t user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad, bool chunked,
+                       int32_t chunk, int32_t flags, int32_t *chunk_used, char *log, int64_t log_bytes) {
+    if (log && log_bytes > 0) log[0] = 0;
+    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
+    if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
+        return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
+    int mode = kUserValue, K = 0;
+    std::string err;
+    if (const int32_t rc = user_law_options(n_params, with_grad, chunked, chunk, flags, mode, K, err)) {
+        copy_log(err, log, log_bytes);
+        return fail(nullptr, rc, err);
+    }
+    if (chunk_used) *chunk_used = mode == kUserGradForward ? K : 0;
     std::string lg, cubin;
-    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, K, lg, cubin, nullptr);
+    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, K, flags, lg, cubin, nullptr);
     copy_log(lg, log, log_bytes);
     if (rc) g_create_error = lg;
     return rc;
 }
-// extmcmc_set_user_law and its chunked form
-int32_t set_user_law(extmcmc_t h, const char *source, int mode, int K) {
+// every extmcmc_set_user_law* entry point; entry: its name, for the messages
+int32_t set_user_law(extmcmc_t h, const char *entry, const char *source, int32_t with_grad, bool chunked,
+                     int32_t chunk, int32_t flags) {
+    if (!h) return EXTMCMC_EINVAL;
+    if (h->cfg.law != EXTMCMC_LAW_USER) return fail(h, EXTMCMC_EINVAL, std::string(entry) + " needs a handle of law EXTMCMC_LAW_USER");
+    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
+    int mode = kUserValue, K = 0;
+    std::string err;
+    if (const int32_t rc = user_law_options(h->cfg.n_params, with_grad, chunked, chunk, flags, mode, K, err))
+        return fail(h, rc, err);
     std::string log, cubin;
     uint64_t hash = 0;
-    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, K, log, cubin, &hash);
+    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, K, flags, log, cubin, &hash);
     if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
     if (rc) return fail(h, rc, log);
     CK(h, cudaSetDevice(h->cfg.device));
@@ -1386,54 +1428,30 @@ extern "C" {
 
 int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                char *log, int64_t log_bytes) {
-    if (log && log_bytes > 0) log[0] = 0;
-    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
-    if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
-        return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
-    const int mode = user_grad_mode(with_grad);
-    if (mode == kUserGradForward && n_params > kUserMaxForwardParams) {
-        const std::string msg = forward_limit_message(n_params);
-        copy_log(msg, log, log_bytes);
-        return fail(nullptr, EXTMCMC_EUNSUPPORTED, msg);
-    }
-    return user_law_check(source, n_params, obs_dim, mode, n_params, log, log_bytes);
+    return user_law_check(source, n_params, obs_dim, with_grad, false, 0, 0, nullptr, log, log_bytes);
 }
 
 int32_t extmcmc_user_law_check_chunked(const char *source, int32_t n_params, int32_t obs_dim, int32_t chunk,
                                        int32_t *chunk_used, char *log, int64_t log_bytes) {
-    if (log && log_bytes > 0) log[0] = 0;
-    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
-    if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
-        return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
-    int K = 0;
-    std::string err;
-    if (user_law_chunk(n_params, chunk, K, err)) {
-        copy_log(err, log, log_bytes);
-        return fail(nullptr, EXTMCMC_EINVAL, err);
-    }
-    if (chunk_used) *chunk_used = K;
-    return user_law_check(source, n_params, obs_dim, kUserGradForward, K, log, log_bytes);
+    return user_law_check(source, n_params, obs_dim, EXTMCMC_USER_GRAD_FORWARD, true, chunk, 0, chunk_used, log,
+                          log_bytes);
+}
+
+int32_t extmcmc_user_law_check_ex(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                                  int32_t chunk, int32_t flags, int32_t *chunk_used, char *log, int64_t log_bytes) {
+    return user_law_check(source, n_params, obs_dim, with_grad, true, chunk, flags, chunk_used, log, log_bytes);
 }
 
 int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad) {
-    if (!h) return EXTMCMC_EINVAL;
-    if (h->cfg.law != EXTMCMC_LAW_USER) return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_law needs a handle of law EXTMCMC_LAW_USER");
-    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
-    const int mode = user_grad_mode(with_grad);
-    if (mode == kUserGradForward && h->cfg.n_params > kUserMaxForwardParams)
-        return fail(h, EXTMCMC_EUNSUPPORTED, forward_limit_message(h->cfg.n_params));
-    return set_user_law(h, source, mode, h->cfg.n_params);
+    return set_user_law(h, "extmcmc_set_user_law", source, with_grad, false, 0, 0);
 }
 
 int32_t extmcmc_set_user_law_chunked(extmcmc_t h, const char *source, int32_t chunk) {
-    if (!h) return EXTMCMC_EINVAL;
-    if (h->cfg.law != EXTMCMC_LAW_USER)
-        return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_law_chunked needs a handle of law EXTMCMC_LAW_USER");
-    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
-    int K = 0;
-    std::string err;
-    if (user_law_chunk(h->cfg.n_params, chunk, K, err)) return fail(h, EXTMCMC_EINVAL, err);
-    return set_user_law(h, source, kUserGradForward, K);
+    return set_user_law(h, "extmcmc_set_user_law_chunked", source, EXTMCMC_USER_GRAD_FORWARD, true, chunk, 0);
+}
+
+int32_t extmcmc_set_user_law_ex(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags) {
+    return set_user_law(h, "extmcmc_set_user_law_ex", source, with_grad, true, chunk, flags);
 }
 
 // ---- checkpoint / resume ------------------------------------------------------------------------

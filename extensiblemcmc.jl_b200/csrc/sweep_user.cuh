@@ -75,8 +75,35 @@ struct UserSweepArgs {
 };
 
 #ifdef __CUDACC_RTC__
+#ifdef EXTMCMC_THETA_TERM
+// Adds the law's parameter-only term (EXTMCMC_USER_THETA_TERM) to a chain's sums: its value to ll and,
+// with a gradient, its derivatives in the coordinates of the sweep's accumulators to g[0..NG-1] --
+// logpdf_theta_grad on a zeroed t (hand-written), or the tangents of logpdf_theta on the Law<Dual<K>> of
+// the chunk (forward mode).  Each sum gets one addition: ll = fl(rows + term), g[k] = fl(rows_k + t_k).
+template <int G, int NG, class LawT>
+__device__ __forceinline__ void user_add_theta_term(const LawT &L, double &ll, double *g) {
+    if constexpr (G == kUserGradForward) {
+        const auto t = logpdf_theta(L);
+        ll += t.v;
+#pragma unroll
+        for (int k = 0; k < NG; ++k) g[k] += t.t[k];
+    } else if constexpr (G == kUserGradHand) {
+        double t[NG];
+#pragma unroll
+        for (int k = 0; k < NG; ++k) t[k] = 0.0;
+        ll += logpdf_theta_grad(L, t);
+#pragma unroll
+        for (int k = 0; k < NG; ++k) g[k] += t[k];
+    } else {
+        ll += logpdf_theta(L);
+    }
+}
+#endif
+
 // K, CI: chunk width and chunk index of a forward-mode sweep (LawT = Law<Dual<K>>); chunk 0 writes
 // ll_part and raises err_flag, every chunk writes only its own rows g_part[S][CI*K ..][C].
+// With EXTMCMC_THETA_TERM the CTAs of segment 0 add the law's parameter-only term to the sums of their
+// own rows (user_add_theta_term).
 template <class LawT, int P, int D, int R, int L, int G, int K = P, int CI = 0>
 __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
     constexpr bool GRAD = G != kUserValue;
@@ -188,9 +215,28 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
+#ifdef EXTMCMC_THETA_TERM
+        // Segment 0 adds the term once per chain to the sums of its rows.  The lanes of a chain are reduced
+        // first: all of them then hold the sums, and all evaluate the term (the warp stays converged), and
+        // the term is not held in registers across the shuffles.
+        constexpr int LR = 1;   // the lanes are reduced here
+        if (L > 1) {
+#pragma unroll
+            for (int o = L / 2; o > 0 && WRITE_LL; o >>= 1) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
+#pragma unroll
+            for (int k = 0; k < NG && GRAD; ++k) {
+                if (K0 + k >= P) break;
+#pragma unroll
+                for (int o = L / 2; o > 0; o >>= 1) g[r][k] += __shfl_xor_sync(0xffffffffu, g[r][k], o);
+            }
+        }
+        if (seg == 0 && c < C && ok[r]) user_add_theta_term<G, NG>(law[r], acc[r], g[r]);
+#else
+        constexpr int LR = L;
+#endif
         if constexpr (WRITE_LL) {
             double v = acc[r];
-            if (L > 1) {
+            if (LR > 1) {
 #pragma unroll
                 for (int o = L / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
             }
@@ -201,7 +247,7 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
             for (int k = 0; k < NG; ++k) {
                 if (K0 + k >= P) break;   // the tangents past P of a narrower last chunk: seeded zero, not written
                 double w = g[r][k];
-                if (L > 1) {
+                if (LR > 1) {
 #pragma unroll
                     for (int o = L / 2; o > 0; o >>= 1) w += __shfl_xor_sync(0xffffffffu, w, o);
                 }

@@ -23,10 +23,11 @@ int32_t user_law_chunk(int P, int chunk, int &K, std::string &err);
 // Compiles every instantiation the planner can pick for (P, D, mode) to an sm_100a cubin, or takes it
 // from the process-wide cache keyed by the exact NVRTC input.  mode: a UserGrad (sweep_user.cuh; the
 // caller resolves the chunk width K of kUserGradForward with user_law_chunk; other modes ignore K).
+// flags: EXTMCMC_USER_* (EXTMCMC_USER_THETA_TERM compiles the law's logpdf_theta into the sweeps).
 // log: NVRTC + ptxas log.  Returns EXTMCMC_OK, EXTMCMC_EINVAL (the source does not compile) or
 // EXTMCMC_EUNSUPPORTED (no NVRTC).
-int32_t user_law_compile(const char *source, int P, int D, int mode, int K, std::string &log, std::string &cubin,
-                         uint64_t *input_hash);
+int32_t user_law_compile(const char *source, int P, int D, int mode, int K, int flags, std::string &log,
+                         std::string &cubin, uint64_t *input_hash);
 
 struct UserLaw {
     bool loaded = false;

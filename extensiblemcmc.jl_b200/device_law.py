@@ -21,6 +21,14 @@ Up to 64 parameters in forward mode with chunk="auto" or a chunk width: the grad
 sweeps of K tangents each (ForwardDiff's chunk mode); the library picks K for "auto", and law.chunk
 reports the width compiled.
 
+With theta_term=True the law also defines a term of theta only, added once to its log-likelihood
+(sum over rows of logpdf, plus logpdf_theta): the hierarchical p(theta_g | mu, tau) of a multilevel model,
+a shrinkage penalty, any term the reference's loglikelihood adds that no row carries:
+
+    __device__ double logpdf_theta(const Law &L);
+    __device__ double logpdf_theta_grad(const Law &L, double *g);                  // gradient=True
+    template <class real> __device__ real logpdf_theta(const Law<real> &L);        // gradient="forward"
+
 Data: dict(P=DeviceLaw(source, n_params, obs_dim), obs=rows [N, obs_dim]); responses and
 covariates are columns of the rows.  The constructor compiles the law for sm_100a (no device
 needed) and raises ValueError with the compiler's log when it does not compile.
@@ -31,10 +39,11 @@ from . import _abi
 
 
 class DeviceLaw:
-    def __init__(self, source, n_params, obs_dim=1, gradient=False, chunk=None):
+    def __init__(self, source, n_params, obs_dim=1, gradient=False, chunk=None, theta_term=False):
         """gradient: False (none), True (the source defines logpdf_grad) or "forward".
         chunk (forward mode only): None (unchunked, at most 16 parameters), "auto" (the library's width)
-        or a chunk width; the library checks the width against n_params."""
+        or a chunk width; the library checks the width against n_params.
+        theta_term: True when the source defines logpdf_theta (and logpdf_theta_grad with gradient=True)."""
         if isinstance(gradient, str) and gradient == "forward":
             self._with_grad = _abi.USER_GRAD_FORWARD
         elif isinstance(gradient, (bool, int)) and gradient in (False, True):
@@ -49,6 +58,9 @@ class DeviceLaw:
             self._chunk_arg = chunk
         else:
             raise ValueError(f"chunk must be None, 'auto' or a positive width, not {chunk!r}")
+        if not isinstance(theta_term, bool):
+            raise ValueError(f"theta_term must be True or False, not {theta_term!r}")
+        self.theta_term = theta_term
         self.source = str(source)
         self._n_params = int(n_params)
         self._obs_dim = int(obs_dim)
@@ -56,7 +68,15 @@ class DeviceLaw:
         self.chunk = None                            # forward mode: the chunk width compiled
         lib = _abi.load()
         buf = C.create_string_buffer(1 << 16)
-        if self._chunk_arg is None:
+        if theta_term:
+            used = C.c_int32(-1)
+            rc = lib.extmcmc_user_law_check_ex(self.source.encode(), self._n_params, self._obs_dim, self._with_grad,
+                                               self._ex_chunk(), _abi.USER_THETA_TERM, C.byref(used), buf, len(buf))
+            if rc == _abi.EINVAL and used.value == -1:   # the arguments were refused before compiling
+                raise ValueError(buf.value.decode(errors="replace"))
+            if self._with_grad == _abi.USER_GRAD_FORWARD:
+                self.chunk = used.value
+        elif self._chunk_arg is None:
             rc = lib.extmcmc_user_law_check(self.source.encode(), self._n_params, self._obs_dim,
                                             self._with_grad, buf, len(buf))
             if rc == _abi.OK and self._with_grad == _abi.USER_GRAD_FORWARD:
@@ -74,6 +94,12 @@ class DeviceLaw:
         if rc != _abi.OK:
             raise _abi.ExtMCMCError(rc, self.log or lib.extmcmc_last_error(None).decode())
 
+    def _ex_chunk(self):
+        """chunk of the _ex entry points: None in forward mode is the unchunked width n_params"""
+        if self._chunk_arg is not None:
+            return self._chunk_arg
+        return self._n_params if self._with_grad == _abi.USER_GRAD_FORWARD else 0
+
     def abi_law(self):
         return _abi.LAW_USER
 
@@ -90,6 +116,9 @@ class DeviceLaw:
 
     def abi_attach(self, lib, handle):
         """Compiles (cached) and installs the law on a freshly created library handle."""
+        if self.theta_term:
+            return lib.extmcmc_set_user_law_ex(handle, self.source.encode(), self._with_grad, self._ex_chunk(),
+                                               _abi.USER_THETA_TERM)
         if self._chunk_arg is not None:
             return lib.extmcmc_set_user_law_chunked(handle, self.source.encode(), self._chunk_arg)
         return lib.extmcmc_set_user_law(handle, self.source.encode(), self._with_grad)

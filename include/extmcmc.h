@@ -74,6 +74,11 @@ enum {
     EXTMCMC_USER_GRAD_FORWARD = 2  /* the source is generic over its scalar; the library
                                       derives the gradient in forward mode (dual numbers)    */
 };
+/* ---- what a user-defined law declares besides logpdf (flags of extmcmc_set_user_law_ex) */
+enum {
+    EXTMCMC_USER_THETA_TERM = 1    /* the source defines logpdf_theta (+ logpdf_theta_grad with a
+                                      hand-written gradient): a term of theta only, added once */
+};
 
 /* ---- transition kernels (src/transition_kernels/random_walk.jl, src/updates.jl) */
 enum {
@@ -269,6 +274,26 @@ int32_t extmcmc_generate_obs_normal(extmcmc_t h, int64_t first, int64_t n_obs,
  * At K = P the program, its hash and its results are those of with_grad = EXTMCMC_USER_GRAD_FORWARD;
  * with the same sweep plan every K gives the same bits.
  *
+ * A term of theta only (flags = EXTMCMC_USER_THETA_TERM, extmcmc_set_user_law_ex): the reference's
+ * loglikelihood may add terms that depend on theta alone, such as the hierarchical p(theta_g | mu, tau)
+ * of a multilevel model, which its priors cannot express (they see only their own update's
+ * coordinates).  The law then also defines, evaluated once per chain and log-likelihood evaluation on
+ * the Law that set_parameters built:
+ *
+ *   __device__ double logpdf_theta(const Law &L);
+ *   // with_grad = 1: returns logpdf_theta and ADDS d logpdf_theta / d th into g[0..P-1]
+ *   __device__ double logpdf_theta_grad(const Law &L, double *g);
+ *   // forward mode: generic over the scalar, differentiated like logpdf
+ *   template <class real> __device__ real logpdf_theta(const Law<real> &L);
+ *
+ * and its log-likelihood is sum_rows logpdf(L, x) + logpdf_theta(L).  The sweep's segment 0 adds the
+ * term after its own rows (ll_part[0] = fl(rows + logpdf_theta), the same for every gradient
+ * component), so forward mode still gives the value sweep's ll bit for bit and every chunk width the
+ * same bits.  A NaN term gives the chain ll = NaN (its proposal is rejected), as a NaN logpdf does.
+ * The flag is declared, not detected: with it, a source without these functions does not compile
+ * (EXTMCMC_EINVAL, the log names the function); without it, the program is the one compiled before
+ * the flag existed.  The flag is part of the compiled program and of a checkpoint's law hash.
+ *
  * P = n_params and D = obs_dim are the macros EXTMCMC_P / EXTMCMC_D (compile-time constants).  The
  * fixed-width integer types are defined; no header can be included.  Responses and covariates are
  * extra columns of the observation row (extmcmc_upload_obs with y = NULL).  The law is compiled for
@@ -302,6 +327,15 @@ int32_t extmcmc_user_law_check_chunked(const char *source, int32_t n_params, int
  * A checkpoint records the width with the law: a blob written at another width is refused
  * (EXTMCMC_EINVAL), since the width can change the sweep plan and so the last bits of the sums. */
 int32_t extmcmc_set_user_law_chunked(extmcmc_t h, const char *source, int32_t chunk);
+/* The general form of the checks above: with_grad (EXTMCMC_USER_GRAD_*), chunk (as in
+ * extmcmc_user_law_check_chunked; must be 0 unless with_grad = EXTMCMC_USER_GRAD_FORWARD) and flags
+ * (EXTMCMC_USER_*; other bits are EXTMCMC_EINVAL).  chunk_used (may be NULL) receives the chunk width
+ * compiled in forward mode and 0 otherwise, once the arguments are accepted. */
+int32_t extmcmc_user_law_check_ex(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                                  int32_t chunk, int32_t flags, int32_t *chunk_used, char *log, int64_t log_bytes);
+/* extmcmc_set_user_law with the arguments of extmcmc_user_law_check_ex.  A checkpoint written by a law
+ * compiled with other flags is refused (EXTMCMC_EINVAL). */
+int32_t extmcmc_set_user_law_ex(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags);
 
 /* Replaces RandomWalkUpdate(rw, coords; prior, adpt) src/updates.jl:170-182. */
 int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd);

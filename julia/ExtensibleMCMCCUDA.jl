@@ -85,6 +85,7 @@ const KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = Int
 const ADAPT_NONE, ADAPT_UNIF_RW, ADAPT_HAARIO, ADAPT_MALA = Int32(0), Int32(1), Int32(2), Int32(3)
 const PRIOR_PRODUCT, PRIOR_MVNORMAL = Int32(5), Int32(11)
 const USER_GRAD_NONE, USER_GRAD_HAND, USER_GRAD_FORWARD = Int32(0), Int32(1), Int32(2)
+const USER_THETA_TERM = Int32(1)
 
 # ---- backend, build-defined laws and the MALA update (an empty stub in the reference) ------------
 struct CUDAMCMCBackend <: eMCMC.MCMCBackend
@@ -104,7 +105,7 @@ struct LogisticLaw; d::Int; end
 struct HierNormalLaw; G::Int; end
 
 """
-    DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing)
+    DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false)
 
 A user-defined law on the device (EXTMCMC_LAW_USER): the counterparts of `set_parameters!(P, θ)` and
 one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_parameters`, `logpdf`, and
@@ -112,7 +113,10 @@ one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_par
 `gradient = :forward` the law is written generic over its scalar (`template <class real> struct Law`,
 `set_parameters`, `logpdf`) and the gradient is derived in forward mode, as ForwardDiff would (at most
 16 parameters; with `chunk = :auto` or a chunk width, up to 64 in chunks of that many tangents, as
-ForwardDiff's chunk mode: `law.chunk` is the width the library compiled).  Compiled for sm_100a when constructed (no device needed); a source that does not
+ForwardDiff's chunk mode: `law.chunk` is the width the library compiled).  With `theta_term = true` the
+source also defines `logpdf_theta` (and `logpdf_theta_grad` with `gradient = true`), a term of θ only
+that is added once to the log-likelihood, such as the hierarchical p(θ_g | μ, τ) of a multilevel model.
+Compiled for sm_100a when constructed (no device needed); a source that does not
 compile throws with the compiler's log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values);
 responses are columns of the rows.
 """
@@ -123,8 +127,9 @@ struct DeviceLaw
     with_grad::Int32                                     # USER_GRAD_NONE / _HAND / _FORWARD
     chunk_arg::Int32                                     # -1: unchunked; 0: the library's width; K
     chunk::Int                                           # forward mode: the width compiled (0 otherwise)
+    flags::Int32                                         # USER_THETA_TERM or 0
     log::String
-    function DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing)
+    function DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false)
         with_grad = gradient === :forward ? USER_GRAD_FORWARD :
                     gradient === true ? USER_GRAD_HAND :
                     gradient === false ? USER_GRAD_NONE :
@@ -134,9 +139,16 @@ struct DeviceLaw
         chunk_arg = chunk === nothing ? Int32(-1) : chunk === :auto ? Int32(0) :
                     chunk isa Integer && !(chunk isa Bool) && chunk >= 1 ? Int32(chunk) :
                     throw(ArgumentError("chunk must be nothing, :auto or a positive width, not $(repr(chunk))"))
+        theta_term isa Bool || throw(ArgumentError("theta_term must be true or false, not $(repr(theta_term))"))
+        flags = theta_term ? USER_THETA_TERM : Int32(0)
         buf = zeros(UInt8, 1 << 16)
         used = Ref{Int32}(with_grad == USER_GRAD_FORWARD ? n_params : 0)
-        rc = if chunk_arg < 0
+        rc = if theta_term                               # chunk: nothing in forward mode is the width n_params
+            GC.@preserve buf ccall((:extmcmc_user_law_check_ex, LIB), Int32,
+                                   (Cstring, Int32, Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{UInt8}, Int64),
+                                   source, n_params, obs_dim, with_grad, ex_chunk(with_grad, chunk_arg, n_params),
+                                   flags, used, pointer(buf), length(buf))
+        elseif chunk_arg < 0
             GC.@preserve buf ccall((:extmcmc_user_law_check, LIB), Int32,
                                    (Cstring, Int32, Int32, Int32, Ptr{UInt8}, Int64),
                                    source, n_params, obs_dim, with_grad, pointer(buf), length(buf))
@@ -147,9 +159,12 @@ struct DeviceLaw
         end
         log = unsafe_string(pointer(buf))
         rc == 0 || throw(ArgumentError("the device law does not compile (status $rc):\n" * log))
-        new(source, n_params, obs_dim, with_grad, chunk_arg, used[], log)
+        new(source, n_params, obs_dim, with_grad, chunk_arg, used[], flags, log)
     end
 end
+# chunk of the _ex entry points
+ex_chunk(with_grad, chunk_arg, n_params) =
+    chunk_arg >= 0 ? chunk_arg : with_grad == USER_GRAD_FORWARD ? Int32(n_params) : Int32(0)
 
 "MALAUpdate(tau, coords; prior, adpt): theta° = theta + tau^2/2 grad(ll + log prior)(theta) + tau z (src/updates.jl:216-218 is an empty stub)"
 struct CUDAMALAUpdate{TP,TA} <: eMCMC.MCMCGradientBasedUpdate
@@ -294,7 +309,11 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
     rc = ccall((:extmcmc_create, LIB), Int32, (Ref{Config}, Ref{Ptr{Cvoid}}), cfg, h)
     rc == 0 || error("extmcmc_create: ", last_error(C_NULL))
     if data.P isa DeviceLaw                              # compiled once per process (cached by the check)
-        if data.P.chunk_arg < 0
+        if data.P.flags != 0
+            check(h[], ccall((:extmcmc_set_user_law_ex, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32, Int32, Int32),
+                             h[], data.P.source, data.P.with_grad,
+                             ex_chunk(data.P.with_grad, data.P.chunk_arg, data.P.n_params), data.P.flags))
+        elseif data.P.chunk_arg < 0
             check(h[], ccall((:extmcmc_set_user_law, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32),
                              h[], data.P.source, data.P.with_grad))
         else

@@ -9,11 +9,16 @@ and with forward-mode gradients (tests/user_laws_forward.py), alternating: ms pe
 gradient-sweep ms per launch of each.  The chunked arm (--chunked) runs the same MALA problem at
 d = 32 and d = 64 (two MALA updates of d/2 coordinates) with the hand-written gradient and with chunked
 forward-mode gradients at the library's chunk width, and at d = 8 at chunk widths 8 (unchunked), 4
-and 2, each set alternating in one process.  One JSON object on stdout (and in --out), with the card's
-name and power limit read in the same process.
+and 2, each set alternating in one process.  The theta-term arm (--theta-term) runs BASELINE cfg 4
+(8192 chains, 8 groups x 4096 rows, MALA on theta_1..8 and two walks, bench.py's updates, 10 iterations per
+extmcmc_run_block) on the built-in HIER_NORMAL law with its data-sum cache off and on, and on its
+DeviceLaw restatement with a theta term (tests/user_laws_theta.py) with the hand-written and the
+forward-mode gradient, alternating: ms per iteration and sweep ms per launch of each.  One JSON object
+on stdout (and in --out), with the card's name and power limit read in the same process.
 
     python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--forward-only]
-                                   [--forward-steps 30] [--chunked] [--chunked-steps 6] [--out FILE]
+                                   [--forward-steps 30] [--chunked] [--chunked-steps 6]
+                                   [--theta-term] [--theta-steps 50] [--out FILE]
 """
 import argparse
 import ctypes
@@ -69,6 +74,8 @@ def main():
     ap.add_argument("--forward-only", action="store_true", help="only the forward arm")
     ap.add_argument("--chunked", action="store_true", help="only the chunked arm")
     ap.add_argument("--chunked-steps", type=int, default=6, help="timed steps of each chunked-arm rep")
+    ap.add_argument("--theta-term", action="store_true", help="only the theta-term arm (cfg 4)")
+    ap.add_argument("--theta-steps", type=int, default=50, help="timed iterations of each theta-term rep")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import extensiblemcmc_jl_b200 as em
@@ -76,7 +83,9 @@ def main():
     from tests import user_laws as ul
 
     out = {"card": card()}
-    if args.chunked:
+    if args.theta_term:
+        theta_term_arm(args, em, _abi, out)
+    elif args.chunked:
         chunked_arm(args, em, _abi, out)
     else:
         if not args.forward_only:
@@ -152,6 +161,70 @@ def forward_arm(args, em, _abi, out):
     res["forward_over_hand_iter"] = res["forward"]["ms_per_iter"] / res["hand"]["ms_per_iter"]
     res["forward_over_hand_sweep"] = res["forward"]["grad_sweep_ms"] / res["hand"]["grad_sweep_ms"]
     out["poisson_reg_d8_mala"] = res
+
+
+def theta_term_arm(args, em, _abi, out):
+    """BASELINE cfg 4 on the built-in HIER_NORMAL law (data-sum cache off / on) and on its DeviceLaw
+    restatement with a theta term (hand-written / forward-mode gradient), alternating."""
+    from extensiblemcmc_jl_b200.mcmc import init_
+    from tests import user_laws_theta as ut
+    C, G, ng, ipb = 8192, 8, 4096, bench.CFG4_BLOCK_ITERS
+    rng = np.random.default_rng(5)                       # bench.py's cfg 4 data, updates and initial state
+    tg = rng.standard_normal(G)
+    yv = np.concatenate([tg[g] + rng.standard_normal(ng) for g in range(G)])
+    grp = np.repeat(np.arange(G), ng)
+    rows = np.stack([yv, grp.astype(np.float64)], axis=1)
+    ups = lambda: [  # noqa: E731
+        em.MALAUpdate(0.02, list(range(1, G + 1)), adpt=em.AdaptationMALA(adapt_every_k_steps=50, scale=1e-3, min=1e-5)),
+        em.RandomWalkUpdate(em.UniformRandomWalk([0.3]), [G + 1], adpt=em.AdaptationUnifRW([0.0], adapt_every_k_steps=50, scale=0.02)),
+        em.RandomWalkUpdate(em.UniformRandomWalk([0.3], [True]), [G + 2], prior=em.ImproperPosPrior(),
+                            adpt=em.AdaptationUnifRW([0.0], adapt_every_k_steps=50, scale=0.02))]
+    th0 = np.concatenate([np.zeros(G), [0.0, 1.0]])
+    P = G + 2
+    arms = {"builtin_no_cache": (dict(P=em.HierNormalLaw(G), obs=yv, groups=grp), "0"),
+            "builtin_cache": (dict(P=em.HierNormalLaw(G), obs=yv, groups=grp), "1"),
+            "device_law_hand": (dict(P=em.DeviceLaw(ut.HIER_HAND, P, 2, gradient=True, theta_term=True), obs=rows), None),
+            "device_law_forward": (dict(P=em.DeviceLaw(ut.HIER_FORWARD, P, 2, gradient="forward", theta_term=True),
+                                        obs=rows), None)}
+    out["theta_term_workload"] = (f"BASELINE cfg 4: hierarchical normal, {G} groups x {ng} rows, {C} chains, MALA(theta_1..8) "
+                                  f"+ RW(mu) + RW-pos(tau), {ipb} iterations per extmcmc_run_block")
+    warm = 3 * ipb
+    steps = -(-args.theta_steps // ipb) * ipb
+
+    def make(data, cache, **bk):
+        # EXTMCMC_DATA_CACHE is read when the sweep is planned: on the first block of the handle
+        os.environ["EXTMCMC_DATA_CACHE"] = cache or "1"
+        mcmc = em.MCMC(ups(), backend=em.CUDAMCMCBackend(n_chains=C, seed=7, history="none", block_len=3 * ipb, **bk))
+        init_(mcmc, 1, data, th0)
+        w = mcmc.workspace
+        bench._generic_timed(w, _abi, 3, 0, warm, ipb=ipb)
+        return w
+    ws = {k: make(d, cache) for k, (d, cache) in arms.items()}
+    it = {k: warm + 1 for k in ws}
+    times = {k: [] for k in ws}
+    for _ in range(args.reps):                           # alternating
+        for k, w in ws.items():
+            times[k].append(bench._generic_timed(w, _abi, 3, steps, 0, it0=it[k], ipb=ipb) / steps)
+            it[k] += steps
+    res = {}
+    for k, w in ws.items():
+        res[k] = {"ms_per_iter": float(np.median(times[k])), "ms_per_iter_reps": times[k],
+                  "variant": w.lib.extmcmc_sweep_variant_name(w.handle).decode()}
+        w.close()
+    for k, (d, cache) in arms.items():
+        wi = make(d, cache, use_graphs=False, instrument=True)
+        msw, nl = ctypes.c_float(), ctypes.c_int64()
+        wi._ck(wi.lib.extmcmc_get_sweep_time(wi.handle, ctypes.byref(msw), ctypes.byref(nl)))
+        bench._generic_timed(wi, _abi, 3, 2 * ipb, 0, it0=warm + 1, ipb=ipb)
+        wi._ck(wi.lib.extmcmc_get_sweep_time(wi.handle, ctypes.byref(msw), ctypes.byref(nl)))
+        res[k]["sweep_ms_per_launch"] = msw.value / max(nl.value, 1)
+        res[k]["sweep_launches_per_iter"] = nl.value / (2 * ipb)
+        wi.close()
+    os.environ.pop("EXTMCMC_DATA_CACHE", None)
+    for k in ("device_law_hand", "device_law_forward"):
+        res[k + "_over_builtin_cache"] = res[k]["ms_per_iter"] / res["builtin_cache"]["ms_per_iter"]
+        res[k + "_over_builtin_no_cache"] = res[k]["ms_per_iter"] / res["builtin_no_cache"]["ms_per_iter"]
+    out["hier_cfg4_theta_term"] = res
 
 
 def builtin_arms(args, em, _abi, ul, out):
