@@ -117,6 +117,10 @@ SIGNATURES = {
     "extmcmc_set_user_law_ex": (C.c_int32, [Handle, C.c_char_p, C.c_int32, C.c_int32, C.c_int32]),
     "extmcmc_user_law_check_ex": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                               C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "extmcmc_set_user_law_theta_only": (C.c_int32, [Handle, C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_uint64]),
+    "extmcmc_user_law_check_theta_only": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                                      C.c_int32, C.c_uint64, C.POINTER(C.c_int32), C.c_char_p,
+                                                      C.c_int64]),
     "extmcmc_set_update": (C.c_int32, [Handle, C.c_int32, C.POINTER(Update)]),
     "extmcmc_set_state": (C.c_int32, [Handle, c_double_p]),
     "extmcmc_set_seed": (C.c_int32, [Handle, C.c_uint64]),

@@ -87,11 +87,15 @@ struct extmcmc_handle {
     unsigned int *tail_counter = nullptr; // CTA counter of the fused sweep tail
     bool tail = false;                   // the obs-mapped sweep finishes the reduction itself
     bool grad_valid = false;             // grad_cur holds d ll/d theta of the CURRENT state
-    // Data-sum cache (dev_state.cuh: dsum_cur / dsum_prop).  dcache: the handle keeps one (HIER_NORMAL,
-    // observations not sharded, EXTMCMC_DATA_CACHE != 0); dc_valid: dsum_cur holds the per-group data
-    // sums of the CURRENT state.
-    bool dcache = false, dc_valid = false;
+    // Data-sum cache (dev_state.cuh: dsum_cur / dsum_prop).  dcache: the handle keeps one (HIER_NORMAL, or
+    // a user law with parameter-only coordinates; observations not sharded, EXTMCMC_DATA_CACHE != 0).
+    // dc_valid: dsum_cur holds the data sums of the CURRENT state (user law: its row sum R); rg_valid:
+    // ... and their gradient (user law: Rg; HIER_NORMAL: always equal to dc_valid).
+    bool dcache = false, dc_valid = false, rg_valid = false;
     double *dsum_buf[2] = {nullptr, nullptr};   // the allocations behind d.dsum_cur / d.dsum_prop
+    // A user law with parameter-only coordinates: [1 + p][C] row sums of the current state / of a
+    // proposal (what its sweeps finish into; with dcache also d.dsum_cur / d.dsum_prop)
+    double *rsum_buf[2] = {nullptr, nullptr};
     bool any_mala = false;
     bool state_set = false;
     SweepPlan plan{};
@@ -238,14 +242,22 @@ int32_t ensure_plan(extmcmc_t h) {
     {
         const char *e = getenv("EXTMCMC_DATA_CACHE");   // read per plan, so that one process can compare both
         const bool on = !e || atoi(e) != 0;
-        h->dcache = on && h->cfg.law == EXTMCMC_LAW_HIER_NORMAL && !obs_sharded(h) && h->d.G <= kDataCacheMaxG;
-        if (h->dcache && !h->dsum_buf[0])
+        const bool rows = h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.theta_only;
+        h->dcache = on && !obs_sharded(h) &&
+                    ((h->cfg.law == EXTMCMC_LAW_HIER_NORMAL && h->d.G <= kDataCacheMaxG) || rows);
+        if (h->dcache && !rows && !h->dsum_buf[0])
             if ((rc = dev_alloc(h, &h->dsum_buf[0], (size_t)2 * h->d.G * h->d.C)) ||
                 (rc = dev_alloc(h, &h->dsum_buf[1], (size_t)2 * h->d.G * h->d.C)))
                 return rc;
-        h->d.dsum_cur = h->dcache ? h->dsum_buf[0] : nullptr;
-        h->d.dsum_prop = h->dcache ? h->dsum_buf[1] : nullptr;
-        h->dc_valid = false;
+        if (rows && !h->rsum_buf[0])
+            if ((rc = dev_alloc(h, &h->rsum_buf[0], (size_t)(1 + h->d.p) * h->d.C)) ||
+                (rc = dev_alloc(h, &h->rsum_buf[1], (size_t)(1 + h->d.p) * h->d.C)))
+                return rc;
+        double *const *buf = rows ? h->rsum_buf : h->dsum_buf;
+        h->d.dsum_cur = h->dcache ? buf[0] : nullptr;
+        h->d.dsum_prop = h->dcache ? buf[1] : nullptr;
+        h->dc_valid = h->rg_valid = false;
+        if (rows) h->grad_valid = false;
     }
     h->plan_valid = true;
     h->blk_planned = false;
@@ -254,19 +266,27 @@ int32_t ensure_plan(extmcmc_t h) {
 }
 
 // ---- data-sum cache: which elements need no sweep ------------------------------------------------
-// The data term of HIER_NORMAL depends on theta_1..G only.  An element whose update moves none of
-// them (mu, tau) proposes a state with the data sums of the current one; a MALA element that follows
-// such elements finds the sums of its current state still in the cache.  kinds[] carries the fact as
-// kDataFree on top of the transition kernel id; step_advance is the one place that says what an
-// element does to (grad_valid, dc_valid) and is used by the descriptor loop, the graph key, the
-// kernel sequence and the end-of-block state alike.
+// The data term of HIER_NORMAL depends on theta_1..G only; the rows of a user law do not read the
+// coordinates it declares parameter-only (extmcmc_set_user_law_theta_only).  An element whose update
+// moves none of the coordinates the data read (mu, tau) proposes a state with the data sums of the
+// current one; a MALA element that follows such elements finds the sums of its current state still in
+// the cache.  kinds[] carries the fact as kDataFree on top of the transition kernel id; step_advance is
+// the one place that says what an element does to (grad_valid, dc_valid, rg_valid) and is used by the
+// descriptor loop, the graph key, the kernel sequence and the end-of-block state alike.
 constexpr int kDataFree = 0x100;
+// What the cache holds: HIER_NORMAL's per-group sums (their gradient is always valid with them), or a
+// user law's row sums R and Rg (R alone is refilled by a value sweep, and kept across a random walk
+// that moved a row coordinate by the commit kernel: rsum_commit_kernel).
+enum { kCacheNone = 0, kCacheGroups = 1, kCacheRows = 2 };
+int cache_kind(extmcmc_t h) { return !h->dcache ? kCacheNone : h->cfg.law == EXTMCMC_LAW_USER ? kCacheRows : kCacheGroups; }
 int step_kind(extmcmc_t h, int u) {
     const DevUpdate &t = h->upd_host[u];
     int kind = t.kernel;
     if (h->dcache && kind != EXTMCMC_KERNEL_MALA && t.n_coords <= kMaxCoords) {
+        const bool user = h->cfg.law == EXTMCMC_LAW_USER;
         bool moves_data = false;
-        for (int i = 0; i < t.n_coords; ++i) moves_data = moves_data || t.coords[i] < h->d.G;
+        for (int i = 0; i < t.n_coords; ++i)
+            moves_data = moves_data || (user ? !((h->ulaw.theta_only >> t.coords[i]) & 1) : t.coords[i] < h->d.G);
         if (!moves_data) kind |= kDataFree;
     }
     return kind;
@@ -274,24 +294,27 @@ int step_kind(extmcmc_t h, int u) {
 inline bool kind_is_mala(int kind) { return (kind & 0xff) == EXTMCMC_KERNEL_MALA; }
 // MALA: returns how the gradient of the current state is obtained (0 = still valid, 1 = sweep,
 // 2 = from the cache).  Random walk: 0 = the element sweeps its proposal; 1 = it runs from the cache;
-// 2 = the cache is refilled first (gradient sweep of the CURRENT state + per-group reduction -- the
-// kernels and the association that fill it on the MALA path, so a data-free element sees the same
-// bits whether the sums were kept or recomputed: start of a run, after a checkpoint load, after an
-// element that moved a theta_g), then as 1.
-int step_advance(bool dcache, int kind, bool &gv, bool &dc) {
+// 2 = the cache is refilled first (HIER_NORMAL: gradient sweep of the CURRENT state + per-group
+// reduction -- the kernels and the association that fill it on the MALA path, so a data-free element
+// sees the same bits whether the sums were kept or recomputed; user law: value sweep of the CURRENT
+// state into R.  Start of a run, after a checkpoint load, after an element that moved a row
+// coordinate), then as 1.  rv, rgv: dc_valid, rg_valid.
+int step_advance(int cache, int kind, bool &gv, bool &rv, bool &rgv) {
     if (kind_is_mala(kind)) {
-        const int mode = gv ? 0 : (dc ? 2 : 1);
-        if (mode == 1 && dcache) dc = true;   // mala_propose stores the sums it finishes
-        gv = true;                            // (an accepted proposal hands its sums over: mala_decide_commit)
+        const int mode = gv ? 0 : (rv && rgv ? 2 : 1);
+        if (mode == 1 && cache) rv = rgv = true;   // the current-state sweep stores the sums it finishes
+        gv = true;                                 // (an accepted proposal hands its sums over: mala_decide_commit)
         return mode;
     }
     gv = false;
     if (kind & kDataFree) {
-        const int mode = dc ? 1 : 2;
-        dc = true;
+        const int mode = rv ? 1 : 2;
+        if (cache == kCacheGroups) rgv = true;
+        rv = true;
         return mode;
     }
-    dc = false;
+    rgv = false;
+    if (cache != kCacheRows) rv = false;
     return 0;
 }
 
@@ -387,9 +410,11 @@ int32_t ensure_total_obs(extmcmc_t h) {
 // laws read the law constants the proposal kernel left in lawc and leave per-segment sums in
 // `partial` (grad: also the first-order sums).  The logistic law reads the parameters from
 // `src` ([p][C]) and finishes ll (-> ll_dst) and the gradient (-> grad_dst, may be NULL) itself.
+// A user law with parameter-only coordinates finishes its rows into rsum (default: the proposal's
+// buffer) and, unless ll_dst is NULL, adds its parameter-only term from there.
 int32_t enqueue_sweep(extmcmc_t h, bool instrument, bool grad = false, const double *src = nullptr,
                       double *ll_dst = nullptr, double *grad_dst = nullptr,
-                      const StepDesc *d_descs = nullptr, int k = 0) {
+                      const StepDesc *d_descs = nullptr, int k = 0, double *rsum = nullptr) {
     std::pair<cudaEvent_t, cudaEvent_t> ev{nullptr, nullptr};
     bool tail_done = false;   // the sweep kernel itself reduced (and, with p2p, delivered) the sums
     if (instrument) {
@@ -443,8 +468,8 @@ int32_t enqueue_sweep(extmcmc_t h, bool instrument, bool grad = false, const dou
         a.obs = h->obs_dev; a.n_obs = h->n_obs_local; a.theta = src; a.C = h->d.C;
         a.ll_part = h->d.partial; a.g_part = h->d.partial + (size_t)h->plan.S * h->d.C;
         a.err_flag = h->d.err_flag; a.S = h->plan.S;
-        CK(h, launch_sweep_user(h->plan, h->ulaw, a, grad, ll_dst, grad_dst, h->stream));
-        h->launches += user_sweep_launches(h->ulaw, grad);
+        CK(h, launch_sweep_user(h->plan, h->ulaw, a, grad, ll_dst, grad_dst, rsum ? rsum : h->rsum_buf[1], h->stream));
+        h->launches += user_sweep_launches(h->ulaw, grad, ll_dst != nullptr);
         if (instrument) {
             CK(h, cudaEventRecord(ev.second, h->stream));
             h->ev_pending.push_back(ev);
@@ -492,8 +517,17 @@ DevState grad_view(extmcmc_t h) {
     return v;
 }
 
+// The parameter-only kernel of a user law on the row sums of the CURRENT state (data-sum cache)
+int32_t enqueue_theta(extmcmc_t h, bool grad, const double *src, double *ll_dst, double *grad_dst) {
+    CK(h, launch_theta_user(h->ulaw, UserThetaArgs{src, h->rsum_buf[0], h->d.C, ll_dst, grad_dst, h->d.err_flag}, grad,
+                            h->stream));
+    h->launches += 1;
+    return EXTMCMC_OK;
+}
+
 int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, int n_steps,
-                      bool instrument, bool &grad_valid, bool &dc_valid) {
+                      bool instrument, bool &grad_valid, bool &dc_valid, bool &rg_valid) {
+    const bool rows = cache_kind(h) == kCacheRows;
     bool fused = false;      // the proposal of element k was already issued by accept(k-1)
     bool cur_prepared = false;  // accept(k-1) already wrote the law constants of the current state
     for (int k = 0; k < n_steps; ++k) {
@@ -502,14 +536,16 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
         const int dflags = step_deferral_flags(h->d, k, n_steps);
         const bool next_mala = k + 1 < n_steps && kind_is_mala(kinds[k + 1]);
         const bool next_rw = k + 1 < n_steps && !kind_is_mala(kinds[k + 1]);
-        const int mode = step_advance(h->dcache, kinds[k], grad_valid, dc_valid);
+        const int mode = step_advance(cache_kind(h), kinds[k], grad_valid, dc_valid, rg_valid);
         if (kind_is_mala(kinds[k])) {
             const bool logi = law_self_finished(h->cfg.law);   // the sweep finishes ll and gradient
             int finalize_cur = 0;
             DevState gv = grad_view(h);
             if (mode == 1) {
                 if (logi) {
-                    if ((rc = enqueue_sweep(h, instrument, true, h->d.theta, h->scratch_ll, h->d.grad_cur))) return rc;
+                    if ((rc = enqueue_sweep(h, instrument, true, h->d.theta, h->scratch_ll, h->d.grad_cur, nullptr, 0,
+                                            h->rsum_buf[0])))
+                        return rc;
                 } else {
                     // current-state gradient sweep; its sums are finished inside mala_propose
                     const bool hier = h->cfg.law == EXTMCMC_LAW_HIER_NORMAL;   // no law constants to prepare
@@ -517,6 +553,9 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
                     if ((rc = enqueue_sweep(h, instrument, true, h->d.theta))) return rc;
                     finalize_cur = 1;
                 }
+            } else if (mode == 2 && rows) {
+                // R and Rg of the current state are in the cache: only its parameter-only term is evaluated
+                if ((rc = enqueue_theta(h, true, h->d.theta, h->scratch_ll, h->d.grad_cur))) return rc;
             } else if (mode == 2) {
                 // the sums of the current state are in the cache: mala_propose finishes them from there
                 gv.partial = h->d.dsum_cur; gv.S = 1;
@@ -536,19 +575,30 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
         } else {
             if (!fused) { launch_propose(h->d, d_descs, k, h->stream); h->launches += 1; }
             const bool from_cache = mode != 0;
-            if (mode == 2) {
+            if (mode == 2 && rows) {
+                // R of the current state (the proposal's own: no row coordinate moved)
+                if ((rc = enqueue_sweep(h, instrument, false, h->d.theta, nullptr, nullptr, nullptr, 0, h->rsum_buf[0])))
+                    return rc;
+            } else if (mode == 2) {
                 if ((rc = enqueue_sweep(h, instrument, true, h->d.theta))) return rc;
                 launch_reduce_group_sums(h->d, h->d.dsum_cur, h->stream);
                 h->launches += 1;
             }
-            if (!from_cache)
+            if (from_cache && rows) {
+                if ((rc = enqueue_theta(h, false, h->d.prop_full, h->d.ssum, nullptr))) return rc;
+            } else if (!from_cache) {
                 if ((rc = enqueue_sweep(h, instrument, false, h->d.prop_full, h->d.ssum, nullptr, d_descs, k))) return rc;
+            }
             fused = next_rw;
             // a MALA element follows and will need the law constants of the (then) current state for
             // its gradient sweep: let this accept kernel write them (fuse_next = 2)
             cur_prepared = next_mala && !law_self_finished(h->cfg.law) && h->cfg.law != EXTMCMC_LAW_HIER_NORMAL;
-            launch_accept(h->d, d_descs, k, fused ? 1 : (cur_prepared ? 2 : 0), dflags, h->stream, from_cache);
+            launch_accept(h->d, d_descs, k, fused ? 1 : (cur_prepared ? 2 : 0), dflags, h->stream, from_cache && !rows);
             h->launches += 1;
+            if (rows && mode == 0 && dc_valid) {   // the accepted proposals' R becomes the current state's
+                launch_rsum_commit(h->d, d_descs, k, h->stream);
+                h->launches += 1;
+            }
         }
     }
     CK(h, cudaGetLastError());
@@ -591,7 +641,7 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
     if ((rc = ensure_total_obs(h))) return rc;
     if ((rc = plan_block_kernels(h))) return rc;
     if ((h->res_ok || h->obsblk_ok) && h->dcache) {   // the persistent block kernels sweep for every element
-        h->dcache = h->dc_valid = false;
+        h->dcache = h->dc_valid = h->rg_valid = false;
         h->d.dsum_cur = h->d.dsum_prop = nullptr;
     }
     // a history fetch still in flight reads ring slots this block is about to overwrite: order the
@@ -644,7 +694,7 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
     const int W = h->d.W;
     int n_sweeps = 0;
     {
-        bool gv = h->grad_valid, dc = h->dc_valid;
+        bool gv = h->grad_valid, dc = h->dc_valid, rg = h->rg_valid;
         for (int s = 0; s < n_steps; ++s) {
             StepDesc &sd = sl.h_descs[s];
             const int u = steps[s].pidx;
@@ -675,7 +725,7 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
             }
             const bool mala = h->upd_host[u].kernel == EXTMCMC_KERNEL_MALA;
             sd.need_cur_grad = (mala && !gv) ? 1 : 0;
-            const int mode = step_advance(h->dcache, step_kind(h, u), gv, dc);
+            const int mode = step_advance(cache_kind(h), step_kind(h, u), gv, dc, rg);
             n_sweeps += mala ? 1 + (mode == 1 ? 1 : 0) : (mode == 1 ? 0 : 1);
             h->ra_iter[u] = it;
             tag = it;
@@ -688,7 +738,8 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
         kinds[s] = step_kind(h, steps[s].pidx);
         hash = (hash ^ (unsigned long long)kinds[s]) * 1099511628211ull;
     }
-    hash = (hash ^ (unsigned long long)((h->grad_valid ? 7 : 3) + (h->dc_valid ? 16 : 0))) * 1099511628211ull;
+    hash = (hash ^ (unsigned long long)((h->grad_valid ? 7 : 3) + (h->dc_valid ? 16 : 0) + (h->rg_valid ? 32 : 0))) *
+           1099511628211ull;
     hash = (hash ^ (unsigned long long)n_steps) * 1099511628211ull;
     const bool instrument = h->cfg.instrument != 0;
     const bool use_graph = h->cfg.use_graphs && !instrument && rng_mode == EXTMCMC_RNG_PHILOX;
@@ -730,11 +781,12 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
             h->ev_pending.push_back(ev);
         }
         h->grad_valid = kind_is_mala(kinds[n_steps - 1]);
-        h->dc_valid = false;
+        h->dc_valid = h->rg_valid = false;
     } else if (!use_graph) {
         CK(h, cudaMemcpyAsync(sl.d_descs, sl.h_descs, sizeof(StepDesc) * n_steps,
                               cudaMemcpyHostToDevice, h->stream));
-        if ((rc = enqueue_steps(h, sl.d_descs, kinds.data(), n_steps, instrument, h->grad_valid, h->dc_valid))) return rc;
+        if ((rc = enqueue_steps(h, sl.d_descs, kinds.data(), n_steps, instrument, h->grad_valid, h->dc_valid, h->rg_valid)))
+            return rc;
     } else {
         // the kernel sequence depends on the kinds of the block's updates (and on whether the
         // current-state gradient is fresh), not on which update each element names
@@ -742,12 +794,12 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
         auto it = h->graphs.find(key);
         if (it == h->graphs.end()) {
             const int64_t launches_before = h->launches;
-            bool gv = h->grad_valid, dc = h->dc_valid;
+            bool gv = h->grad_valid, dc = h->dc_valid, rg = h->rg_valid;
             cudaGraph_t g = nullptr;
             CK(h, cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
             cudaError_t e1 = cudaMemcpyAsync(sl.d_descs, sl.h_descs, sizeof(StepDesc) * n_steps,
                                              cudaMemcpyHostToDevice, h->stream);
-            int32_t rc2 = e1 == cudaSuccess ? enqueue_steps(h, sl.d_descs, kinds.data(), n_steps, false, gv, dc) : EXTMCMC_ECUDA;
+            int32_t rc2 = e1 == cudaSuccess ? enqueue_steps(h, sl.d_descs, kinds.data(), n_steps, false, gv, dc, rg) : EXTMCMC_ECUDA;
             cudaError_t e2 = cudaStreamEndCapture(h->stream, &g);
             h->graph_launches[key] = h->launches - launches_before;
             h->launches = launches_before;
@@ -764,7 +816,7 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
         }
         CK(h, cudaGraphLaunch(it->second, h->stream));
         h->launches += h->graph_launches[key];
-        for (int s = 0; s < n_steps; ++s) step_advance(h->dcache, kinds[s], h->grad_valid, h->dc_valid);
+        for (int s = 0; s < n_steps; ++s) step_advance(cache_kind(h), kinds[s], h->grad_valid, h->dc_valid, h->rg_valid);
     }
     CK(h, cudaEventRecord(sl.done, h->stream));
     sl.in_flight = true;
@@ -870,6 +922,7 @@ int32_t extmcmc_create(const extmcmc_config_t *cfg, extmcmc_t *out) {
     d.p_u_max = 1; d.seed = cfg->seed;
     d.obs_dim = cfg->obs_dim;
     d.G = cfg->law == EXTMCMC_LAW_HIER_NORMAL ? cfg->n_params - 2 : 1;
+    d.dsum_rows = cfg->law == EXTMCMC_LAW_USER ? 1 + cfg->n_params : 2 * d.G;
     d.lawc_k = cfg->law == EXTMCMC_LAW_GSN_IID_1D ? 3
              : law_self_finished(cfg->law) ? 1
              : cfg->law == EXTMCMC_LAW_HIER_NORMAL ? d.G
@@ -996,7 +1049,7 @@ static int32_t install_obs(extmcmc_t h, int64_t n_obs, const std::vector<int64_t
     h->plan_valid = false;
     h->n_total_known = false;
     h->grad_valid = false;
-    h->dc_valid = false;
+    h->dc_valid = h->rg_valid = false;
     return EXTMCMC_OK;
 }
 
@@ -1027,7 +1080,7 @@ int32_t extmcmc_upload_obs(extmcmc_t h, const double *obs, int64_t n_obs, int32_
         h->plan_valid = false;
         h->n_total_known = false;
         h->grad_valid = false;
-        h->dc_valid = false;
+        h->dc_valid = h->rg_valid = false;
         return EXTMCMC_OK;
     }
     if (h->cfg.law == EXTMCMC_LAW_USER) {
@@ -1044,7 +1097,7 @@ int32_t extmcmc_upload_obs(extmcmc_t h, const double *obs, int64_t n_obs, int32_
         h->plan_valid = false;
         h->n_total_known = false;
         h->grad_valid = false;
-        h->dc_valid = false;
+        h->dc_valid = h->rg_valid = false;
         return EXTMCMC_OK;
     }
     std::vector<int64_t> glen(h->d.G, 0);
@@ -1261,6 +1314,7 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
     h->upd_set[u] = true;
     h->upd_dirty = true;
     h->blk_planned = false;
+    if (h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.theta_only) h->grad_valid = h->dc_valid = h->rg_valid = false;
     int nh = 0;
     h->any_mala = false;
     for (int v = 0; v < h->cfg.n_updates; ++v) {
@@ -1328,7 +1382,7 @@ int32_t extmcmc_set_state(extmcmc_t h, const double *theta) {
     std::fill(h->haario_M.begin(), h->haario_M.end(), 0);
     h->seq_next = 0;
     h->grad_valid = false;
-    h->dc_valid = false;
+    h->dc_valid = h->rg_valid = false;
     if (h->fetch_active) { cudaEventSynchronize(h->fetch_done); h->fetch_active = false; }
     std::fill(h->ra_iter.begin(), h->ra_iter.end(), 0);
     std::fill(h->acc_tag.begin(), h->acc_tag.end(), 0);
@@ -1356,13 +1410,29 @@ void copy_log(const std::string &msg, char *log, int64_t log_bytes) {
     }
 }
 // The options of every user-law entry point, checked and resolved to a UserGrad mode and the chunk
-// width K of forward mode.  chunked: the width comes from `chunk` (the _chunked and _ex entry points);
-// otherwise forward mode is the unchunked program and keeps its limit of kUserMaxForwardParams.
-int32_t user_law_options(int32_t P, int32_t with_grad, bool chunked, int32_t chunk, int32_t flags, int &mode, int &K,
-                         std::string &err) {
+// width K of forward mode.  chunked: the width comes from `chunk` (the _chunked, _ex and _theta_only
+// entry points); otherwise forward mode is the unchunked program and keeps its limit of
+// kUserMaxForwardParams.  declared: the _theta_only entry points, whose theta_only must name at least
+// one coordinate below P and needs EXTMCMC_USER_THETA_TERM (the other entry points pass 0).
+int32_t user_law_options(int32_t P, int32_t with_grad, bool chunked, int32_t chunk, int32_t flags, bool declared,
+                         uint64_t theta_only, int &mode, int &K, std::string &err) {
     if (flags & ~EXTMCMC_USER_THETA_TERM) {
         err = "unknown user-law flags " + std::to_string(flags) + " (known: EXTMCMC_USER_THETA_TERM = 1)";
         return EXTMCMC_EINVAL;
+    }
+    if (declared) {
+        if (!(flags & EXTMCMC_USER_THETA_TERM)) {
+            err = "theta_only needs flags with EXTMCMC_USER_THETA_TERM: only logpdf_theta may read those coordinates";
+            return EXTMCMC_EINVAL;
+        }
+        if (theta_only == 0) {
+            err = "theta_only declares no coordinate (bit k = 0-based coordinate k)";
+            return EXTMCMC_EINVAL;
+        }
+        if (P < 64 && (theta_only >> P)) {
+            err = "theta_only names a coordinate at or above n_params = " + std::to_string(P) + " (bit k = 0-based coordinate k)";
+            return EXTMCMC_EINVAL;
+        }
     }
     mode = user_grad_mode(with_grad);
     K = P;
@@ -1378,43 +1448,44 @@ int32_t user_law_options(int32_t P, int32_t with_grad, bool chunked, int32_t chu
 }
 // every extmcmc_user_law_check* entry point
 int32_t user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad, bool chunked,
-                       int32_t chunk, int32_t flags, int32_t *chunk_used, char *log, int64_t log_bytes) {
+                       int32_t chunk, int32_t flags, bool declared, uint64_t theta_only, int32_t *chunk_used, char *log,
+                       int64_t log_bytes) {
     if (log && log_bytes > 0) log[0] = 0;
     if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
     if (n_params < 1 || n_params > kUserMaxParams || obs_dim < 1 || obs_dim > kUserMaxObsDim)
         return fail(nullptr, EXTMCMC_EUNSUPPORTED, "user laws need 1 <= n_params <= 64 and 1 <= obs_dim <= 64");
     int mode = kUserValue, K = 0;
     std::string err;
-    if (const int32_t rc = user_law_options(n_params, with_grad, chunked, chunk, flags, mode, K, err)) {
+    if (const int32_t rc = user_law_options(n_params, with_grad, chunked, chunk, flags, declared, theta_only, mode, K, err)) {
         copy_log(err, log, log_bytes);
         return fail(nullptr, rc, err);
     }
     if (chunk_used) *chunk_used = mode == kUserGradForward ? K : 0;
     std::string lg, cubin;
-    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, K, flags, lg, cubin, nullptr);
+    const int32_t rc = user_law_compile(source, n_params, obs_dim, mode, K, flags, theta_only, lg, cubin, nullptr);
     copy_log(lg, log, log_bytes);
     if (rc) g_create_error = lg;
     return rc;
 }
 // every extmcmc_set_user_law* entry point; entry: its name, for the messages
 int32_t set_user_law(extmcmc_t h, const char *entry, const char *source, int32_t with_grad, bool chunked,
-                     int32_t chunk, int32_t flags) {
+                     int32_t chunk, int32_t flags, bool declared = false, uint64_t theta_only = 0) {
     if (!h) return EXTMCMC_EINVAL;
     if (h->cfg.law != EXTMCMC_LAW_USER) return fail(h, EXTMCMC_EINVAL, std::string(entry) + " needs a handle of law EXTMCMC_LAW_USER");
     if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
     int mode = kUserValue, K = 0;
     std::string err;
-    if (const int32_t rc = user_law_options(h->cfg.n_params, with_grad, chunked, chunk, flags, mode, K, err))
+    if (const int32_t rc = user_law_options(h->cfg.n_params, with_grad, chunked, chunk, flags, declared, theta_only, mode, K, err))
         return fail(h, rc, err);
     std::string log, cubin;
     uint64_t hash = 0;
-    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, K, flags, log, cubin, &hash);
+    const int32_t rc = user_law_compile(source, h->cfg.n_params, h->cfg.obs_dim, mode, K, flags, theta_only, log, cubin, &hash);
     if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user law does not compile:\n" + log);
     if (rc) return fail(h, rc, log);
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
     invalidate_graphs(h);
-    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, mode, K, hash);
+    const cudaError_t e = user_law_load(h->ulaw, cubin, h->cfg.n_params, h->cfg.obs_dim, mode, K, theta_only, hash);
     if (e != cudaSuccess) {
         user_law_unload(h->ulaw);
         return fail(h, EXTMCMC_ECUDA, std::string("loading the user law: ") + cudaGetErrorString(e));
@@ -1428,18 +1499,25 @@ extern "C" {
 
 int32_t extmcmc_user_law_check(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                char *log, int64_t log_bytes) {
-    return user_law_check(source, n_params, obs_dim, with_grad, false, 0, 0, nullptr, log, log_bytes);
+    return user_law_check(source, n_params, obs_dim, with_grad, false, 0, 0, false, 0, nullptr, log, log_bytes);
 }
 
 int32_t extmcmc_user_law_check_chunked(const char *source, int32_t n_params, int32_t obs_dim, int32_t chunk,
                                        int32_t *chunk_used, char *log, int64_t log_bytes) {
-    return user_law_check(source, n_params, obs_dim, EXTMCMC_USER_GRAD_FORWARD, true, chunk, 0, chunk_used, log,
+    return user_law_check(source, n_params, obs_dim, EXTMCMC_USER_GRAD_FORWARD, true, chunk, 0, false, 0, chunk_used, log,
                           log_bytes);
 }
 
 int32_t extmcmc_user_law_check_ex(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
                                   int32_t chunk, int32_t flags, int32_t *chunk_used, char *log, int64_t log_bytes) {
-    return user_law_check(source, n_params, obs_dim, with_grad, true, chunk, flags, chunk_used, log, log_bytes);
+    return user_law_check(source, n_params, obs_dim, with_grad, true, chunk, flags, false, 0, chunk_used, log, log_bytes);
+}
+
+int32_t extmcmc_user_law_check_theta_only(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                                          int32_t chunk, int32_t flags, uint64_t theta_only, int32_t *chunk_used,
+                                          char *log, int64_t log_bytes) {
+    return user_law_check(source, n_params, obs_dim, with_grad, true, chunk, flags, true, theta_only, chunk_used, log,
+                          log_bytes);
 }
 
 int32_t extmcmc_set_user_law(extmcmc_t h, const char *source, int32_t with_grad) {
@@ -1452,6 +1530,11 @@ int32_t extmcmc_set_user_law_chunked(extmcmc_t h, const char *source, int32_t ch
 
 int32_t extmcmc_set_user_law_ex(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags) {
     return set_user_law(h, "extmcmc_set_user_law_ex", source, with_grad, true, chunk, flags);
+}
+
+int32_t extmcmc_set_user_law_theta_only(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags,
+                                        uint64_t theta_only) {
+    return set_user_law(h, "extmcmc_set_user_law_theta_only", source, with_grad, true, chunk, flags, true, theta_only);
 }
 
 // ---- checkpoint / resume ------------------------------------------------------------------------
@@ -1552,7 +1635,7 @@ int32_t extmcmc_checkpoint_load(extmcmc_t h, const void *blob, int64_t bytes) {
     });
     if (rc) return rc;
     h->seq_next = hd.seq_next;
-    h->dc_valid = false;
+    h->dc_valid = h->rg_valid = false;
     h->grad_valid = false;          // (the gradient buffers are not part of the blob: recomputed on demand)
     h->state_set = true;
     h->fetch_active = false;

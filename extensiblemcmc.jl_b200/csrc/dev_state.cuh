@@ -95,13 +95,15 @@ struct DevState {
                             // the launchers pick the SpecLean instantiations (step_device.cuh)
     int32_t obs_dim, lawc_k;  // observation dimension; per-chain law constants in lawc
     int32_t G;              // observation groups (HIER_NORMAL; 1 otherwise)
+    int32_t dsum_rows;      // rows per chain of dsum_cur / dsum_prop: 2 G (HIER_NORMAL), 1 + p (USER)
     double *ll_prop;        // [C] finalized proposal log-likelihood (gradient path)
     double *grad_cur;       // [p][C] d ll / d theta at the current state
     double *grad_prop;      // [p][C] ... at the proposal
-    // Data-sum cache (HIER_NORMAL, api.cu: data_cache_on): the per-group sums of both orders of the
-    // CURRENT state and of the proposal in flight, laid out like a partial buffer with one segment per
-    // group ([2][G][C]).  They depend on theta_1..G only, so an update of mu / tau reuses them instead
-    // of streaming the observations again.  NULL: no cache.
+    // Data-sum cache (api.cu: ensure_plan): the sums of the CURRENT state and of the proposal in flight.
+    // HIER_NORMAL: the per-group sums of both orders, laid out like a partial buffer with one segment per
+    // group ([2][G][C]); they depend on theta_1..G only, so an update of mu / tau reuses them instead of
+    // streaming the observations again.  A user law with parameter-only coordinates: the row sums R and
+    // their gradient Rg ([1 + p][C]).  NULL: no cache.
     double *dsum_cur, *dsum_prop;
     uint64_t seed;
     // current state

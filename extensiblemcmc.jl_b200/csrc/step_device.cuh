@@ -981,8 +981,8 @@ __device__ __forceinline__ Decision mala_decide_commit(const DevState &d, const 
 #pragma unroll
             for (int q = 0; q < 4; ++q) if (j0 + q < d.p) d.grad_cur[(int64_t)(j0 + q) * C + c] = g[q];
         }
-        if (HANDOVER && d.dsum_cur) {   // data-sum cache: the proposal's per-group sums become the current state's
-            const int rows = 2 * d.G;
+        if (HANDOVER && d.dsum_cur) {   // data-sum cache: the proposal's sums become the current state's
+            const int rows = d.dsum_rows;
             for (int r0 = 0; r0 < rows; r0 += 4) {
                 double g[4];
 #pragma unroll
@@ -995,14 +995,14 @@ __device__ __forceinline__ Decision mala_decide_commit(const DevState &d, const 
     return Decision{accepted, ll_new, ll_prop};
 }
 // What an accepted MALA proposal hands over to the current state -- the gradient and, with the data-sum
-// cache, the per-group sums: p + 2 G rows per chain, copied by the threads of slices [s0, s0 + ns) of an
+// cache, its sums: p + dsum_rows rows per chain, copied by the threads of slices [s0, s0 + ns) of an
 // nch-chains-per-slice CTA (acc[ch] = the chain's decision, written before a CTA barrier).
 __device__ __forceinline__ void mala_handover_coop(const DevState &d, int64_t c0, int nch, const uint8_t *acc,
                                                    int tid, int s0, int ns) {
     const int ch = tid % nch, slice = tid / nch - s0;
     const int64_t C = d.C, c = c0 + ch;
     if (slice < 0 || slice >= ns || c >= C || !acc[ch]) return;
-    const int rows = d.p + (d.dsum_cur ? 2 * d.G : 0);
+    const int rows = d.p + (d.dsum_cur ? d.dsum_rows : 0);
 #pragma unroll 2
     for (int r = slice; r < rows; r += ns) {
         if (r < d.p) d.grad_cur[(int64_t)r * C + c] = d.grad_prop[(int64_t)r * C + c];

@@ -533,6 +533,16 @@ mala_accept_kernel(DevState d, const StepDesc *__restrict__ descs, int k, int fi
     if (worker && fuse_next) propose_chain<SP>(d, ctx_next.sd, ctx_next.u, c);
 }
 
+// Row-sum cache of a user law (api.cu): an accepted random-walk proposal that moved a coordinate the rows
+// read hands the row sum R of its sweep over to the current state.  After the accept kernel, which wrote
+// the decision into the history row of descs[k].
+__global__ void __launch_bounds__(256)
+rsum_commit_kernel(DevState d, const StepDesc *__restrict__ descs, int k) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= d.C) return;
+    if (d.h_acc[(descs[k].seq % d.H) * d.gC + d.g0 + c]) d.dsum_cur[c] = d.dsum_prop[c];
+}
+
 // ---------------------------------------------------------------------------------
 // utilities
 // ---------------------------------------------------------------------------------
@@ -665,6 +675,9 @@ void launch_accept(const DevState &d0, const StepDesc *descs, int k, int fuse_ne
         else if (sl == 8) cudaLaunchKernelEx(&cfg, accept_kernel<8, SP>, d, descs, k, fuse_next, flags);
         else cudaLaunchKernelEx(&cfg, accept_kernel<1, SP>, d, descs, k, fuse_next, flags);
     });
+}
+void launch_rsum_commit(const DevState &d, const StepDesc *descs, int k, cudaStream_t st) {
+    rsum_commit_kernel<<<blocks_for(d.C), 256, 0, st>>>(d, descs, k);
 }
 void launch_grad_finalize(const DevState &d, const double *src, double *ll_out, double *grad_out,
                           cudaStream_t st) {

@@ -12,6 +12,8 @@ void launch_accept(const DevState &d, const StepDesc *descs, int k, int fuse_nex
 void launch_prepare_current(const DevState &d, cudaStream_t st);
 // lower Cholesky factors of `count` column-major n x n matrices (element stride `stride`, matrix c at + c)
 void launch_chol_factor(double *S, double *L, int n, int64_t stride, int64_t count, cudaStream_t st);
+// user-law row-sum cache: R of an accepted random-walk proposal -> the current state's (api.cu)
+void launch_rsum_commit(const DevState &d, const StepDesc *descs, int k, cudaStream_t st);
 void launch_grad_finalize(const DevState &d, const double *src, double *ll_out, double *grad_out, cudaStream_t st);
 void launch_mala_propose(const DevState &d, const StepDesc *descs, int k, int finalize_cur, double *ll_scratch,
                          int flags, cudaStream_t st);

@@ -74,8 +74,19 @@ struct UserSweepArgs {
     int S;
 };
 
+// The parameter-only kernel of a law that declares coordinates its rows do not read (EXTMCMC_THETA_ONLY):
+// its sweeps leave the row sums R (and Rg) in rsum, and this kernel adds the term per chain.
+struct UserThetaArgs {
+    const double *theta;   // [P][C] the evaluated state
+    const double *rsum;    // [1 + P][C] row sums of a state with the same row coordinates: R, then Rg (GRAD)
+    int64_t C;
+    double *ll;            // [C]
+    double *grad;          // [P][C] (GRAD)
+    int32_t *err_flag;     // set when a chain's set_parameters returns false
+};
+
 #ifdef __CUDACC_RTC__
-#ifdef EXTMCMC_THETA_TERM
+#if defined(EXTMCMC_THETA_TERM) && !defined(EXTMCMC_THETA_ONLY)
 // Adds the law's parameter-only term (EXTMCMC_USER_THETA_TERM) to a chain's sums: its value to ll and,
 // with a gradient, its derivatives in the coordinates of the sweep's accumulators to g[0..NG-1] --
 // logpdf_theta_grad on a zeroed t (hand-written), or the tangents of logpdf_theta on the Law<Dual<K>> of
@@ -103,7 +114,8 @@ __device__ __forceinline__ void user_add_theta_term(const LawT &L, double &ll, d
 // K, CI: chunk width and chunk index of a forward-mode sweep (LawT = Law<Dual<K>>); chunk 0 writes
 // ll_part and raises err_flag, every chunk writes only its own rows g_part[S][CI*K ..][C].
 // With EXTMCMC_THETA_TERM the CTAs of segment 0 add the law's parameter-only term to the sums of their
-// own rows (user_add_theta_term).
+// own rows (user_add_theta_term); with EXTMCMC_THETA_ONLY too the sweep sums rows only, and
+// user_theta adds the term to the finished sums.
 template <class LawT, int P, int D, int R, int L, int G, int K = P, int CI = 0>
 __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
     constexpr bool GRAD = G != kUserValue;
@@ -215,7 +227,7 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int64_t c = cbase + (L == 1 ? (int64_t)r * kUserNT + tid : (int64_t)(tid / L));
-#ifdef EXTMCMC_THETA_TERM
+#if defined(EXTMCMC_THETA_TERM) && !defined(EXTMCMC_THETA_ONLY)
         // Segment 0 adds the term once per chain to the sums of its rows.  The lanes of a chain are reduced
         // first: all of them then hold the sums, and all evaluate the term (the warp stays converged), and
         // the term is not held in registers across the shuffles.
@@ -257,6 +269,73 @@ __device__ __forceinline__ void user_sweep(const UserSweepArgs &a) {
         if (WRITE_LL && lane == 0 && c < C && !ok[r] && seg == 0) *a.err_flag = 1;
     }
 }
+
+#ifdef EXTMCMC_THETA_ONLY
+// One thread per chain: ll = fl(R + logpdf_theta) and, with a gradient, g_k = fl(Rg_k + t_k).  t comes
+// from logpdf_theta_grad on a zeroed t[P] (hand-written) or from the tangents of logpdf_theta on
+// Law<Dual<K>>, one chunk after the other (forward mode; the value from chunk 0).  Domain and canonical
+// NaN exactly as in user_sweep: set_parameters false.  PDL as in user_sweep.
+template <class LawT, int P, int G, int K = P>
+__device__ __forceinline__ void user_theta(const UserThetaArgs &a) {
+    griddep_wait();
+    griddep_launch_dependents();
+    const int64_t C = a.C;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    const double R = a.rsum[c];
+    bool ok;
+    if constexpr (G == kUserGradForward) {
+        constexpr int NC = (P + K - 1) / K;
+        ok = true;
+#pragma unroll
+        for (int ci = 0; ci < NC; ++ci) {
+            Dual<K> th[P];
+#pragma unroll
+            for (int k = 0; k < P; ++k) {
+                th[k].v = a.theta[(int64_t)k * C + c];
+#pragma unroll
+                for (int j = 0; j < K; ++j) th[k].t[j] = ci * K + j == k ? 1.0 : 0.0;
+            }
+            LawT law;
+            const bool okc = set_parameters(law, th);
+            ok = ok && okc;
+            if (!okc) continue;
+            const auto t = logpdf_theta(law);
+            if (ci == 0) a.ll[c] = R + t.v;
+#pragma unroll
+            for (int j = 0; j < K; ++j)
+                if (ci * K + j < P) a.grad[(int64_t)(ci * K + j) * C + c] = a.rsum[(int64_t)(1 + ci * K + j) * C + c] + t.t[j];
+        }
+    } else {
+        double th[P];
+#pragma unroll
+        for (int k = 0; k < P; ++k) th[k] = a.theta[(int64_t)k * C + c];
+        LawT law;
+        ok = set_parameters(law, th);
+        if (ok) {
+            if constexpr (G == kUserGradHand) {
+                double t[P];
+#pragma unroll
+                for (int k = 0; k < P; ++k) t[k] = 0.0;
+                a.ll[c] = R + logpdf_theta_grad(law, t);
+#pragma unroll
+                for (int k = 0; k < P; ++k) a.grad[(int64_t)k * C + c] = a.rsum[(int64_t)(1 + k) * C + c] + t[k];
+            } else {
+                a.ll[c] = R + logpdf_theta(law);
+            }
+        }
+    }
+    if (!ok) {
+        a.ll[c] = nan;
+        if constexpr (G != kUserValue) {
+#pragma unroll
+            for (int k = 0; k < P; ++k) a.grad[(int64_t)k * C + c] = nan;
+        }
+        *a.err_flag = 1;
+    }
+}
+#endif
 #endif
 
 }  // namespace extmcmc

@@ -336,6 +336,30 @@ int32_t extmcmc_user_law_check_ex(const char *source, int32_t n_params, int32_t 
 /* extmcmc_set_user_law with the arguments of extmcmc_user_law_check_ex.  A checkpoint written by a law
  * compiled with other flags is refused (EXTMCMC_EINVAL). */
 int32_t extmcmc_set_user_law_ex(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags);
+/* Parameter-only coordinates (theta_only; bit k = 0-based coordinate k): coordinates that logpdf (and
+ * logpdf_grad) does not depend on -- the value and gradient of every row depend only on the other
+ * coordinates.  Only logpdf_theta may read them; set_parameters may read every coordinate.  Such a law
+ * is compiled as a program variant (EXTMCMC_THETA_ONLY = the mask, part of the NVRTC input and of the
+ * law hash): its sweeps sum rows only, and a per-chain kernel adds logpdf_theta to the row sums.  The
+ * handle then keeps the row sums R and their gradient of the current state, so that a random-walk update
+ * that moves only parameter-only coordinates (the mu and tau of a hierarchical model, a prior precision)
+ * runs without a likelihood sweep, and a MALA update after it finds the rows' part of its current
+ * gradient still valid.  EXTMCMC_DATA_CACHE=0 (read per plan) turns this cache off: every element then
+ * sweeps, with the same program and kernels, and gives the same bits, log-likelihoods included.
+ * The list is declared, not detected, and not verified: a false declaration gives wrong sums.  The
+ * check is to run the same seed with EXTMCMC_DATA_CACHE=0 and compare: a true declaration gives
+ * bit-identical histories (with logpdf_grad, when it returns the value logpdf returns, bit for bit).
+ * Against the same source without the declaration, the term is added to the finished row sums instead
+ * of to segment 0: ll and gradient agree to rounding (one addition associated differently).
+ * flags must contain EXTMCMC_USER_THETA_TERM; theta_only must be non-zero and name coordinates below
+ * n_params; otherwise EXTMCMC_EINVAL, with a message and without compiling.  The other arguments are
+ * those of extmcmc_user_law_check_ex.  A checkpoint is refused across different declarations, and
+ * between a declared and an undeclared law. */
+int32_t extmcmc_user_law_check_theta_only(const char *source, int32_t n_params, int32_t obs_dim, int32_t with_grad,
+                                          int32_t chunk, int32_t flags, uint64_t theta_only, int32_t *chunk_used,
+                                          char *log, int64_t log_bytes);
+int32_t extmcmc_set_user_law_theta_only(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags,
+                                        uint64_t theta_only);
 
 /* Replaces RandomWalkUpdate(rw, coords; prior, adpt) src/updates.jl:170-182. */
 int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd);

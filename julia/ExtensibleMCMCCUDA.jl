@@ -105,7 +105,7 @@ struct LogisticLaw; d::Int; end
 struct HierNormalLaw; G::Int; end
 
 """
-    DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false)
+    DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false, theta_only=Int[])
 
 A user-defined law on the device (EXTMCMC_LAW_USER): the counterparts of `set_parameters!(P, θ)` and
 one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_parameters`, `logpdf`, and
@@ -116,6 +116,9 @@ one term of `loglikelihood(P, obs)`, written in CUDA C++ (`struct Law`, `set_par
 ForwardDiff's chunk mode: `law.chunk` is the width the library compiled).  With `theta_term = true` the
 source also defines `logpdf_theta` (and `logpdf_theta_grad` with `gradient = true`), a term of θ only
 that is added once to the log-likelihood, such as the hierarchical p(θ_g | μ, τ) of a multilevel model.
+`theta_only` (1-based, like the updates' coordinates; needs `theta_term = true`) declares coordinates the
+rows do not read, only `logpdf_theta`: a random-walk update of those alone then runs without a likelihood
+sweep (include/extmcmc.h, extmcmc_set_user_law_theta_only).
 Compiled for sm_100a when constructed (no device needed); a source that does not
 compile throws with the compiler's log.  data = (P = DeviceLaw(...), obs = rows of obs_dim values);
 responses are columns of the rows.
@@ -128,8 +131,10 @@ struct DeviceLaw
     chunk_arg::Int32                                     # -1: unchunked; 0: the library's width; K
     chunk::Int                                           # forward mode: the width compiled (0 otherwise)
     flags::Int32                                         # USER_THETA_TERM or 0
+    theta_only::UInt64                                   # bit k = 0-based coordinate k; 0: none declared
     log::String
-    function DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false)
+    function DeviceLaw(source::String, n_params, obs_dim; gradient=false, chunk=nothing, theta_term=false,
+                       theta_only=Int[])
         with_grad = gradient === :forward ? USER_GRAD_FORWARD :
                     gradient === true ? USER_GRAD_HAND :
                     gradient === false ? USER_GRAD_NONE :
@@ -141,9 +146,19 @@ struct DeviceLaw
                     throw(ArgumentError("chunk must be nothing, :auto or a positive width, not $(repr(chunk))"))
         theta_term isa Bool || throw(ArgumentError("theta_term must be true or false, not $(repr(theta_term))"))
         flags = theta_term ? USER_THETA_TERM : Int32(0)
+        isempty(theta_only) || theta_term || throw(ArgumentError("theta_only needs theta_term = true"))
+        allunique(theta_only) || throw(ArgumentError("theta_only lists a coordinate twice: $(repr(theta_only))"))
+        all(k -> k isa Integer && !(k isa Bool) && 1 <= k <= n_params, theta_only) ||
+            throw(ArgumentError("theta_only must hold coordinates in 1:$n_params, not $(repr(theta_only))"))
+        mask = reduce(|, (UInt64(1) << (k - 1) for k in theta_only); init=UInt64(0))
         buf = zeros(UInt8, 1 << 16)
         used = Ref{Int32}(with_grad == USER_GRAD_FORWARD ? n_params : 0)
-        rc = if theta_term                               # chunk: nothing in forward mode is the width n_params
+        rc = if mask != 0
+            GC.@preserve buf ccall((:extmcmc_user_law_check_theta_only, LIB), Int32,
+                                   (Cstring, Int32, Int32, Int32, Int32, Int32, UInt64, Ptr{Int32}, Ptr{UInt8}, Int64),
+                                   source, n_params, obs_dim, with_grad, ex_chunk(with_grad, chunk_arg, n_params),
+                                   flags, mask, used, pointer(buf), length(buf))
+        elseif theta_term                                # chunk: nothing in forward mode is the width n_params
             GC.@preserve buf ccall((:extmcmc_user_law_check_ex, LIB), Int32,
                                    (Cstring, Int32, Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{UInt8}, Int64),
                                    source, n_params, obs_dim, with_grad, ex_chunk(with_grad, chunk_arg, n_params),
@@ -159,7 +174,7 @@ struct DeviceLaw
         end
         log = unsafe_string(pointer(buf))
         rc == 0 || throw(ArgumentError("the device law does not compile (status $rc):\n" * log))
-        new(source, n_params, obs_dim, with_grad, chunk_arg, used[], flags, log)
+        new(source, n_params, obs_dim, with_grad, chunk_arg, used[], flags, mask, log)
     end
 end
 # chunk of the _ex entry points
@@ -309,7 +324,13 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
     rc = ccall((:extmcmc_create, LIB), Int32, (Ref{Config}, Ref{Ptr{Cvoid}}), cfg, h)
     rc == 0 || error("extmcmc_create: ", last_error(C_NULL))
     if data.P isa DeviceLaw                              # compiled once per process (cached by the check)
-        if data.P.flags != 0
+        if data.P.theta_only != 0
+            check(h[], ccall((:extmcmc_set_user_law_theta_only, LIB), Int32,
+                             (Ptr{Cvoid}, Cstring, Int32, Int32, Int32, UInt64),
+                             h[], data.P.source, data.P.with_grad,
+                             ex_chunk(data.P.with_grad, data.P.chunk_arg, data.P.n_params), data.P.flags,
+                             data.P.theta_only))
+        elseif data.P.flags != 0
             check(h[], ccall((:extmcmc_set_user_law_ex, LIB), Int32, (Ptr{Cvoid}, Cstring, Int32, Int32, Int32),
                              h[], data.P.source, data.P.with_grad,
                              ex_chunk(data.P.with_grad, data.P.chunk_arg, data.P.n_params), data.P.flags))

@@ -13,12 +13,17 @@ and 2, each set alternating in one process.  The theta-term arm (--theta-term) r
 (8192 chains, 8 groups x 4096 rows, MALA on theta_1..8 and two walks, bench.py's updates, 10 iterations per
 extmcmc_run_block) on the built-in HIER_NORMAL law with its data-sum cache off and on, and on its
 DeviceLaw restatement with a theta term (tests/user_laws_theta.py) with the hand-written and the
-forward-mode gradient, alternating: ms per iteration and sweep ms per launch of each.  One JSON object
-on stdout (and in --out), with the card's name and power limit read in the same process.
+forward-mode gradient, alternating: ms per iteration and sweep ms per launch of each.  The theta-only
+arm (--theta-only) runs cfg 4 on the built-in law with its cache and on the restatement without and with
+theta_only = [mu, tau] (hand-written and forward-mode gradient), and a ridge-penalised Poisson regression
+(d = 9: 8 coefficients + log lambda, 4096 chains x 1e6 rows) under RW(beta) + RW(log lambda) and
+MALA(beta) + RW(log lambda) without and with theta_only = [log lambda], each set alternating in one
+process: ms per iteration, sweeps per iteration and sweep ms per launch.  One JSON object on stdout (and
+in --out), with the card's name and power limit read in the same process.
 
     python tools/user_law_bench.py [--steps 300] [--warmup 30] [--reps 3] [--forward-only]
                                    [--forward-steps 30] [--chunked] [--chunked-steps 6]
-                                   [--theta-term] [--theta-steps 50] [--out FILE]
+                                   [--theta-term] [--theta-steps 50] [--theta-only] [--out FILE]
 """
 import argparse
 import ctypes
@@ -76,6 +81,7 @@ def main():
     ap.add_argument("--chunked-steps", type=int, default=6, help="timed steps of each chunked-arm rep")
     ap.add_argument("--theta-term", action="store_true", help="only the theta-term arm (cfg 4)")
     ap.add_argument("--theta-steps", type=int, default=50, help="timed iterations of each theta-term rep")
+    ap.add_argument("--theta-only", action="store_true", help="only the theta-only arm (cfg 4 and ridge)")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import extensiblemcmc_jl_b200 as em
@@ -83,7 +89,9 @@ def main():
     from tests import user_laws as ul
 
     out = {"card": card()}
-    if args.theta_term:
+    if args.theta_only:
+        theta_only_arm(args, em, _abi, out)
+    elif args.theta_term:
         theta_term_arm(args, em, _abi, out)
     elif args.chunked:
         chunked_arm(args, em, _abi, out)
@@ -225,6 +233,100 @@ def theta_term_arm(args, em, _abi, out):
         res[k + "_over_builtin_cache"] = res[k]["ms_per_iter"] / res["builtin_cache"]["ms_per_iter"]
         res[k + "_over_builtin_no_cache"] = res[k]["ms_per_iter"] / res["builtin_no_cache"]["ms_per_iter"]
     out["hier_cfg4_theta_term"] = res
+
+
+def alternate(args, em, _abi, arms, ipb):
+    """arms: name -> (data, updates(), EXTMCMC_DATA_CACHE, initial state): ms per iteration (median of
+    args.reps alternating timings), sweeps per iteration and sweep ms per launch (instrumented handles)."""
+    from extensiblemcmc_jl_b200.mcmc import init_
+    warm = 3 * ipb
+    steps = -(-args.theta_steps // ipb) * ipb
+
+    def make(data, ups, cache, th0, **bk):
+        os.environ["EXTMCMC_DATA_CACHE"] = cache    # read when the sweep is planned: the handle's first block
+        mcmc = em.MCMC(ups(), backend=em.CUDAMCMCBackend(n_chains=th0.shape[1], seed=7, history="none",
+                                                         block_len=3 * ipb, **bk))
+        init_(mcmc, 1, data, th0)
+        w = mcmc.workspace
+        bench._generic_timed(w, _abi, len(ups()), 0, warm, ipb=ipb)
+        return w
+    ws = {k: make(*a) for k, a in arms.items()}
+    it = {k: warm + 1 for k in ws}
+    times = {k: [] for k in ws}
+    for _ in range(args.reps):
+        for k, w in ws.items():
+            times[k].append(bench._generic_timed(w, _abi, len(arms[k][1]()), steps, 0, it0=it[k], ipb=ipb) / steps)
+            it[k] += steps
+    res = {}
+    for k, w in ws.items():
+        res[k] = {"ms_per_iter": float(np.median(times[k])), "ms_per_iter_reps": times[k],
+                  "variant": w.lib.extmcmc_sweep_variant_name(w.handle).decode()}
+        w.close()
+    for k, a in arms.items():
+        wi = make(*a, use_graphs=False, instrument=True)
+        msw, nl = ctypes.c_float(), ctypes.c_int64()
+        wi._ck(wi.lib.extmcmc_get_sweep_time(wi.handle, ctypes.byref(msw), ctypes.byref(nl)))
+        bench._generic_timed(wi, _abi, len(a[1]()), 2 * ipb, 0, it0=warm + 1, ipb=ipb)
+        wi._ck(wi.lib.extmcmc_get_sweep_time(wi.handle, ctypes.byref(msw), ctypes.byref(nl)))
+        res[k]["sweep_ms_per_launch"] = msw.value / max(nl.value, 1)
+        res[k]["sweeps_per_iter"] = nl.value / (2 * ipb)
+        wi.close()
+    os.environ.pop("EXTMCMC_DATA_CACHE", None)
+    return res
+
+
+def theta_only_arm(args, em, _abi, out):
+    """cfg 4 and a ridge-penalised Poisson regression, each law without and with theta_only."""
+    from tests import user_laws_theta as ut
+    C, G, ng, ipb = 8192, 8, 4096, bench.CFG4_BLOCK_ITERS
+    rng = np.random.default_rng(5)                       # bench.py's cfg 4 data, updates and initial state
+    tg = rng.standard_normal(G)
+    yv = np.concatenate([tg[g] + rng.standard_normal(ng) for g in range(G)])
+    grp = np.repeat(np.arange(G), ng)
+    rows = np.stack([yv, grp.astype(np.float64)], axis=1)
+    ups = lambda: [  # noqa: E731
+        em.MALAUpdate(0.02, list(range(1, G + 1)), adpt=em.AdaptationMALA(adapt_every_k_steps=50, scale=1e-3, min=1e-5)),
+        em.RandomWalkUpdate(em.UniformRandomWalk([0.3]), [G + 1], adpt=em.AdaptationUnifRW([0.0], adapt_every_k_steps=50, scale=0.02)),
+        em.RandomWalkUpdate(em.UniformRandomWalk([0.3], [True]), [G + 2], prior=em.ImproperPosPrior(),
+                            adpt=em.AdaptationUnifRW([0.0], adapt_every_k_steps=50, scale=0.02))]
+    P = G + 2
+    th0 = np.repeat(np.concatenate([np.zeros(G), [0.0, 1.0]])[:, None], C, axis=1)
+    arms = {"builtin_cache": (dict(P=em.HierNormalLaw(G), obs=yv, groups=grp), ups, "1", th0)}
+    for grad, src in ((True, ut.HIER_HAND), ("forward", ut.HIER_FORWARD)):
+        name = "hand" if grad is True else "forward"
+        for decl in (None, (P - 1, P)):
+            law = em.DeviceLaw(src, P, 2, gradient=grad, theta_term=True, theta_only=decl)
+            arms[f"device_law_{name}_{'declared' if decl else 'undeclared'}"] = (dict(P=law, obs=rows), ups, "1", th0)
+    out["theta_only_cfg4_workload"] = (f"BASELINE cfg 4: hierarchical normal, {G} groups x {ng} rows, {C} chains, "
+                                       f"MALA(theta_1..8) + RW(mu) + RW-pos(tau), {ipb} iterations per extmcmc_run_block")
+    res = alternate(args, em, _abi, arms, ipb)
+    for name in ("hand", "forward"):
+        res[f"{name}_declared_over_undeclared"] = (res[f"device_law_{name}_declared"]["ms_per_iter"] /
+                                                   res[f"device_law_{name}_undeclared"]["ms_per_iter"])
+        res[f"{name}_declared_over_builtin_cache"] = (res[f"device_law_{name}_declared"]["ms_per_iter"] /
+                                                      res["builtin_cache"]["ms_per_iter"])
+    out["hier_cfg4_theta_only"] = res
+
+    # ridge-penalised Poisson regression: theta = [beta_0..beta_7, log lambda], rows = [x_1..x_7, y]
+    Cr, N, d = bench.CHAINS_PER_GPU, 1_000_000, 9
+    Xr = ut.data("ridge", N, d, seed=5)
+    thr = np.zeros((d, Cr))
+    thr[:d - 1] = 1e-3 * np.random.default_rng(6).standard_normal((d - 1, Cr))
+    beta = list(range(1, d))
+    walk_lam = lambda: em.RandomWalkUpdate(em.UniformRandomWalk([0.3]), [d],  # noqa: E731
+                                           adpt=em.AdaptationUnifRW([0.0], adapt_every_k_steps=50, scale=0.02))
+    schedules = {"rw_rw": lambda: [em.RandomWalkUpdate(em.UniformRandomWalk([1e-3] * (d - 1)), beta), walk_lam()],
+                 "mala_rw": lambda: [em.MALAUpdate(1e-3, beta), walk_lam()]}
+    for sname, sups in schedules.items():
+        arms = {}
+        for decl in (None, (d,)):
+            law = em.DeviceLaw(ut.RIDGE_POISSON, d, d - 1, gradient=True, theta_term=True, theta_only=decl)
+            arms["declared" if decl else "undeclared"] = (dict(P=law, obs=Xr), sups, "1", thr)
+        r = alternate(args, em, _abi, arms, ipb)
+        r["declared_over_undeclared"] = r["declared"]["ms_per_iter"] / r["undeclared"]["ms_per_iter"]
+        out[f"ridge_poisson_d9_{sname}"] = r
+    out["ridge_workload"] = (f"ridge-penalised Poisson regression, d = {d} (8 coefficients + log lambda), {Cr} chains x "
+                             f"{N} rows, logpdf_grad, {ipb} iterations per extmcmc_run_block")
 
 
 def builtin_arms(args, em, _abi, ul, out):
