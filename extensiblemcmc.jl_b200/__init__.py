@@ -11,7 +11,8 @@ from .random_walk import UniformRandomWalk, GaussianRandomWalk, GaussianRandomWa
 from .adaptation import (NoAdaptation, AdaptationUnifRW, HaarioTypeAdaptation, AdaptationMALA,
                          isequal_except)
 from .priors import (Prior, ImproperPrior, ImproperPosPrior, StandardPrior, ProductPrior,
-                     Normal, Gamma, Uniform, Exponential, InverseGamma, Beta, LogNormal, Cauchy, MvNormal)
+                     Normal, Gamma, Uniform, Exponential, InverseGamma, Beta, LogNormal, Cauchy, MvNormal,
+                     DevicePrior)
 from .updates import RandomWalkUpdate, MALAUpdate, HamiltonianMCUpdate
 from .gsn_target import GsnTargetLaw
 from .hier_normal import HierNormalLaw

@@ -25,6 +25,7 @@ KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = 1, 2, 3, 
 PRIOR_IMPROPER, PRIOR_IMPROPER_POS, PRIOR_NORMAL, PRIOR_GAMMA, PRIOR_UNIFORM, PRIOR_PRODUCT = 0, 1, 2, 3, 4, 5
 PRIOR_EXPONENTIAL, PRIOR_INV_GAMMA, PRIOR_BETA, PRIOR_LOGNORMAL, PRIOR_CAUCHY = 6, 7, 8, 9, 10
 PRIOR_MVNORMAL = 11
+PRIOR_USER = 12
 # adaptation
 ADAPT_NONE, ADAPT_UNIF_RW, ADAPT_HAARIO, ADAPT_MALA = 0, 1, 2, 3
 # sharding
@@ -121,6 +122,9 @@ SIGNATURES = {
     "extmcmc_user_law_check_theta_only": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                                       C.c_int32, C.c_uint64, C.POINTER(C.c_int32), C.c_char_p,
                                                       C.c_int64]),
+    "extmcmc_user_prior_check": (C.c_int32, [C.c_char_p, C.c_int32, C.c_int32, C.c_char_p, C.c_int64]),
+    "extmcmc_set_user_prior": (C.c_int32, [Handle, C.c_int32, C.c_char_p, C.c_int32]),
+    "extmcmc_eval_user_prior": (C.c_int32, [Handle, C.c_int32, c_double_p, c_double_p]),
     "extmcmc_set_update": (C.c_int32, [Handle, C.c_int32, C.POINTER(Update)]),
     "extmcmc_set_state": (C.c_int32, [Handle, c_double_p]),
     "extmcmc_set_seed": (C.c_int32, [Handle, C.c_uint64]),

@@ -83,6 +83,8 @@ struct extmcmc_handle {
     int64_t *goff_dev = nullptr, *glen_dev = nullptr;  // [G] padded group offsets / true lengths
     double *y_dev = nullptr;             // LOGISTIC: responses, padded like the rows of X
     UserLaw ulaw;                        // USER: the compiled law (extmcmc_set_user_law)
+    std::vector<UserPrior> uprior;       // [NU] user-defined priors (extmcmc_set_user_prior)
+    StepDesc *prior_desc = nullptr;      // device descriptor naming the update of extmcmc_eval_user_prior
     int logi_D = 0;                      // LOGISTIC: padded feature dimension
     unsigned int *tail_counter = nullptr; // CTA counter of the fused sweep tail
     bool tail = false;                   // the obs-mapped sweep finishes the reduction itself
@@ -274,6 +276,11 @@ int32_t ensure_plan(extmcmc_t h) {
 // the one place that says what an element does to (grad_valid, dc_valid, rg_valid) and is used by the
 // descriptor loop, the graph key, the kernel sequence and the end-of-block state alike.
 constexpr int kDataFree = 0x100;
+// The update has a user-defined prior (EXTMCMC_PRIOR_USER), whose index the kind carries from bit 10 up
+// (the graph of a block launches that update's own prior kernels): its random-walk proposal is drawn by
+// the prior's kernel, never fused into the previous accept kernel; a MALA element runs the prior's
+// gradient kernel on the current state and on the proposal.
+constexpr int kUserPrior = 0x200, kUserPriorShift = 10;
 // What the cache holds: HIER_NORMAL's per-group sums (their gradient is always valid with them), or a
 // user law's row sums R and Rg (R alone is refilled by a value sweep, and kept across a random walk
 // that moved a row coordinate by the commit kernel: rsum_commit_kernel).
@@ -289,6 +296,7 @@ int step_kind(extmcmc_t h, int u) {
             moves_data = moves_data || (user ? !((h->ulaw.theta_only >> t.coords[i]) & 1) : t.coords[i] < h->d.G);
         if (!moves_data) kind |= kDataFree;
     }
+    if (t.prior == EXTMCMC_PRIOR_USER) kind |= kUserPrior | (u << kUserPriorShift);
     return kind;
 }
 inline bool kind_is_mala(int kind) { return (kind & 0xff) == EXTMCMC_KERNEL_MALA; }
@@ -535,12 +543,18 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
         // deferred bookkeeping between consecutive elements of this block (step_kernels.cu, run_deferred)
         const int dflags = step_deferral_flags(h->d, k, n_steps);
         const bool next_mala = k + 1 < n_steps && kind_is_mala(kinds[k + 1]);
-        const bool next_rw = k + 1 < n_steps && !kind_is_mala(kinds[k + 1]);
+        // a proposal drawn by a user prior's kernel cannot ride on the previous accept kernel
+        const bool next_rw = k + 1 < n_steps && !kind_is_mala(kinds[k + 1]) && !(kinds[k + 1] & kUserPrior);
+        const UserPrior *up = (kinds[k] & kUserPrior) ? &h->uprior[kinds[k] >> kUserPriorShift] : nullptr;
         const int mode = step_advance(cache_kind(h), kinds[k], grad_valid, dc_valid, rg_valid);
         if (kind_is_mala(kinds[k])) {
             const bool logi = law_self_finished(h->cfg.law);   // the sweep finishes ll and gradient
             int finalize_cur = 0;
             DevState gv = grad_view(h);
+            if (up) {   // the prior's lp and gradient at the current state (read behind mala_propose's griddep_wait)
+                CK(h, launch_prior_grad(*up, h->d, d_descs, k, h->d.theta, 0, h->stream));
+                h->launches += 1;
+            }
             if (mode == 1) {
                 if (logi) {
                     if ((rc = enqueue_sweep(h, instrument, true, h->d.theta, h->scratch_ll, h->d.grad_cur, nullptr, 0,
@@ -563,6 +577,10 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
             }
             launch_mala_propose(gv, d_descs, k, finalize_cur, h->scratch_ll, dflags, h->stream);
             gv = grad_view(h);
+            if (up) {   // ... and at the proposal, finished before the proposal's sweep starts
+                CK(h, launch_prior_grad(*up, h->d, d_descs, k, h->d.prop_full, 1, h->stream));
+                h->launches += 1;
+            }
             if (logi) {
                 if ((rc = enqueue_sweep(h, instrument, true, h->d.prop_full, h->d.ll_prop, h->d.grad_prop))) return rc;
             } else {
@@ -573,6 +591,10 @@ int32_t enqueue_steps(extmcmc_t h, const StepDesc *d_descs, const int *kinds, in
             h->launches += 2;
             cur_prepared = false;
         } else {
+            if (up) {   // the draw with the prior's redraw loop, lp of proposal and current state
+                CK(h, launch_prior_rw(*up, h->d, d_descs, k, h->stream));
+                h->launches += 1;
+            }
             if (!fused) { launch_propose(h->d, d_descs, k, h->stream); h->launches += 1; }
             const bool from_cache = mode != 0;
             if (mode == 2 && rows) {
@@ -634,12 +656,23 @@ int32_t run_block_impl(extmcmc_t h, const extmcmc_step_t *steps, int32_t n_steps
     for (int s = 0; s < n_steps; ++s)
         if (steps[s].pidx < 0 || steps[s].pidx >= h->cfg.n_updates || steps[s].mcmciter < 1)
             return fail(h, EXTMCMC_EINVAL, "step out of range");
+    bool any_uprior = false;
+    for (int u = 0; u < h->cfg.n_updates; ++u) {
+        if (h->upd_host[u].prior != EXTMCMC_PRIOR_USER) continue;
+        any_uprior = true;
+        if (!h->uprior[u].loaded)
+            return fail(h, EXTMCMC_EINVAL, "update " + std::to_string(u) + " has a user prior: call extmcmc_set_user_prior first");
+        if (h->upd_host[u].kernel == EXTMCMC_KERNEL_MALA && h->uprior[u].mode == kUserValue)
+            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user prior with a gradient (extmcmc_set_user_prior with_grad = 1 or 2)");
+    }
     CK(h, cudaSetDevice(h->cfg.device));
     int32_t rc;
     if ((rc = ensure_plan(h))) return rc;
     if ((rc = upload_updates(h))) return rc;
     if ((rc = ensure_total_obs(h))) return rc;
     if ((rc = plan_block_kernels(h))) return rc;
+    if ((h->res_ok || h->obsblk_ok) && any_uprior)
+        return fail(h, EXTMCMC_EUNSUPPORTED, "the persistent block kernels (sweep_variant 3 / 4) do not run user priors");
     if ((h->res_ok || h->obsblk_ok) && h->dcache) {   // the persistent block kernels sweep for every element
         h->dcache = h->dc_valid = h->rg_valid = false;
         h->d.dsum_cur = h->d.dsum_prop = nullptr;
@@ -951,6 +984,7 @@ int32_t extmcmc_create(const extmcmc_config_t *cfg, extmcmc_t *out) {
         return bail(rc);
     CKC(cudaMemset(d.err_flag, 0, sizeof(int32_t)));
     h->upd_host.assign(NU, DevUpdate{});
+    h->uprior.assign(NU, UserPrior{});
     h->upd_set.assign(NU, false);
     h->ra_iter.assign(NU, 0);
     h->acc_tag.assign((size_t)NU * d.W, 0);
@@ -1004,6 +1038,7 @@ int32_t extmcmc_destroy(extmcmc_t h) {
     if (h->obs_dev) cudaFree(h->obs_dev);
     if (h->y_dev) cudaFree(h->y_dev);
     user_law_unload(h->ulaw);
+    for (UserPrior &p : h->uprior) user_prior_unload(p);
     if (h->rp_prop) cudaFree(h->rp_prop);
     if (h->rp_exp) cudaFree(h->rp_exp);
     if (h->flush_buf) cudaFree(h->flush_buf);
@@ -1174,14 +1209,19 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
             return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a law with a device gradient (GSN_IID_1D, HIER_NORMAL, LOGISTIC, USER)");
         if (h->cfg.law == EXTMCMC_LAW_USER && h->ulaw.loaded && !h->ulaw.grad)
             return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user law with a gradient (extmcmc_set_user_law with_grad = 1 or 2)");
-        if (upd->prior != EXTMCMC_PRIOR_IMPROPER && upd->prior != EXTMCMC_PRIOR_NORMAL)
-            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA supports ImproperPrior and Normal priors only");
+        if (upd->prior != EXTMCMC_PRIOR_IMPROPER && upd->prior != EXTMCMC_PRIOR_NORMAL && upd->prior != EXTMCMC_PRIOR_USER)
+            return fail(h, EXTMCMC_EUNSUPPORTED, "MALA supports ImproperPrior, Normal and user-defined priors only");
         if (upd->pos)
             for (int i = 0; i < upd->n_coords; ++i)
                 if (upd->pos[i]) return fail(h, EXTMCMC_EUNSUPPORTED, "MALA on positivity-constrained coordinates is not implemented");
     }
-    if (upd->prior < EXTMCMC_PRIOR_IMPROPER || upd->prior > EXTMCMC_PRIOR_MVNORMAL)
+    if (upd->prior < EXTMCMC_PRIOR_IMPROPER || upd->prior > EXTMCMC_PRIOR_USER)
         return fail(h, EXTMCMC_EUNSUPPORTED, "prior not implemented on the GPU path");
+    const bool uprior = upd->prior == EXTMCMC_PRIOR_USER;
+    if (uprior && obs_sharded(h))
+        return fail(h, EXTMCMC_EUNSUPPORTED, "user priors are not implemented under EXTMCMC_SHARD_OBS with several ranks");
+    if (uprior && upd->n_coords > kUserPriorMaxCoords)
+        return fail(h, EXTMCMC_EUNSUPPORTED, "a user prior needs 1 <= n_coords <= 64");
     if (upd->n_coords < 1 || upd->n_coords > (mala ? std::min(h->cfg.n_params, 32768) : kMaxCoords))
         return fail(h, EXTMCMC_EUNSUPPORTED, mala ? "1 <= n_coords <= min(n_params, 32768) for MALA"
                                                   : "1 <= n_coords <= 32 for random-walk updates on the GPU path");
@@ -1212,7 +1252,7 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
             return fail(h, EXTMCMC_EINVAL, "bad prior parameters");
         // parameters each StandardPrior family reads
         const int pk = upd->prior;
-        const int need = (pk == EXTMCMC_PRIOR_IMPROPER || pk == EXTMCMC_PRIOR_IMPROPER_POS) ? 0
+        const int need = (pk == EXTMCMC_PRIOR_IMPROPER || pk == EXTMCMC_PRIOR_IMPROPER_POS || pk == EXTMCMC_PRIOR_USER) ? 0
                        : pk == EXTMCMC_PRIOR_EXPONENTIAL ? 1 : 2;
         if (upd->n_prior_params < need) return fail(h, EXTMCMC_EINVAL, "prior parameters missing");
     }
@@ -1239,7 +1279,8 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
         const DevUpdate &cur = h->upd_host[u];
         if (!fresh && cur.n_coords != nc) return fail(h, EXTMCMC_EINVAL, "cannot change n_coords of an update");
         if (!fresh && ((mix && !cur.sigB) || (gauss && !cur.sigA) || (haario && !cur.hmean) ||
-                       (upd->prior == EXTMCMC_PRIOR_MVNORMAL && !cur.prior_dev)))
+                       (upd->prior == EXTMCMC_PRIOR_MVNORMAL && !cur.prior_dev) ||
+                       uprior != (cur.prior == EXTMCMC_PRIOR_USER)))
             return fail(h, EXTMCMC_EINVAL, "cannot change the kernel or prior family of an update");
     }
 
@@ -1273,6 +1314,8 @@ int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd) 
         if (mix && ((rc = dev_alloc(h, &t.sigB, (size_t)nn * C)) || (rc = dev_alloc(h, &t.LB, (size_t)nn * C)))) return rc;
         if (haario && ((rc = dev_alloc(h, &t.hmean, (size_t)nc * C)) || (rc = dev_alloc(h, &t.hcov, (size_t)nn * C)))) return rc;
         if (mvn) { if ((rc = dev_alloc(h, &pd, (size_t)(nc + nn)))) return rc; t.prior_dev = pd; }
+        // user prior: what its kernels leave for the step kernels, [2][1 + p_u][C] (prior_user.cuh)
+        if (uprior) { if ((rc = dev_alloc(h, &pd, (size_t)2 * (1 + nc) * C))) return rc; t.prior_dev = pd; }
     }
     if ((gauss || haario || mvn) && (rc = ensure_gw_scratch(h, nc))) return rc;
     CK(h, cudaStreamSynchronize(h->stream));
@@ -1535,6 +1578,63 @@ int32_t extmcmc_set_user_law_ex(extmcmc_t h, const char *source, int32_t with_gr
 int32_t extmcmc_set_user_law_theta_only(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags,
                                         uint64_t theta_only) {
     return set_user_law(h, "extmcmc_set_user_law_theta_only", source, with_grad, true, chunk, flags, true, theta_only);
+}
+
+// ---- user-defined priors ------------------------------------------------------------------------
+static int32_t user_prior_limits(int32_t p_u, int mode, std::string &err) {
+    if (p_u < 1 || p_u > kUserPriorMaxCoords) {
+        err = "user priors need 1 <= p_u <= 64; got p_u = " + std::to_string(p_u);
+        return EXTMCMC_EUNSUPPORTED;
+    }
+    if (mode == kUserGradForward && p_u > kUserMaxForwardParams) {
+        err = "forward-mode prior gradients need p_u <= 16 (PU + 1 doubles per value in registers); got p_u = " +
+              std::to_string(p_u) + ": write logprior_grad (with_grad = 1)";
+        return EXTMCMC_EUNSUPPORTED;
+    }
+    return EXTMCMC_OK;
+}
+
+int32_t extmcmc_user_prior_check(const char *source, int32_t p_u, int32_t with_grad, char *log, int64_t log_bytes) {
+    if (log && log_bytes > 0) log[0] = 0;
+    if (!source) return fail(nullptr, EXTMCMC_EINVAL, "null source");
+    const int mode = user_grad_mode(with_grad);
+    std::string err;
+    if (const int32_t rc = user_prior_limits(p_u, mode, err)) {
+        copy_log(err, log, log_bytes);
+        return fail(nullptr, rc, err);
+    }
+    std::string lg, cubin;
+    const int32_t rc = user_prior_compile(source, p_u, mode, lg, cubin);
+    copy_log(lg, log, log_bytes);
+    if (rc) g_create_error = lg;
+    return rc;
+}
+
+int32_t extmcmc_set_user_prior(extmcmc_t h, int32_t u, const char *source, int32_t with_grad) {
+    if (!h) return EXTMCMC_EINVAL;
+    if (u < 0 || u >= h->cfg.n_updates) return fail(h, EXTMCMC_EINVAL, "update index out of range");
+    if (!source) return fail(h, EXTMCMC_EINVAL, "null source");
+    const DevUpdate &t = h->upd_host[u];
+    if (!h->upd_set[u] || t.prior != EXTMCMC_PRIOR_USER)
+        return fail(h, EXTMCMC_EINVAL, "extmcmc_set_user_prior needs an update set with prior EXTMCMC_PRIOR_USER");
+    const int mode = user_grad_mode(with_grad);
+    std::string err;
+    if (const int32_t rc = user_prior_limits(t.n_coords, mode, err)) return fail(h, rc, err);
+    if (t.kernel == EXTMCMC_KERNEL_MALA && mode == kUserValue)
+        return fail(h, EXTMCMC_EUNSUPPORTED, "MALA needs a user prior with a gradient (with_grad = 1 or 2)");
+    std::string log, cubin;
+    const int32_t rc = user_prior_compile(source, t.n_coords, mode, log, cubin);
+    if (rc == EXTMCMC_EINVAL) return fail(h, rc, "the user prior does not compile:\n" + log);
+    if (rc) return fail(h, rc, log);
+    CK(h, cudaSetDevice(h->cfg.device));
+    CK(h, cudaStreamSynchronize(h->stream));   // no queued launch may still use the old kernels
+    invalidate_graphs(h);
+    const cudaError_t e = user_prior_load(h->uprior[u], cubin, t.n_coords, mode);
+    if (e != cudaSuccess) {
+        user_prior_unload(h->uprior[u]);
+        return fail(h, EXTMCMC_ECUDA, std::string("loading the user prior: ") + cudaGetErrorString(e));
+    }
+    return EXTMCMC_OK;
 }
 
 // ---- checkpoint / resume ------------------------------------------------------------------------
@@ -1920,6 +2020,31 @@ int32_t extmcmc_eval_loglik(extmcmc_t h, double *ll_out) {
     }
     CK(h, cudaGetLastError());
     CK(h, cudaMemcpyAsync(ll_out, h->scratch_ll, sizeof(double) * h->d.C, cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaStreamSynchronize(h->stream));
+    return EXTMCMC_OK;
+}
+
+int32_t extmcmc_eval_user_prior(extmcmc_t h, int32_t u, double *lp_out, double *grad_out) {
+    if (!h || !lp_out || !grad_out) return EXTMCMC_EINVAL;
+    if (u < 0 || u >= h->cfg.n_updates) return fail(h, EXTMCMC_EINVAL, "update index out of range");
+    if (!h->state_set) return fail(h, EXTMCMC_EINVAL, "extmcmc_set_state not called");
+    const DevUpdate &t = h->upd_host[u];
+    if (!h->upd_set[u] || t.prior != EXTMCMC_PRIOR_USER || !h->uprior[u].loaded)
+        return fail(h, EXTMCMC_EINVAL, "update " + std::to_string(u) + " has no user prior installed");
+    if (h->uprior[u].mode == kUserValue)
+        return fail(h, EXTMCMC_EUNSUPPORTED, "the user prior has no gradient (extmcmc_set_user_prior with_grad = 1 or 2)");
+    CK(h, cudaSetDevice(h->cfg.device));
+    int32_t rc;
+    if ((rc = upload_updates(h))) return rc;
+    if (!h->prior_desc && (rc = dev_alloc(h, &h->prior_desc, 1))) return rc;
+    StepDesc sd{};
+    sd.pidx = u;
+    CK(h, cudaMemcpyAsync(h->prior_desc, &sd, sizeof sd, cudaMemcpyHostToDevice, h->stream));
+    CK(h, launch_prior_grad(h->uprior[u], h->d, h->prior_desc, 0, h->d.theta, 0, h->stream));
+    h->launches += 1;
+    const int64_t C = h->d.C, n = t.n_coords;
+    CK(h, cudaMemcpyAsync(lp_out, t.prior_dev, sizeof(double) * C, cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaMemcpyAsync(grad_out, t.prior_dev + C, sizeof(double) * n * C, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
     return EXTMCMC_OK;
 }

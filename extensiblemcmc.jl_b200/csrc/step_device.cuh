@@ -14,36 +14,19 @@
 #include "dev_state.cuh"
 #include "philox.cuh"
 #include "exchange.cuh"
+#include "rw_draw.cuh"
 
 namespace extmcmc {
 
 constexpr double kLog2Pi = 1.8378770664093454835606594728112;
 constexpr double kLogPi = 1.1447298858494001741434273513531;
 
-// ---- accessors ---------------------------------------------------------------------------------
-struct StrideGet {            // q[i * stride] (one chain's column of an SoA array)
-    const double *p;
-    int64_t stride;
-    __device__ __forceinline__ double operator()(int i) const { return p[(int64_t)i * stride]; }
-};
-struct CoordGet {             // theta[coords[i]] of one chain
-    const double *col;        // theta + c
-    const int32_t *coords;
-    int64_t C;
-    __device__ __forceinline__ double operator()(int i) const { return col[(int64_t)coords[i] * C]; }
-};
+// ---- accessors (StrideGet, CoordGet, MatRef: rw_draw.cuh) ------------------------------------
 template <class G>
 struct OffsetGet {
     G g;
     int off;
     __device__ __forceinline__ double operator()(int i) const { return g(off + i); }
-};
-// column-major n x n matrix, either shared by all chains (stride 1) or per chain (stride C, + c)
-struct MatRef {
-    double *p;
-    int64_t stride;
-    __device__ __forceinline__ double get(int idx) const { return p[(int64_t)idx * stride]; }
-    __device__ __forceinline__ void set(int idx, double v) const { p[(int64_t)idx * stride] = v; }
 };
 
 // ---- compile-time specialisation ---------------------------------------------------------------
@@ -264,9 +247,6 @@ __device__ __forceinline__ double log_q_gauss(const DevState &d, const DevUpdate
     return mvn_logpdf_chol(L, n, LogPosGet<FromGet>{from, u.pos}, LogPosGet<ToGet>{to, u.pos}, d.gw + c, d.C) + logJ;
 }
 
-__device__ __forceinline__ MatRef mat_LA(const DevUpdate &u) { return MatRef{u.LA, 1}; }
-__device__ __forceinline__ MatRef mat_LB(const DevUpdate &u, int64_t C, int64_t c) { return MatRef{u.LB + c, C}; }
-
 // q(from -> to) of a Gaussian walk (GaussianRandomWalkMix random_walk.jl:229-232: no log-sum-exp
 // guard, as in the reference); NaN when a factor is missing (Sigma not positive definite)
 template <class FromGet, class ToGet>
@@ -400,63 +380,7 @@ struct CtaSync { __device__ __forceinline__ void operator()() const { __syncthre
 // its history row by then).  propose_chain = both, back to back.
 template <class SP = SpecAny>
 __device__ __forceinline__ void propose_draw(const DevState &d, const StepDesc &sd, const DevUpdate &u, int64_t c) {
-    const int kern = sp_rw_kernel<SP>(u);
-    const int n = u.n_coords;
-    const int64_t C = d.C;
-    const CoordGet th{d.theta + c, u.coords, C};
-    const StrideGet prop{d.prop_loc + c, C};
-    double *pl = d.prop_loc + c;
-
-    uint32_t used = 0;
-    if (d.rng_mode == EXTMCMC_RNG_REPLAY) {
-        for (int i = 0; i < n; ++i) pl[(int64_t)i * C] = d.rp_prop[((int64_t)sd.replay_row * d.p_u_max + i) * d.gC + d.g0 + c];
-    } else {
-        ChainStepStream rng(d.seed, (uint64_t)(d.chain_offset + c), sd.mcmciter, sd.pidx);
-        for (;;) {
-            if (kern == EXTMCMC_KERNEL_RW_UNIFORM) {
-                for (int i = 0; i < n; ++i) {
-                    const double r = rng.next();
-                    const double e = u.eps[(int64_t)i * C + c];
-                    const double a = -e, b = e;
-                    const double U = a + (b - a) * r;  // rand(Uniform(-eps, eps))
-                    const double t = th(i);
-                    pl[(int64_t)i * C] = u.pos[i] ? t * exp(U) : t + U;  // random_walk.jl:72
-                }
-            } else {
-                // rand(rw::GaussianRandomWalk[Mix]) random_walk.jl:145-151,213-227
-                bool useB = false;
-                if (kern == EXTMCMC_KERNEL_RW_GAUSS_MIX) useB = rng.next() <= sd.lambda;  // Bernoulli(lambda)
-                double *z = d.gw + c;
-                for (int q = 0; q < n; q += 2) {  // randn via Box-Muller on the uniform stream
-                    const double u1 = rng.next(), u2 = rng.next();
-                    const double rad = sqrt(-2.0 * log(u1));
-                    double sn, cs;
-                    sincospi(2.0 * u2, &sn, &cs);
-                    z[(int64_t)q * C] = rad * cs;
-                    if (q + 1 < n) z[(int64_t)(q + 1) * C] = rad * sn;
-                }
-                const MatRef L = useB ? mat_LB(u, C, c) : mat_LA(u);
-                if (isnan(L.get(0))) {
-                    *d.err_flag = 1;  // reference: PosDefException from MvNormal(theta, Sigma)
-                    for (int i = 0; i < n; ++i) pl[(int64_t)i * C] = NAN;
-                    break;
-                }
-                for (int i = 0; i < n; ++i) {
-                    const double x = th(i);
-                    double t = u.pos[i] ? log(x) : x;
-                    double a = 0.0;
-                    for (int k = 0; k <= i; ++k) a += L.get(i + k * n) * z[(int64_t)k * C];
-                    t = a + t;
-                    pl[(int64_t)i * C] = u.pos[i] ? exp(t) : t;
-                }
-            }
-            // whole-vector redraw while the prior is exactly -Inf (updates.jl:193-195)
-            if (!(log_prior<SP>(d, u, prop, c) == -INFINITY)) break;
-            if (rng.j > 60000u) break;
-        }
-        used = rng.j;
-    }
-    d.n_used[c] = used;
+    rw_draw(d, sd, u, c, sp_rw_kernel<SP>(u), [&](const StrideGet &prop) { return log_prior<SP>(d, u, prop, c); });
 }
 
 template <class SP = SpecAny>
@@ -776,8 +700,14 @@ __device__ __forceinline__ RwPre rw_accept_prologue(const DevState &d, const Ste
             r.q_fwd = log_q_gauss_any(d, u, sd.lambda, th, prop, c);    // theta -> theta°
         }
     }
-    r.lp_prop = log_prior<SP>(d, u, prop, c);
-    r.lp_cur = log_prior<SP>(d, u, th, c);
+    if (!SP::kLean && u.prior == EXTMCMC_PRIOR_USER) {
+        // a user-defined prior: its kernel drew the proposal and left both terms in prior_dev ([2][C])
+        r.lp_prop = u.prior_dev[c];
+        r.lp_cur = u.prior_dev[C + c];
+    } else {
+        r.lp_prop = log_prior<SP>(d, u, prop, c);
+        r.lp_cur = log_prior<SP>(d, u, th, c);
+    }
     r.E = draw_exp(d, sd, c);
     return r;
 }
@@ -883,6 +813,15 @@ __device__ __forceinline__ double prior_logpdf1(const DevUpdate &u, double th) {
     return 0.0;
 }
 
+// d log prior / d theta_i of a MALA update: the built-in families, or -- a user-defined prior, general
+// path only -- what its gradient kernel left in prior_dev: [2][1 + p_u][C], state s = 0 the current one,
+// s = 1 the proposal, row 0 the log prior and row 1 + i its derivative in coordinate i
+template <class SP>
+__device__ __forceinline__ double mala_prior_grad(const DevUpdate &u, double th, int64_t C, int64_t c, int s, int i) {
+    if (!SP::kLean && u.prior == EXTMCMC_PRIOR_USER) return u.prior_dev[((int64_t)s * (1 + u.n_coords) + 1 + i) * C + c];
+    return prior_grad(u, th);
+}
+
 // MALA proposal  theta° = theta + (tau^2/2) g(theta) + tau z,  g = grad(ll + log prior)
 template <class SP = SpecAny>
 __device__ __forceinline__ void mala_propose_chain(const DevState &d, const StepDesc &sd, const DevUpdate &u, int64_t c) {
@@ -912,7 +851,7 @@ __device__ __forceinline__ void mala_propose_chain(const DevState &d, const Step
                 if (i + q >= n) break;
                 const int64_t j = u.coords_dev[i + q];
                 const double th = d.theta[j * C + c];
-                const double g = d.grad_cur[j * C + c] + prior_grad(u, th);
+                const double g = d.grad_cur[j * C + c] + mala_prior_grad<SP>(u, th, C, c, 0, i + q);
                 d.prop_full[j * C + c] = th + h2 * g + tau * (rad * (q ? sn : cs));
             }
         }
@@ -947,14 +886,20 @@ __device__ __forceinline__ Decision mala_decide_commit(const DevState &d, const 
 #pragma unroll
         for (int q = 0; q < 2; ++q)
             if (i0 + q < n) {
-                const double gaq = ga[q] + prior_grad(u, a[q]);
-                const double gbq = gb[q] + prior_grad(u, b[q]);
+                const double gaq = ga[q] + mala_prior_grad<SP>(u, a[q], C, c, 0, i0 + q);
+                const double gbq = gb[q] + mala_prior_grad<SP>(u, b[q], C, c, 1, i0 + q);
                 const double rf = b[q] - a[q] - h2 * gaq, rb = a[q] - b[q] - h2 * gbq;
                 qf += rf * rf;
                 qb += rb * rb;
-                lp_prop += prior_logpdf1(u, b[q]);
-                lp_cur += prior_logpdf1(u, a[q]);
+                if (SP::kLean || u.prior != EXTMCMC_PRIOR_USER) {
+                    lp_prop += prior_logpdf1(u, b[q]);
+                    lp_cur += prior_logpdf1(u, a[q]);
+                }
             }
+    }
+    if (!SP::kLean && u.prior == EXTMCMC_PRIOR_USER) {   // the prior kernel's values (mala_prior_grad)
+        lp_cur = u.prior_dev[c];
+        lp_prop = u.prior_dev[(int64_t)(1 + n) * C + c];
     }
     const double inv = 1.0 / (2.0 * tau * tau);
     qf = -qf * inv;  // theta -> theta°

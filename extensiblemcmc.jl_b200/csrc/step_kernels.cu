@@ -35,7 +35,9 @@ propose_kernel(DevState d, const StepDesc *__restrict__ descs, int k) {
     load_step_ctx(&ctx, d, descs, k, threadIdx.x, blockDim.x, CtaSync{});
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= d.C || exchange_failed(d)) return;
-    propose_chain<SP>(d, ctx.sd, ctx.u, c);
+    // a user-defined prior's kernel has drawn the proposal (rw_draw inside its redraw loop)
+    if (!SP::kLean && ctx.u.prior == EXTMCMC_PRIOR_USER) propose_set<SP>(d, ctx.u, c);
+    else propose_chain<SP>(d, ctx.sd, ctx.u, c);
 }
 
 // Law constants of the CURRENT state (extmcmc_eval_loglik).

@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 #include "sweep.h"
 #include "sweep_user.cuh"
+#include "dev_state.cuh"
 
 namespace extmcmc {
 
@@ -68,5 +69,30 @@ cudaError_t launch_sweep_user(const SweepPlan &pl, const UserLaw &u, const UserS
                               double *ll_dst, double *grad_dst, double *rsum, cudaStream_t st);
 // The parameter-only kernel of a law with theta_only: a.ll (and a.grad with grad) from a.rsum and a.theta
 cudaError_t launch_theta_user(const UserLaw &u, const UserThetaArgs &a, bool grad, cudaStream_t st);
+
+// ---- user-defined priors (EXTMCMC_PRIOR_USER, prior_user.cuh) -------------------------------------
+constexpr int kUserPriorNT = 128;        // threads per CTA of the prior kernels (a chain each)
+constexpr int kUserPriorMaxCoords = 64;  // p_u of a user prior (MALA; the random walks stop at kMaxCoords)
+
+// Compiles the prior's kernels for (PU, mode) -- mode: a UserGrad; the random-walk kernel when
+// PU <= kMaxCoords, the gradient kernel when mode != kUserValue -- through the cache of user_law_compile.
+// EXTMCMC_OK, EXTMCMC_EINVAL (does not compile) or EXTMCMC_EUNSUPPORTED (no NVRTC).
+int32_t user_prior_compile(const char *source, int PU, int mode, std::string &log, std::string &cubin);
+
+struct UserPrior {
+    bool loaded = false;
+    int mode = kUserValue;      // UserGrad of the compiled program
+    int PU = 0;
+    cudaLibrary_t lib = nullptr;
+    cudaKernel_t rw = nullptr;    // draw + redraw loop + lp of proposal and current state
+    cudaKernel_t grad = nullptr;  // lp and gradient of a state (mode != kUserValue)
+};
+cudaError_t user_prior_load(UserPrior &p, const std::string &cubin, int PU, int mode);
+void user_prior_unload(UserPrior &p);
+// The kernels on element k of descs: the draw (writes prop_loc, n_used, prior_dev [2][C]); lp and gradient of
+// the state src into prior_dev + s (1 + PU) C (s = 0 the current state, 1 the proposal)
+cudaError_t launch_prior_rw(const UserPrior &p, const DevState &d, const StepDesc *descs, int k, cudaStream_t st);
+cudaError_t launch_prior_grad(const UserPrior &p, const DevState &d, const StepDesc *descs, int k, const double *src,
+                              int s, cudaStream_t st);
 
 }  // namespace extmcmc

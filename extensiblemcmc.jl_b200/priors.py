@@ -1,7 +1,10 @@
 """Priors (src/priors.jl).  Evaluated on the device on the update's own coordinates only
 (src/run.jl:374-385, src/updates.jl:104).  Arbitrary `dist` objects cannot cross the C ABI:
 the enumerated families below are supported, anything else raises at workspace creation
-(the reference's convention for a missing method is error("... not implemented"))."""
+(the reference's convention for a missing method is error("... not implemented")).  A prior of any
+other form is written as CUDA C++ and compiled at run time: DevicePrior."""
+import ctypes as C
+
 import numpy as np
 
 from . import _abi
@@ -129,8 +132,56 @@ class ProductPrior(Prior):                            # priors.jl:60-88
         for dist, dim in zip(self.dists, self.dims):
             pr = dist if isinstance(dist, Prior) else StandardPrior(dist)
             kind, pp = pr.to_abi()
-            if kind in (_abi.PRIOR_PRODUCT, _abi.PRIOR_MVNORMAL):
+            if kind in (_abi.PRIOR_PRODUCT, _abi.PRIOR_MVNORMAL, _abi.PRIOR_USER):
                 raise NotImplementedError("ProductPrior factors must be iid families on the GPU path")
             pp = list(pp) + [0.0, 0.0]
             out += [float(kind), float(dim), pp[0], pp[1]]
         return _abi.PRIOR_PRODUCT, np.array(out)
+
+
+class DevicePrior(Prior):
+    """A user-defined prior on the device: the reference's open Prior type (a subtype with
+    logpdf(prior, th), priors.jl:4-39) written as CUDA C++ over the update's own EXTMCMC_PU coordinates
+    and compiled at run time (csrc/prior_user.cuh; the contract is in include/extmcmc.h and INTEGRATION.md):
+
+        __device__ double logprior(const double *th, const double *pp);            // -INFINITY off the support
+        __device__ double logprior_grad(const double *th, const double *pp, double *g);   // gradient=True
+        template <class real> __device__ real logprior(const real *th, const double *pp); // gradient="forward"
+
+    pp are `params`, passed at run time (new hyperparameters need no recompilation).  Usable as the
+    prior= of RandomWalkUpdate (the proposal is redrawn while logprior is -INFINITY) and, with a
+    gradient, of MALAUpdate.  The constructor compiles the source for sm_100a at n_coords coordinates
+    (default 1; the workspace compiles it again at its update's p_u) and raises ValueError with the
+    compiler's log when it does not compile."""
+
+    def __init__(self, source, gradient=False, params=(), n_coords=1):
+        if isinstance(gradient, str) and gradient == "forward":
+            self._with_grad = _abi.USER_GRAD_FORWARD
+        elif isinstance(gradient, (bool, int)) and gradient in (False, True):
+            self._with_grad = _abi.USER_GRAD_HAND if gradient else _abi.USER_GRAD_NONE
+        else:
+            raise ValueError(f"gradient must be False, True or 'forward', not {gradient!r}")
+        self.source = str(source)
+        self.gradient = "forward" if self._with_grad == _abi.USER_GRAD_FORWARD else bool(gradient)
+        self.params = np.ascontiguousarray(np.atleast_1d(np.asarray(params, dtype=np.float64)))
+        self.log = self.check(int(n_coords))
+
+    def check(self, n_coords):
+        """Compiles the prior's kernels for n_coords coordinates; returns the NVRTC + ptxas log
+        (registers, spill bytes).  ValueError when the source does not compile."""
+        lib = _abi.load()
+        buf = C.create_string_buffer(1 << 16)
+        rc = lib.extmcmc_user_prior_check(self.source.encode(), n_coords, self._with_grad, buf, len(buf))
+        log = buf.value.decode(errors="replace")
+        if rc == _abi.EINVAL:
+            raise ValueError("the device prior does not compile:\n" + log)
+        if rc != _abi.OK:
+            raise _abi.ExtMCMCError(rc, log or lib.extmcmc_last_error(None).decode())
+        return log
+
+    def to_abi(self):
+        return _abi.PRIOR_USER, self.params
+
+    def abi_attach(self, lib, handle, u):
+        """Compiles (cached) and installs the prior of update u (0-based), after extmcmc_set_update."""
+        return lib.extmcmc_set_user_prior(handle, u, self.source.encode(), self._with_grad)

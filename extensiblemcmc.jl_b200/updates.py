@@ -60,7 +60,8 @@ class MALAUpdate(MCMCGradientBasedUpdate):
     src/updates.jl:129-133, the `grad ll` buffer src/workspaces.jl:417).  Build-defined
     semantics: theta° = theta + tau^2/2 * grad(ll + log prior)(theta) + tau * z, z ~ N(0, I),
     Metropolis-Hastings corrected with the same llr association and Exp(1) test as every other
-    update (src/run.jl:268-281).  Priors: ImproperPrior, StandardPrior(Normal)."""
+    update (src/run.jl:268-281).  Priors: ImproperPrior, StandardPrior(Normal), and a DevicePrior
+    with a gradient."""
 
     def __init__(self, tau, idx_of_global, prior=None, adpt=None):
         self.tau = float(tau)

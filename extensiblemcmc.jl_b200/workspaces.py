@@ -170,6 +170,9 @@ class CUDAGlobalWorkspace(GlobalWorkspace):
                 self._keep.append(keep)
                 self._kernels.append(u.kernel)
                 self._ck(lib.extmcmc_set_update(self.handle, i, C.byref(u)))
+                prior = getattr(updt, "prior", None)
+                if hasattr(prior, "abi_attach"):                # DevicePrior: compile and install the prior
+                    self._ck(prior.abi_attach(lib, self.handle, i))
                 cb = getattr(getattr(updt, "adpt", None), "lambda_callback", lambda: None)()
                 if cb is not None:                              # HaarioTypeAdaptation(...; f = ...)
                     self._keep.append(cb)

@@ -110,11 +110,13 @@ enum {
     EXTMCMC_PRIOR_BETA         = 8, /* Beta(alpha, beta)                                       */
     EXTMCMC_PRIOR_LOGNORMAL    = 9, /* LogNormal(mu, sigma)                                    */
     EXTMCMC_PRIOR_CAUCHY       = 10, /* Cauchy(mu, sigma)                                      */
-    EXTMCMC_PRIOR_MVNORMAL     = 11  /* StandardPrior(MvNormal(mu, Sigma)) on the whole coordinate
+    EXTMCMC_PRIOR_MVNORMAL     = 11, /* StandardPrior(MvNormal(mu, Sigma)) on the whole coordinate
                                         block of a joint update (priors.jl:35-39 wraps any
                                         Distributions object): params = {mu[p_u], L[p_u*p_u]}, L the
                                         lower Cholesky factor of Sigma, column-major (the host side
                                         factorises; the device whitens, as PDMats does)            */
+    EXTMCMC_PRIOR_USER         = 12  /* user-defined prior: CUDA C++ logprior compiled at run time
+                                        (extmcmc_set_user_prior); params = its pp[]               */
 };
 
 /* ---- adaptation schemes (src/transition_kernels/adaptation.jl) ----------- */
@@ -360,6 +362,39 @@ int32_t extmcmc_user_law_check_theta_only(const char *source, int32_t n_params, 
                                           char *log, int64_t log_bytes);
 int32_t extmcmc_set_user_law_theta_only(extmcmc_t h, const char *source, int32_t with_grad, int32_t chunk, int32_t flags,
                                         uint64_t theta_only);
+
+/* ---- user-defined priors (EXTMCMC_PRIOR_USER) -------------------------------
+ * The reference's open Prior type (a user subtype with logpdf(prior, th), priors.jl:4-39) as a string of
+ * CUDA C++ over the update's own p_u coordinates (the compile-time macro EXTMCMC_PU); pp points to the
+ * update's prior_params, so new hyperparameters need no recompilation:
+ *
+ *   __device__ double logprior(const double *th, const double *pp);   // -INFINITY outside the support
+ *   // optional (with_grad = 1): returns logprior and ADDS d logprior / d th into g[0..PU-1]
+ *   __device__ double logprior_grad(const double *th, const double *pp, double *g);
+ *   // forward mode (with_grad = EXTMCMC_USER_GRAD_FORWARD), differentiated on extmcmc::Dual<PU>:
+ *   template <class real> __device__ real logprior(const real *th, const double *pp);
+ *
+ * The rules are those of a user law: -fmad=false, no headers, the EXTMCMC_USER_GRAD_* values.  A
+ * random-walk update draws its proposal inside the prior's own kernel, which redraws while logprior is
+ * exactly -INFINITY (at most 60000 uniforms, as the built-in priors); a MALA update evaluates logprior and
+ * its gradient at the current state and at the proposal, and needs with_grad != 0.  Limits:
+ * 1 <= p_u <= 64 (p_u <= 32 for the random walks), p_u <= 16 in forward mode; beyond them
+ * EXTMCMC_EUNSUPPORTED.  Not with EXTMCMC_SHARD_OBS over several ranks, nor with the persistent block
+ * kernels (sweep_variant 3 / 4): EXTMCMC_EUNSUPPORTED. */
+/* Compiles every kernel of the prior for (p_u, with_grad) for sm_100a, without a handle or a device;
+ * log as in extmcmc_user_law_check.  EXTMCMC_OK, EXTMCMC_EINVAL (does not compile) or
+ * EXTMCMC_EUNSUPPORTED (limits, no NVRTC). */
+int32_t extmcmc_user_prior_check(const char *source, int32_t p_u, int32_t with_grad, char *log, int64_t log_bytes);
+/* Compiles (cached by the exact input) and installs the prior of update u, which extmcmc_set_update set
+ * with prior EXTMCMC_PRIOR_USER; replaces the one it had and invalidates the cached graphs.  A run on a
+ * handle with such an update and no prior installed returns EXTMCMC_EINVAL; a MALA update with a prior
+ * without gradient, EXTMCMC_EUNSUPPORTED. */
+int32_t extmcmc_set_user_prior(extmcmc_t h, int32_t u, const char *source, int32_t with_grad);
+/* logprior of update u's user prior and its gradient at the current state: lp_out[n_chains],
+ * grad_out[p_u * n_chains] (d/dth_i of the update's coordinate i, chain-major), with the kernel a MALA
+ * update runs.  EXTMCMC_EINVAL without a state or an installed user prior, EXTMCMC_EUNSUPPORTED for a
+ * prior without gradient. */
+int32_t extmcmc_eval_user_prior(extmcmc_t h, int32_t u, double *lp_out, double *grad_out);
 
 /* Replaces RandomWalkUpdate(rw, coords; prior, adpt) src/updates.jl:170-182. */
 int32_t extmcmc_set_update(extmcmc_t h, int32_t u, const extmcmc_update_t *upd);

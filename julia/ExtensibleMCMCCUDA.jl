@@ -83,7 +83,7 @@ end
 const LAW_GSN_IID_1D, LAW_GSN_MV, LAW_LOGISTIC, LAW_HIER_NORMAL, LAW_USER = Int32(1), Int32(2), Int32(3), Int32(4), Int32(5)
 const KERNEL_RW_UNIFORM, KERNEL_RW_GAUSS, KERNEL_RW_GAUSS_MIX, KERNEL_MALA = Int32(1), Int32(2), Int32(3), Int32(4)
 const ADAPT_NONE, ADAPT_UNIF_RW, ADAPT_HAARIO, ADAPT_MALA = Int32(0), Int32(1), Int32(2), Int32(3)
-const PRIOR_PRODUCT, PRIOR_MVNORMAL = Int32(5), Int32(11)
+const PRIOR_PRODUCT, PRIOR_MVNORMAL, PRIOR_USER = Int32(5), Int32(11), Int32(12)
 const USER_GRAD_NONE, USER_GRAD_HAND, USER_GRAD_FORWARD = Int32(0), Int32(1), Int32(2)
 const USER_THETA_TERM = Int32(1)
 
@@ -215,12 +215,42 @@ function run_seed(seed::UInt64, run::Int)
     z ⊻ (z >> 31)
 end
 
+"""
+    DevicePrior(source::String; gradient=false, params=Float64[], n_coords=1)
+
+A user-defined prior on the device (EXTMCMC_PRIOR_USER), the reference's open `Prior` type
+(`logpdf(prior, θ)`, src/priors.jl:4-39) written in CUDA C++ over the update's own coordinates
+(`logprior(th, pp)`, and `logprior_grad` with `gradient = true`, or a `logprior<real>` template with
+`gradient = :forward`; contract in include/extmcmc.h and INTEGRATION.md).  `params` are passed as `pp` at
+run time.  Usable as the prior of a random-walk update and, with a gradient, of a CUDAMALAUpdate.  Compiled
+for sm_100a at `n_coords` coordinates when constructed (the workspace compiles it at its update's p_u);
+a source that does not compile throws with the compiler's log.
+"""
+struct DevicePrior <: eMCMC.Prior
+    source::String
+    with_grad::Int32
+    params::Vector{Float64}
+    log::String
+    function DevicePrior(source::String; gradient=false, params=Float64[], n_coords=1)
+        with_grad = gradient === :forward ? USER_GRAD_FORWARD :
+                    gradient === true ? USER_GRAD_HAND :
+                    gradient === false ? USER_GRAD_NONE :
+                    throw(ArgumentError("gradient must be false, true or :forward, not $(repr(gradient))"))
+        buf = zeros(UInt8, 1 << 16)
+        rc = GC.@preserve buf ccall((:extmcmc_user_prior_check, LIB), Int32, (Cstring, Int32, Int32, Ptr{UInt8}, Int64),
+                                    source, n_coords, with_grad, pointer(buf), length(buf))
+        log = unsafe_string(pointer(buf))
+        rc == 0 || throw(ArgumentError("the device prior does not compile (status $rc):\n" * log))
+        new(source, with_grad, Float64.(collect(params)), log)
+    end
+end
 # ---- priors (src/priors.jl:18-88) -> (EXTMCMC_PRIOR_* kind, parameters) -------------------------
 # params(dist) of Distributions.jl returns exactly the parameter order the header documents.
 const PRIOR_KIND = Dict(Normal => 2, Gamma => 3, Uniform => 4, Exponential => 6, InverseGamma => 7,
                         Beta => 8, LogNormal => 9, Cauchy => 10)
 prior_abi(::eMCMC.ImproperPrior) = (Int32(0), Float64[])
 prior_abi(::eMCMC.ImproperPosPrior) = (Int32(1), Float64[])
+prior_abi(pr::DevicePrior) = (PRIOR_USER, pr.params)
 function prior_abi(pr::eMCMC.StandardPrior)
     if pr.dist isa AbstractMvNormal                       # joint prior: {mu[n], L[n*n] column-major}
         L = cholesky(Symmetric(Matrix(cov(pr.dist)))).L
@@ -235,7 +265,8 @@ function prior_abi(pr::eMCMC.ProductPrior)                  # {K, then per facto
     out = Float64[length(pr.dists)]
     for (dist, idx) in zip(pr.dists, pr.idx)
         k, pp = prior_abi(dist isa eMCMC.Prior ? dist : eMCMC.StandardPrior(dist))
-        (k == PRIOR_PRODUCT || k == PRIOR_MVNORMAL) && error("ProductPrior factors must be iid families on the GPU path")
+        (k == PRIOR_PRODUCT || k == PRIOR_MVNORMAL || k == PRIOR_USER) &&
+            error("ProductPrior factors must be iid families on the GPU path")
         append!(out, (Float64(k), Float64(length(idx)), get(pp, 1, 0.0), get(pp, 2, 0.0)))
     end
     (PRIOR_PRODUCT, out)
@@ -356,6 +387,10 @@ function eMCMC.init_global_workspace(b::CUDAMCMCBackend, M, updates::Vector{<:eM
             upd = Update(kern, length(coords), pointer(coords), pointer(step), isempty(pos) ? C_NULL : pointer(pos),
                          prior, length(pp), isempty(pp) ? C_NULL : pointer(pp), adapt)
             check(h[], ccall((:extmcmc_set_update, LIB), Int32, (Ptr{Cvoid}, Int32, Ref{Update}), h[], u - 1, upd))
+        end
+        if updt.prior isa DevicePrior                    # compiled (cached) for this update's p_u
+            check(h[], ccall((:extmcmc_set_user_prior, LIB), Int32, (Ptr{Cvoid}, Int32, Cstring, Int32),
+                             h[], u - 1, updt.prior.source, updt.prior.with_grad))
         end
         if updt.adpt isa eMCMC.HaarioTypeAdaptation
             fref = Ref{Any}(updt.adpt.fλ); push!(keep, fref)
